@@ -1,6 +1,6 @@
-"""Benchmark of the B200-native ORT / ACORT captioning hot path (driver contract: one JSON line on stdout).
+"""Benchmark of the B200-native ORT / ACORT captioning hot path: one JSON result line on stdout.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config infer|train|acort|scst]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config infer|train|acort|scst] [--dump-outputs DIR]
 
 Workloads (BASELINE.json `configs`; synthetic 36-region x 2048-d features + boxes, random-init randomly pruned weights):
   infer (default, configs[2]): ORT 6x512, 95 % sparse binarized-mask weights, beam-3 incremental decoding, L = 16, 512 images
@@ -19,8 +19,13 @@ N > 1: one process per GPU (torchrun), images sharded by rank, no collective on 
                  of one step, alone and with the timed region's concurrency, against MEASURED_PEAKS.json; "hbm_kernels": the
                  HBM-bound decode kernels (cross / self attention, LayerNorm) as GB/s against the measured copy bandwidth.
   cpu_baseline : the CPU oracle (a port of the reference's PyTorch path) on this box's host cores, bounded sample.
+  --dump-outputs DIR : after the timed steps, what the timed path returned for its last step as DIR/<name>.npy (float32 /
+                 float64, rank 0): infer / acort / scst the tokens (beam<b>_seq) and log-probs (beam<b>_logprobs) of each decode
+                 of the last timed device launch, [images, b, L]; train the loss and a seeded sample of the weights and mask
+                 logits the last step left.  Inputs are seeded, so two builds run with the same arguments can be compared file
+                 by file.
   --impl reference : the same CPU arm alone (the reference is pure Python/PyTorch; its hot path restated in
-                 oracle/ort_oracle.py is what runs - /root/reference does not exist on the GPU box).
+                 oracle/ort_oracle.py is what runs).
 """
 import argparse
 import json
@@ -33,6 +38,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 CFG = dict(d_model=512, dim_feedforward=2048, num_layers=6, num_heads=8, max_seq_length=16, att_feat_size=2048,
@@ -70,6 +76,24 @@ def load_traffic():
     (scripts/ncu_gemm_traffic.sh -> profiles/r02_gemm_traffic.json, keys "M,N,K,out_bytes,residual")."""
     p = os.path.join(ROOT, "profiles", "r02_gemm_traffic.json")
     return json.load(open(p)) if os.path.exists(p) else {}
+
+
+def write_outputs(path, arrays, cap=64 << 20):
+    """--dump-outputs: each array as <path>/<name>.npy, float64 kept, everything else as float32 (token ids are exact there).
+    Above `cap` bytes in all, the arrays (which then must share their leading, per-image dimension) keep the same fixed,
+    seeded sample of rows, in order, and rows.npy lists the kept indices."""
+    arrays = {k: v if v.dtype == np.float64 else v.astype(np.float32) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > cap:
+        lead = {v.shape[0] for v in arrays.values()}
+        assert len(lead) == 1, f"cannot sample arrays of different leading dimensions {sorted(lead)} down to {cap} bytes"
+        n = lead.pop()
+        keep = np.sort(np.random.default_rng(0).choice(n, max(1, n * cap // (total + 8 * n)), replace=False))
+        arrays = {k: v[keep] for k, v in arrays.items()}
+        arrays["rows"] = keep.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), v)
 
 
 class ClockSampler(threading.Thread):
@@ -304,10 +328,11 @@ def hbm_kernel_roofline(dev, B, beam, N, cfg, peaks):
 # ----------------------------------------------------------------------------------------------------------------------
 # SMP training arm (BASELINE.json configs[1])
 # ----------------------------------------------------------------------------------------------------------------------
-def train_arm(args, dev, world, rank, dist_mod=None, e2e=False):
+def train_arm(args, dev, world, rank, dist_mod=None, e2e=False, dump=None):
     """ORT supermask training, bf16 tensor-core GEMMs with fp32 master weights + fp32 mask logits, 5 captions/image with the
     encoder run once, Bernoulli masks + dropout + sparsity loss + clip + Adam inside the timed step; at N > 1 the NCCL
-    all-reduce of the flat dWm buffer (tests/test_ddp_cpu.py covers the sharding logic)."""
+    all-reduce of the flat dWm buffer (tests/test_ddp_cpu.py covers the sharding logic).  ``dump``: a dict that receives
+    the last timed step's loss and a seeded sample of the weights and mask logits it left."""
     from sparse_caption_b200 import lib
     from sparse_caption_b200 import synthetic
     from sparse_caption_b200.engine import ModelCfg
@@ -348,6 +373,11 @@ def train_arm(args, dev, world, rank, dist_mod=None, e2e=False):
     e1.record()
     barrier()
     ms_dev = e0.elapsed_time(e1)
+    if dump is not None:   # (110 M weights and as many logits: 2^20 of each, the same positions in every run)
+        g = torch.Generator().manual_seed(0)
+        for name, flat in (("weights_sample", tr.flat_w), ("mask_logits_sample", tr.flat_s)):
+            dump[name] = flat[torch.randint(flat.numel(), (1 << 20,), generator=g).to(dev)].cpu().numpy()
+        dump["loss"] = loss.detach().double().reshape(1).cpu().numpy()
     launches = (lib.launch_count - before) // n_steps
     # end to end: the same step with the loss read back to the host every step (the reference loop's loss.item(), :142,155)
     host_loss = torch.zeros(1).pin_memory()
@@ -448,7 +478,11 @@ def main():
     ap.add_argument("--dec-ctas", default="48,60", help="persistent-grid targets of the decode GEMMs in the throughput regime: CTAs for the wide "
                          "(qkv, ff1) and for the N = d_model GEMMs (OrtEngine dec_ctas); 0,0 = one CTA per SM / two tiles per CTA as before")
     ap.add_argument("--e2e-schedule", default="", help="queued batches per launch of the end-to-end arm, e.g. 2,2,4,4,4,4 (sums to --steps)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="", help="after the timed steps, write what the timed path returned for its "
+                         "last step as DIR/<name>.npy (float32 / float64, at most 64 MB, rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -552,8 +586,7 @@ def main():
         s = slots[i % S]
         with torch.cuda.stream(eng.stream(s)):
             eng.run_encoder(encs[s])
-            for o in opts:
-                eng.decode(encs[s], o)
+            return [eng.decode(encs[s], o) for o in opts]
 
     def fork():
         for s in slots:
@@ -576,11 +609,18 @@ def main():
     e0.record()
     fork()
     for i in range(n_timed):
-        dev_step(i)
+        last = dev_step(i)
     join()
     e1.record()
     barrier()
     ms_dev = e0.elapsed_time(e1)
+    dump = None
+    if args.dump_outputs and rank == 0:
+        # (seq, log-probs) [B, beam, L] per decode of the last timed launch (its G coalesced batches), views of the slot's
+        # workspaces: copied now, outside the timed region; the beam size names the decode (scst: beam 5 and greedy, beam 1)
+        dump = {}
+        for (seq, lp), b in zip(last, beams):
+            dump[f"beam{b}_seq"], dump[f"beam{b}_logprobs"] = seq.cpu().numpy(), lp.cpu().numpy()
 
     # ---------------- end-to-end arm: pinned host inputs -> tokens on the host ----------------
     # --e2e-coalesce 0 (default): 4 queued batches per launch when --steps allows it (else 2 / 1).  The H2D copy of a launch's
@@ -805,6 +845,8 @@ def main():
                               "ms_per_step": ms_e2e16 / args.steps, "host_features": "bf16 pinned"},
             "gpu_launches": launches_per_call * n_timed, "clocks": sampler.summary(), "roofline": roofline,
             "cpu_baseline": cpu, "train": train}
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
     print(json.dumps(line), file=out, flush=True)
     if dist is not None:
         dist.destroy_process_group()
@@ -845,7 +887,8 @@ def train_main(args, out, rank, local_rank, world):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    tr = train_arm(args, dev, world, rank, dist_mod=dist, e2e=True)
+    dump = {} if args.dump_outputs and rank == 0 else None
+    tr = train_arm(args, dev, world, rank, dist_mod=dist, e2e=True, dump=dump)
     sampler.stop_flag = True
     if rank != 0:
         if dist is not None:
@@ -862,6 +905,8 @@ def train_main(args, out, rank, local_rank, world):
             "data": "synthetic", "config": config, "e2e": tr["e2e"], "gpu_launches": tr["gpu_launches_per_step"] * args.steps,
             "clocks": sampler.summary(), "roofline": tr["roofline"], "cpu_baseline": cpu,
             "train_detail": {k: v for k, v in tr.items() if k not in ("roofline", "e2e")}}
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
     print(json.dumps(line), file=out, flush=True)
     if dist is not None:
         dist.destroy_process_group()
