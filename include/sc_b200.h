@@ -196,6 +196,25 @@ int sc_beam_step(const float* logits, int B, int beam, int V, int L, int t, int 
                  const float* lp_in, float* lp_out, float* sum, const int* anc_in, int* anc_out, int* tokens_out,
                  int* done_seq, float* done_lp, double* done_p, int* done_count, void* workspace, size_t workspace_bytes,
                  sc_stream_t stream);
+/* Diverse beam search (group_size G > 1, caption_model.py:30-226 with add_diversity :33-52): the beam step of group `group`
+ * (its bdash = `beam` beams per image) at its local step t.  Candidates are ranked by sum + (log-prob - diversity_lambda *
+ * count), count = the number of beams of groups p < group whose token at position t of their CURRENT history is that column;
+ * the running sum and the finished-beam score take the penalised value, the stored per-token log-prob (lp_out, done_lp) the
+ * unpenalised one.  group_seq: every group's seq ping-pong buffers as one int32 [G][2][B*beam][L] tensor (seq_in / seq_out
+ * are two of them); the groups are staggered in time, so group p has run its local step min(t + group - p, L-1) already and
+ * its current history is buffer (that step + 1) % 2.  Everything else as sc_beam_step / sc_beam_step_partials; group * beam
+ * <= 256, and for the records path (group + 1) * beam <= 5 with sc_linear_topk candidates >= (group + 1) * beam. */
+int sc_beam_step_diverse(const float* logits, int B, int beam, int V, int L, int t, int eos, int pad, float temperature,
+                         int decoding_constraint, int penalty_kind, float penalty_alpha, const int* suppress_tok, int penalized_col,
+                         const int* group_seq, int group, float diversity_lambda, const int* seq_in, int* seq_out,
+                         const float* lp_in, float* lp_out, float* sum, const int* anc_in, int* anc_out, int* tokens_out,
+                         int* done_seq, float* done_lp, double* done_p, int* done_count, void* workspace, size_t workspace_bytes,
+                         sc_stream_t stream);
+int sc_beam_step_partials_diverse(const float* partials, int parts_per_row, int B, int beam, int V, int L, int t, int eos, int pad,
+                                  int penalty_kind, float penalty_alpha, const int* group_seq, int group, float diversity_lambda,
+                                  const int* seq_in, int* seq_out, const float* lp_in, float* lp_out, float* sum,
+                                  const int* anc_in, int* anc_out, int* tokens_out, int* done_seq, float* done_lp, double* done_p,
+                                  int* done_count, void* workspace, size_t workspace_bytes, sc_stream_t stream);
 
 /* greedy branch of _generate_captions (models/transformer.py:507-561) */
 int sc_greedy_step(const float* logits, int R, int V, int L, int t, int eos, int decoding_constraint, int* seq,

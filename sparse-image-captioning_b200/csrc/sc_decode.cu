@@ -332,7 +332,59 @@ struct BeamArgs {
   // suppress_UNK (:169-170): column whose log-prob is lowered by 1000 (-1 = none).  Both act AFTER the normalisation.
   const int* suppress_tok;
   int penalized_col;
+  // diverse beam search (sc_beam_step_diverse, caption_model.py:33-52): the candidates of this group are ranked by
+  // log-prob - div_lambda * (number of beams of the groups p < div_group whose token at position t is that column).
+  // div_hist holds every group's seq ping-pong buffers [G][2][B*beam][L]; t is this group's local step.
+  const int* div_hist;
+  int div_group;
+  float div_lambda;
 };
+
+// Diverse beam search: tokens at position a.t of the current beams of groups p < a.div_group for image b.  The groups are
+// staggered (group p runs at local step a.t + div_group - p in the same global step and has already taken it, or stopped
+// at L-1), so group p's current history is its ping-pong buffer (min(a.t + div_group - p, L-1) + 1) & 1.
+__device__ __forceinline__ int diversity_token(const BeamArgs& a, int NB, int b, int i) {
+  const int p = i / NB, j = i - p * NB;
+  const int tp = min(a.t + a.div_group - p, a.L - 1);
+  return a.div_hist[(((size_t)p * 2 + ((tp + 1) & 1)) * a.B * NB + (size_t)b * NB + j) * a.L + a.t];
+}
+
+// Block-wide: s_tok[i] = the i-th earlier-group token, s_cnt[i] = its multiplicity at its first occurrence, 0 at repeats.
+// Returns the number of entries (div_group * NB <= kBeamThreads).
+__device__ __forceinline__ int diversity_table(const BeamArgs& a, int NB, int b, int* s_tok, float* s_cnt) {
+  const int n = a.div_group * NB, tid = threadIdx.x;
+  int tok = -1;
+  if (tid < n) s_tok[tid] = tok = diversity_token(a, NB, b, tid);
+  __syncthreads();
+  if (tid < n) {
+    int c = 0;
+    bool first = true;
+    for (int i = 0; i < n; ++i) {
+      c += s_tok[i] == tok;
+      first = first && !(i < tid && s_tok[i] == tok);
+    }
+    s_cnt[tid] = first ? (float)c : 0.f;
+  }
+  __syncthreads();
+  return n;
+}
+
+__device__ __forceinline__ float diversity_count(int col, int n, const int* s_tok, const float* s_cnt) {
+  float c = 0.f;
+  for (int i = 0; i < n; ++i) c += (s_tok[i] == col) ? s_cnt[i] : 0.f;
+  return c;
+}
+
+// Smallest penalised column > `after` owned by this thread in a column-strided scan (col % kBeamThreads == threadIdx.x);
+// 0x7fffffff when none is left.
+__device__ __forceinline__ int diversity_next(int after, int n, const int* s_tok, const float* s_cnt) {
+  int best = 0x7fffffff;
+  for (int i = 0; i < n; ++i) {
+    const int c = s_tok[i];
+    if (s_cnt[i] > 0.f && c > after && c < best && c % kBeamThreads == (int)threadIdx.x) best = c;
+  }
+  return best;
+}
 
 __device__ __forceinline__ float block_max(float v, float* s_red) {
   v = sc::warp_max(v);
@@ -358,7 +410,9 @@ __device__ __forceinline__ float block_sum(float v, float* s_red) {
 // Phase A — one CTA per ROW (image, beam): the row is read from HBM exactly once into registers (kRegs: V <= 256*40;
 // otherwise re-read through L2), log-softmax statistics, then the row's top-NB candidates by FINAL score
 // (sum + log-prob, ties to the smaller flat index == stable descending sort) -> workspace.
-template <int NB, bool kRegs>
+// kDiv (diverse beam search): the final score is sum + (log-prob - lambda * count); log-softmax statistics come from the
+// row without the penalty, and within the row the score is monotone in x - T * lambda * count (as for suppress_UNK).
+template <int NB, bool kRegs, bool kDiv = false>
 __global__ void __launch_bounds__(kBeamThreads, 4) beam_row_kernel(const BeamArgs a, float* __restrict__ ws_stats,
                                                                 Cand* __restrict__ ws_cand) {
   const int r = blockIdx.x;            // row = b*NB + k
@@ -369,6 +423,9 @@ __global__ void __launch_bounds__(kBeamThreads, 4) beam_row_kernel(const BeamArg
   const int V = a.V;
   __shared__ float s_red[kBeamWarps];
   __shared__ Cand s_top[kBeamWarps][NB];
+  __shared__ int s_dtok[kDiv ? kBeamThreads : 1];
+  __shared__ float s_dcnt[kDiv ? kBeamThreads : 1];
+  const int ndiv = kDiv ? diversity_table(a, NB, r / NB, s_dtok, s_dcnt) : 0;
   // init_logprobs (t == 0) are never temperature-scaled (caption_model.py:135, 218)
   const float T = (a.t == 0) ? 1.0f : a.temperature;
   const float* x = a.logits + (size_t)r * V;
@@ -433,11 +490,45 @@ __global__ void __launch_bounds__(kBeamThreads, 4) beam_row_kernel(const BeamArg
       }
       ls2 = logf(block_sum(se2, s_red));
     }
+    if (kDiv) {
+      // The scan above ranked unpenalised logits.  A thread that owns a penalised column (at most g*bdash of the 256) ranks
+      // its columns again by x - T * lambda * count, re-read through L1 now that the row's registers are free; the other
+      // threads' lists hold no penalised column and stand.
+      bool owner = false;
+      for (int d = 0; d < ndiv; ++d) owner |= s_dcnt[d] > 0.f && (s_dtok[d] >> 2) % kBeamThreads == tid;
+      if (owner) {
+#pragma unroll
+        for (int i = 0; i < NB; ++i) { rawtop[i].s = -INFINITY; rawtop[i].idx = 0x7fffffff; }
+        for (int c0 = tid * 4; c0 < V; c0 += kBeamThreads * 4) {
+          for (int e = 0; e < 4; ++e) {
+            const int col = c0 + e;
+            float v = __ldg(x + col);
+            if (col == prev || col == sup) v = -INFINITY;
+            if (col == pen) v -= 1000.f * T;
+            v -= T * a.div_lambda * diversity_count(col, ndiv, s_dtok, s_dcnt);
+            if (v > rawtop[NB - 1].s) {  // ascending index order: strict '>' keeps the smaller index on ties
+              Cand cd; cd.s = v; cd.idx = col;
+              topk_insert<NB>(rawtop, cd);
+            }
+          }
+        }
+      }
+    }
 #pragma unroll
     for (int i = 0; i < NB; ++i) {
       if (rawtop[i].idx != 0x7fffffff && rawtop[i].s > -INFINITY) {
-        float lp = (rawtop[i].s - mx) - ls;
-        if (T != 1.0f) lp = (lp / T - mx2) - ls2;
+        float lp;
+        if (kDiv) {
+          // exact score of the survivor from its unpenalised logit: (log-prob [- 1000]) - lambda * count
+          const int col = rawtop[i].idx;
+          lp = (__ldg(x + col) - mx) - ls;
+          if (T != 1.0f) lp = (lp / T - mx2) - ls2;
+          if (col == pen) lp -= 1000.f;
+          lp = __fsub_rn(lp, __fmul_rn(a.div_lambda, diversity_count(col, ndiv, s_dtok, s_dcnt)));
+        } else {
+          lp = (rawtop[i].s - mx) - ls;
+          if (T != 1.0f) lp = (lp / T - mx2) - ls2;
+        }
         Cand cd; cd.s = base + lp; cd.idx = k * V + rawtop[i].idx;
         topk_insert<NB>(top, cd);
       }
@@ -455,11 +546,17 @@ __global__ void __launch_bounds__(kBeamThreads, 4) beam_row_kernel(const BeamArg
       for (int i = tid; i < V; i += kBeamThreads) se2 += __expf(((x[i] - mx) - ls) / T - mx2);
       ls2 = logf(block_sum(se2, s_red));
     }
+    // kDiv: the thread walks its own penalised columns in ascending order next to the scan (O(V) plus O(g*bdash) per hit)
+    int next_pen = kDiv ? diversity_next(-1, ndiv, s_dtok, s_dcnt) : -1;
     for (int i = tid; i < V; i += kBeamThreads) {
       float lp = (x[i] - mx) - ls;
       if (T != 1.0f) lp = (lp / T - mx2) - ls2;
       if (i == prev || i == sup) lp = -INFINITY;
       if (i == pen) lp -= 1000.f;
+      if (kDiv && i == next_pen) {
+        lp = __fsub_rn(lp, __fmul_rn(a.div_lambda, diversity_count(i, ndiv, s_dtok, s_dcnt)));
+        next_pen = diversity_next(i, ndiv, s_dtok, s_dcnt);
+      }
       Cand cd; cd.s = base + lp; cd.idx = k * V + i;
       topk_insert<NB>(top, cd);
     }
@@ -514,10 +611,14 @@ __global__ void __launch_bounds__(kBeamThreads, 4) beam_row_kernel(const BeamArg
 // candidates (same outputs as beam_row_kernel, plus the raw logit of each candidate for the merge kernel).
 constexpr int kPartTopK = 5;
 constexpr int kPartRec = 2 + 2 * kPartTopK;
-template <int NB>
+// kDiv (diverse beam search, group g of bdash = NB beams): the row keeps its top NB + g*NB <= kPartTopK raw candidates (the
+// records must hold that many: sc_linear_topk candidates = the whole beam size); at most g*NB distinct columns are
+// penalised, so the top NB by penalised score are among them.
+template <int NB, bool kDiv = false>
 __global__ void __launch_bounds__(256) beam_row_partials_kernel(const BeamArgs a, const float* __restrict__ part, int P,
                                                                 float* __restrict__ ws_stats, Cand* __restrict__ ws_cand,
                                                                 float* __restrict__ ws_raw) {
+  constexpr int NR = kDiv ? kPartTopK : NB;  // raw candidates kept per row
   sc::pdl_launch();
   sc::pdl_wait();
   const int lane = threadIdx.x & 31;
@@ -526,11 +627,11 @@ __global__ void __launch_bounds__(256) beam_row_partials_kernel(const BeamArgs a
   const int k = r % NB;
   if (a.t == 0 && k != 0) return;  // first step: only beam 0 is expanded
   const float* pr = part + (size_t)r * P * kPartRec;
-  // lane-local: running (max, sum) and top-NB by (raw logit, smaller column)
+  // lane-local: running (max, sum) and top-NR by (raw logit, smaller column)
   float m = -INFINITY, sum = 0.f;
-  Cand top[NB];
+  Cand top[NR];
 #pragma unroll
-  for (int i = 0; i < NB; ++i) { top[i].s = -INFINITY; top[i].idx = 0x7fffffff; }
+  for (int i = 0; i < NR; ++i) { top[i].s = -INFINITY; top[i].idx = 0x7fffffff; }
   for (int p = lane; p < P; p += 32) {
     const float* rec = pr + (size_t)p * kPartRec;
     const float pm = rec[0], ps = rec[1];
@@ -540,9 +641,9 @@ __global__ void __launch_bounds__(256) beam_row_partials_kernel(const BeamArgs a
     }
 #pragma unroll
     for (int i = 0; i < kPartTopK; ++i) {
-      if (i >= NB) break;  // a record's i-th entry can only matter for i < NB
+      if (i >= NR) break;  // a record's i-th entry can only matter for i < NR
       Cand cd; cd.s = rec[2 + i]; cd.idx = __float_as_int(rec[2 + kPartTopK + i]);
-      if (cd.idx != 0x7fffffff) topk_insert<NB>(top, cd);
+      if (cd.idx != 0x7fffffff) topk_insert<NR>(top, cd);
     }
   }
   // warp: global max, rescaled sum
@@ -554,11 +655,12 @@ __global__ void __launch_bounds__(256) beam_row_partials_kernel(const BeamArgs a
   // warp merge of the lanes' sorted lists (NB rounds of arg-best over the heads), ranking by (raw logit, column) - within
   // a row the final score base + (x - M) - ls is monotone in x
   int head = 0;
+  Cand raw[NR];  // the row's top-NR (raw logit, column), warp-uniform
 #pragma unroll
-  for (int rnd = 0; rnd < NB; ++rnd) {
+  for (int rnd = 0; rnd < NR; ++rnd) {
     Cand c; c.s = -INFINITY; c.idx = 0x7fffffff;
 #pragma unroll
-    for (int i = 0; i < NB; ++i) if (i == head) c = top[i];
+    for (int i = 0; i < NR; ++i) if (i == head) c = top[i];
     Cand best = c;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
@@ -567,12 +669,43 @@ __global__ void __launch_bounds__(256) beam_row_partials_kernel(const BeamArgs a
       other.idx = __shfl_xor_sync(0xffffffffu, best.idx, o);
       if (better(other, best)) best = other;
     }
-    if (head < NB && c.idx == best.idx && c.s == best.s) head++;
-    if (lane == 0) {
+    if (head < NR && c.idx == best.idx && c.s == best.s) head++;
+    raw[rnd] = best;
+    if (!kDiv && lane == 0) {
       Cand out; out.s = -INFINITY; out.idx = 0x7fffffff;
       if (best.idx != 0x7fffffff) { out.s = base + ((best.s - M) - ls); out.idx = k * a.V + best.idx; }
       ws_cand[(size_t)r * NB + rnd] = out;
       ws_raw[(size_t)r * NB + rnd] = best.s;
+    }
+  }
+  if (kDiv) {
+    // lane i < g*NB holds the i-th earlier-group token; exact penalised scores of the NR raw candidates, then the top NB
+    const int n = a.div_group * NB;
+    const int tok = lane < n ? diversity_token(a, NB, r / NB, lane) : -1;
+    Cand sc[NR];
+#pragma unroll
+    for (int i = 0; i < NR; ++i) {
+      float c = 0.f;
+      for (int j = 0; j < n; ++j) c += (__shfl_sync(0xffffffffu, tok, j) == raw[i].idx) ? 1.f : 0.f;
+      sc[i].s = -INFINITY; sc[i].idx = 0x7fffffff;
+      if (raw[i].idx != 0x7fffffff) {
+        sc[i].s = base + __fsub_rn((raw[i].s - M) - ls, __fmul_rn(a.div_lambda, c));
+        sc[i].idx = k * a.V + raw[i].idx;
+      }
+    }
+    unsigned used = 0;
+#pragma unroll
+    for (int rnd = 0; rnd < NB; ++rnd) {
+      int bj = 0;
+      Cand best; best.s = -INFINITY; best.idx = 0x7fffffff;
+#pragma unroll
+      for (int i = 0; i < NR; ++i)
+        if (!(used >> i & 1u) && better(sc[i], best)) { best = sc[i]; bj = i; }
+      used |= 1u << bj;
+      if (lane == 0) {
+        ws_cand[(size_t)r * NB + rnd] = best;
+        ws_raw[(size_t)r * NB + rnd] = raw[bj].s;
+      }
     }
   }
   if (lane == 0) { ws_stats[r * 4 + 0] = M; ws_stats[r * 4 + 1] = ls; ws_stats[r * 4 + 2] = 0.f; ws_stats[r * 4 + 3] = 0.f; }
@@ -886,33 +1019,26 @@ size_t sc_beam_step_workspace_bytes_impl(int B, int beam) {
   return (size_t)B * beam * (4 * sizeof(float) + (size_t)beam * sizeof(Cand) + (size_t)beam * sizeof(float));
 }
 
-int sc_beam_step(const float* logits, int B, int beam, int V, int L, int t, int eos, int pad, float temperature,
-                 int decoding_constraint, int penalty_kind, float penalty_alpha, const int* suppress_tok, int penalized_col,
-                 const int* seq_in, int* seq_out,
-                 const float* lp_in, float* lp_out, float* sum, const int* anc_in, int* anc_out, int* tokens_out,
-                 int* done_seq, float* done_lp, double* done_p, int* done_count, void* workspace, size_t workspace_bytes,
-                 cudaStream_t stream) {
-  SC_CHECK(B > 0 && beam >= 1 && beam <= kMaxBeam, SC_ERR_UNSUPPORTED, "sc_beam_step: beam=%d not in [1,%d]", beam, kMaxBeam);
-  SC_CHECK(V >= beam && L > 0 && t >= 0 && t < L, SC_ERR_SHAPE, "sc_beam_step: V=%d L=%d t=%d", V, L, t);
-  SC_CHECK(temperature > 0.f, SC_ERR_SHAPE, "sc_beam_step: temperature must be > 0");
+// Row pass + merge over materialised logits; a.div_hist != nullptr selects the diverse-beam row pass.
+static int beam_step_launch(const char* name, const BeamArgs& a, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+  const int B = a.B, beam = a.beam, V = a.V, L = a.L, t = a.t;
+  SC_CHECK(B > 0 && beam >= 1 && beam <= kMaxBeam, SC_ERR_UNSUPPORTED, "%s: beam=%d not in [1,%d]", name, beam, kMaxBeam);
+  SC_CHECK(V >= beam && L > 0 && t >= 0 && t < L, SC_ERR_SHAPE, "%s: V=%d L=%d t=%d", name, V, L, t);
+  SC_CHECK(a.temperature > 0.f, SC_ERR_SHAPE, "%s: temperature must be > 0", name);
   SC_CHECK(workspace != nullptr && ((uintptr_t)workspace & 15) == 0 && workspace_bytes >= sc_beam_step_workspace_bytes_impl(B, beam),
-           SC_ERR_WORKSPACE, "sc_beam_step: workspace of %zu bytes (16-byte aligned) needed, got %zu",
+           SC_ERR_WORKSPACE, "%s: workspace of %zu bytes (16-byte aligned) needed, got %zu", name,
            sc_beam_step_workspace_bytes_impl(B, beam), workspace_bytes);
-  BeamArgs a;
-  a.logits = logits; a.B = B; a.beam = beam; a.V = V; a.L = L; a.t = t; a.eos = eos; a.pad = pad;
-  a.temperature = temperature; a.constraint = decoding_constraint; a.penalty_kind = penalty_kind;
-  a.penalty_alpha = penalty_alpha; a.seq_in = seq_in; a.seq_out = seq_out; a.lp_in = lp_in; a.lp_out = lp_out;
-  a.sum = sum; a.anc_in = anc_in; a.anc_out = anc_out; a.tokens_out = tokens_out; a.done_seq = done_seq;
-  a.done_lp = done_lp; a.done_p = done_p; a.done_count = done_count; a.ws_raw = nullptr;
-  a.suppress_tok = suppress_tok; a.penalized_col = (penalized_col >= 0 && penalized_col < V) ? penalized_col : -1;
   float* ws_stats = (float*)workspace;
   Cand* ws_cand = (Cand*)(ws_stats + (size_t)B * beam * 4);
-  const bool regs = V <= kBeamThreads * kBeamRegs && (V & 3) == 0 && ((uintptr_t)logits & 15) == 0;
-#define BEAM_LAUNCH(NBV)                                                                                     \
-  do {                                                                                                        \
-    if (regs) sc::launch_pdl(beam_row_kernel<NBV, true>, dim3(B * NBV), dim3(kBeamThreads), 0, stream, a, ws_stats, ws_cand);  \
-    else sc::launch_pdl(beam_row_kernel<NBV, false>, dim3(B * NBV), dim3(kBeamThreads), 0, stream, a, ws_stats, ws_cand);      \
-    sc::launch_pdl(beam_merge_kernel<NBV>, dim3(B), dim3(kMergeThreads), 0, stream, a, ws_stats, (const Cand*)ws_cand);         \
+  const bool regs = V <= kBeamThreads * kBeamRegs && (V & 3) == 0 && ((uintptr_t)a.logits & 15) == 0;
+  const bool div = a.div_hist != nullptr;
+#define BEAM_LAUNCH(NBV)                                                                                                     \
+  do {                                                                                                                        \
+    if (div && regs) sc::launch_pdl(beam_row_kernel<NBV, true, true>, dim3(B * NBV), dim3(kBeamThreads), 0, stream, a, ws_stats, ws_cand);   \
+    else if (div) sc::launch_pdl(beam_row_kernel<NBV, false, true>, dim3(B * NBV), dim3(kBeamThreads), 0, stream, a, ws_stats, ws_cand);    \
+    else if (regs) sc::launch_pdl(beam_row_kernel<NBV, true>, dim3(B * NBV), dim3(kBeamThreads), 0, stream, a, ws_stats, ws_cand);          \
+    else sc::launch_pdl(beam_row_kernel<NBV, false>, dim3(B * NBV), dim3(kBeamThreads), 0, stream, a, ws_stats, ws_cand);                   \
+    sc::launch_pdl(beam_merge_kernel<NBV>, dim3(B), dim3(kMergeThreads), 0, stream, a, ws_stats, (const Cand*)ws_cand);                   \
   } while (0)
   switch (beam) {
     case 1: BEAM_LAUNCH(1); break;
@@ -925,38 +1051,73 @@ int sc_beam_step(const float* logits, int B, int beam, int V, int L, int t, int 
     default: BEAM_LAUNCH(8); break;
   }
 #undef BEAM_LAUNCH
-  SC_LAUNCH_CHECK("sc_beam_step");
+  SC_LAUNCH_CHECK(name);
   return SC_OK;
+}
+
+static BeamArgs beam_args(const float* logits, int B, int beam, int V, int L, int t, int eos, int pad, float temperature,
+                          int decoding_constraint, int penalty_kind, float penalty_alpha, const int* suppress_tok, int penalized_col,
+                          const int* seq_in, int* seq_out, const float* lp_in, float* lp_out, float* sum, const int* anc_in,
+                          int* anc_out, int* tokens_out, int* done_seq, float* done_lp, double* done_p, int* done_count) {
+  BeamArgs a;
+  a.logits = logits; a.B = B; a.beam = beam; a.V = V; a.L = L; a.t = t; a.eos = eos; a.pad = pad;
+  a.temperature = temperature; a.constraint = decoding_constraint; a.penalty_kind = penalty_kind;
+  a.penalty_alpha = penalty_alpha; a.seq_in = seq_in; a.seq_out = seq_out; a.lp_in = lp_in; a.lp_out = lp_out;
+  a.sum = sum; a.anc_in = anc_in; a.anc_out = anc_out; a.tokens_out = tokens_out; a.done_seq = done_seq;
+  a.done_lp = done_lp; a.done_p = done_p; a.done_count = done_count; a.ws_raw = nullptr;
+  a.suppress_tok = suppress_tok; a.penalized_col = (penalized_col >= 0 && penalized_col < V) ? penalized_col : -1;
+  a.div_hist = nullptr; a.div_group = 0; a.div_lambda = 0.f;
+  return a;
+}
+
+int sc_beam_step(const float* logits, int B, int beam, int V, int L, int t, int eos, int pad, float temperature,
+                 int decoding_constraint, int penalty_kind, float penalty_alpha, const int* suppress_tok, int penalized_col,
+                 const int* seq_in, int* seq_out,
+                 const float* lp_in, float* lp_out, float* sum, const int* anc_in, int* anc_out, int* tokens_out,
+                 int* done_seq, float* done_lp, double* done_p, int* done_count, void* workspace, size_t workspace_bytes,
+                 cudaStream_t stream) {
+  const BeamArgs a = beam_args(logits, B, beam, V, L, t, eos, pad, temperature, decoding_constraint, penalty_kind, penalty_alpha,
+                               suppress_tok, penalized_col, seq_in, seq_out, lp_in, lp_out, sum, anc_in, anc_out, tokens_out,
+                               done_seq, done_lp, done_p, done_count);
+  return beam_step_launch("sc_beam_step", a, workspace, workspace_bytes, stream);
+}
+
+int sc_beam_step_diverse(const float* logits, int B, int beam, int V, int L, int t, int eos, int pad, float temperature,
+                         int decoding_constraint, int penalty_kind, float penalty_alpha, const int* suppress_tok, int penalized_col,
+                         const int* group_seq, int group, float diversity_lambda, const int* seq_in, int* seq_out,
+                         const float* lp_in, float* lp_out, float* sum, const int* anc_in, int* anc_out, int* tokens_out,
+                         int* done_seq, float* done_lp, double* done_p, int* done_count, void* workspace, size_t workspace_bytes,
+                         cudaStream_t stream) {
+  SC_CHECK(group_seq != nullptr && group >= 0 && group * beam <= kBeamThreads, SC_ERR_SHAPE,
+           "sc_beam_step_diverse: group=%d x beam=%d earlier-group beams (at most %d)", group, beam, kBeamThreads);
+  BeamArgs a = beam_args(logits, B, beam, V, L, t, eos, pad, temperature, decoding_constraint, penalty_kind, penalty_alpha,
+                         suppress_tok, penalized_col, seq_in, seq_out, lp_in, lp_out, sum, anc_in, anc_out, tokens_out,
+                         done_seq, done_lp, done_p, done_count);
+  a.div_hist = group_seq; a.div_group = group; a.div_lambda = diversity_lambda;
+  return beam_step_launch("sc_beam_step_diverse", a, workspace, workspace_bytes, stream);
 }
 
 // Beam step from the records of sc_linear_topk instead of materialised logits (temperature 1, no decoding constraint,
 // beam <= 5 = the record's candidate count; other options: run sc_linear + sc_beam_step).
-int sc_beam_step_partials(const float* partials, int parts_per_row, int B, int beam, int V, int L, int t, int eos, int pad,
-                          int penalty_kind, float penalty_alpha, const int* seq_in, int* seq_out, const float* lp_in,
-                          float* lp_out, float* sum, const int* anc_in, int* anc_out, int* tokens_out, int* done_seq,
-                          float* done_lp, double* done_p, int* done_count, void* workspace, size_t workspace_bytes,
-                          cudaStream_t stream) {
-  SC_CHECK(B > 0 && beam >= 1 && beam <= kPartTopK, SC_ERR_UNSUPPORTED, "sc_beam_step_partials: beam=%d not in [1,%d]", beam, kPartTopK);
+static int beam_step_partials_launch(const char* name, BeamArgs& a, const float* partials, int parts_per_row, void* workspace,
+                                     size_t workspace_bytes, cudaStream_t stream) {
+  const int B = a.B, beam = a.beam, V = a.V, L = a.L, t = a.t;
+  SC_CHECK(B > 0 && beam >= 1 && beam <= kPartTopK, SC_ERR_UNSUPPORTED, "%s: beam=%d not in [1,%d]", name, beam, kPartTopK);
   SC_CHECK(V >= beam && L > 0 && t >= 0 && t < L && parts_per_row > 0 && partials != nullptr, SC_ERR_SHAPE,
-           "sc_beam_step_partials: V=%d L=%d t=%d parts=%d", V, L, t, parts_per_row);
+           "%s: V=%d L=%d t=%d parts=%d", name, V, L, t, parts_per_row);
   SC_CHECK(workspace != nullptr && ((uintptr_t)workspace & 15) == 0 && workspace_bytes >= sc_beam_step_workspace_bytes_impl(B, beam),
-           SC_ERR_WORKSPACE, "sc_beam_step_partials: workspace of %zu bytes (16-byte aligned) needed, got %zu",
+           SC_ERR_WORKSPACE, "%s: workspace of %zu bytes (16-byte aligned) needed, got %zu", name,
            sc_beam_step_workspace_bytes_impl(B, beam), workspace_bytes);
-  BeamArgs a;
-  a.logits = nullptr; a.B = B; a.beam = beam; a.V = V; a.L = L; a.t = t; a.eos = eos; a.pad = pad;
-  a.temperature = 1.0f; a.constraint = 0; a.penalty_kind = penalty_kind;
-  a.penalty_alpha = penalty_alpha; a.seq_in = seq_in; a.seq_out = seq_out; a.lp_in = lp_in; a.lp_out = lp_out;
-  a.sum = sum; a.anc_in = anc_in; a.anc_out = anc_out; a.tokens_out = tokens_out; a.done_seq = done_seq;
-  a.done_lp = done_lp; a.done_p = done_p; a.done_count = done_count;
-  a.suppress_tok = nullptr; a.penalized_col = -1;
   float* ws_stats = (float*)workspace;
   Cand* ws_cand = (Cand*)(ws_stats + (size_t)B * beam * 4);
   float* ws_raw = (float*)(ws_cand + (size_t)B * beam * beam);
   a.ws_raw = ws_raw;
   const int R = B * beam;
+  const bool div = a.div_hist != nullptr;
 #define BEAMP_LAUNCH(NBV)                                                                                                   \
   do {                                                                                                                       \
-    sc::launch_pdl(beam_row_partials_kernel<NBV>, dim3((R + 7) / 8), dim3(256), 0, stream, a, partials, parts_per_row, ws_stats, ws_cand, ws_raw); \
+    if (div) sc::launch_pdl(beam_row_partials_kernel<NBV, true>, dim3((R + 7) / 8), dim3(256), 0, stream, a, partials, parts_per_row, ws_stats, ws_cand, ws_raw); \
+    else sc::launch_pdl(beam_row_partials_kernel<NBV>, dim3((R + 7) / 8), dim3(256), 0, stream, a, partials, parts_per_row, ws_stats, ws_cand, ws_raw); \
     sc::launch_pdl(beam_merge_kernel<NBV>, dim3(B), dim3(kMergeThreads), 0, stream, a, (const float*)ws_stats, (const Cand*)ws_cand); \
   } while (0)
   switch (beam) {
@@ -967,8 +1128,32 @@ int sc_beam_step_partials(const float* partials, int parts_per_row, int B, int b
     default: BEAMP_LAUNCH(5); break;
   }
 #undef BEAMP_LAUNCH
-  SC_LAUNCH_CHECK("sc_beam_step_partials");
+  SC_LAUNCH_CHECK(name);
   return SC_OK;
+}
+
+int sc_beam_step_partials(const float* partials, int parts_per_row, int B, int beam, int V, int L, int t, int eos, int pad,
+                          int penalty_kind, float penalty_alpha, const int* seq_in, int* seq_out, const float* lp_in,
+                          float* lp_out, float* sum, const int* anc_in, int* anc_out, int* tokens_out, int* done_seq,
+                          float* done_lp, double* done_p, int* done_count, void* workspace, size_t workspace_bytes,
+                          cudaStream_t stream) {
+  BeamArgs a = beam_args(nullptr, B, beam, V, L, t, eos, pad, 1.0f, 0, penalty_kind, penalty_alpha, nullptr, -1, seq_in, seq_out,
+                         lp_in, lp_out, sum, anc_in, anc_out, tokens_out, done_seq, done_lp, done_p, done_count);
+  return beam_step_partials_launch("sc_beam_step_partials", a, partials, parts_per_row, workspace, workspace_bytes, stream);
+}
+
+int sc_beam_step_partials_diverse(const float* partials, int parts_per_row, int B, int beam, int V, int L, int t, int eos, int pad,
+                                  int penalty_kind, float penalty_alpha, const int* group_seq, int group, float diversity_lambda,
+                                  const int* seq_in, int* seq_out, const float* lp_in, float* lp_out, float* sum,
+                                  const int* anc_in, int* anc_out, int* tokens_out, int* done_seq, float* done_lp, double* done_p,
+                                  int* done_count, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+  SC_CHECK(group_seq != nullptr && group >= 0 && (group + 1) * beam <= kPartTopK, SC_ERR_UNSUPPORTED,
+           "sc_beam_step_partials_diverse: (group=%d + 1) x beam=%d raw candidates per row exceed the record's %d", group, beam,
+           kPartTopK);
+  BeamArgs a = beam_args(nullptr, B, beam, V, L, t, eos, pad, 1.0f, 0, penalty_kind, penalty_alpha, nullptr, -1, seq_in, seq_out,
+                         lp_in, lp_out, sum, anc_in, anc_out, tokens_out, done_seq, done_lp, done_p, done_count);
+  a.div_hist = group_seq; a.div_group = group; a.div_lambda = diversity_lambda;
+  return beam_step_partials_launch("sc_beam_step_partials_diverse", a, partials, parts_per_row, workspace, workspace_bytes, stream);
 }
 
 int sc_beam_step_workspace_bytes(int B, int beam) { return (int)sc_beam_step_workspace_bytes_impl(B, beam); }

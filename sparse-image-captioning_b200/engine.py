@@ -543,7 +543,7 @@ class OrtEngine:
         return (self.fuse_topk and self.adt == torch.bfloat16 and g.w is not None and g.w.dtype == torch.bfloat16 and beam <= 5
                 and g.K % 8 == 0)
 
-    def _decode_step(self, ws, enc, t, anc, fused_topk=False):
+    def _decode_step(self, ws, enc, t, anc, fused_topk=False, candidates=None):
         c = self.cfg
         R, d, h, N = ws.R, c.d_model, c.num_heads, ws.N
         fold = self.fold_dec
@@ -595,7 +595,7 @@ class OrtEngine:
         # folded-LayerNorm variant, and one LayerNorm per step is 1/19 of them)
         self.dec_norm(ws.x, ws.xn)
         if fused_topk:
-            K.linear_topk(ws.xn, self.generator.w, self.generator.bias, ws.topk_part, candidates=ws.beam)
+            K.linear_topk(ws.xn, self.generator.w, self.generator.bias, ws.topk_part, candidates=candidates or ws.beam)
         else:
             self.generator(ws.xn, ws.logits)
 
@@ -605,17 +605,13 @@ class OrtEngine:
         st = ws.state
         st.reset(c.bos_token_id, c.pad_token_id)
         kind, alpha = _parse_penalty(opt.get("length_penalty", ""))
-        bad = opt.get("bad_endings_ix")      # remove_bad_endings (caption_model.py:161-168): token 0 may not follow these
         pen_col = int(opt.get("penalized_col", -1))  # suppress_UNK (:169-170)
-        bad_t = opt.get("_bad_t") if bad else None   # (device tensor made by decode() outside the graph capture)
+        bad_t = self._bad_endings(ws, opt)
         fused = (ws.topk_part is not None and float(opt.get("temperature", 1.0)) == 1.0 and not opt.get("decoding_constraint", 0)
                  and bad_t is None and pen_col < 0)
         for t in range(L):
             self._decode_step(ws, enc, t, st.anc[t & 1], fused_topk=fused)
-            sup = None
-            if bad_t is not None and t > 0:
-                # rows whose previous token (= the token just fed) is a bad ending: token 0 is suppressed at this step
-                sup = torch.where(torch.isin(st.tokens, bad_t), 0, -1).to(torch.int32)
+            sup = _suppress_bad(st, bad_t, t)
             if fused:
                 K.beam_step_partials(ws.topk_part, st, t, B=ws.B, beam=ws.beam, V=V, L=L, eos=c.eos_token_id, pad=c.pad_token_id,
                                      penalty_kind=kind, penalty_alpha=alpha)
@@ -623,6 +619,79 @@ class OrtEngine:
                 K.beam_step(ws.logits, st, t, B=ws.B, beam=ws.beam, V=V, L=L, eos=c.eos_token_id, pad=c.pad_token_id,
                             temperature=opt.get("temperature", 1.0), constraint=opt.get("decoding_constraint", 0),
                             penalty_kind=kind, penalty_alpha=alpha, suppress_tok=sup, penalized_col=pen_col)
+
+    def _bad_endings(self, ws, opt):
+        """remove_bad_endings (caption_model.py:161-168): the ids as a device tensor held by the workspace, made outside any
+        graph capture, so that a captured decode reads live memory on every replay (None when the option is off)."""
+        bad = opt.get("bad_endings_ix")
+        if not bad:
+            return None
+        ids = sorted(int(i) for i in bad)
+        if getattr(ws, "bad_ids", None) != ids:
+            ws.bad_ids, ws.bad_t = ids, torch.tensor(ids, dtype=torch.int32, device=self.dev)
+        return ws.bad_t
+
+    def _get_diverse_ws(self, B, N, G, bdash, slot):
+        """Diverse beam search: one decode workspace + BeamState per group (B*bdash rows each); the groups' seq ping-pong
+        buffers live in one int32 [G, 2, B*bdash, L] tensor, from which each group's beam step reads the earlier groups'
+        tokens (sc_beam_step_diverse)."""
+        key = (B, G * bdash, N, "diverse", G, slot)
+        dv = self._dec_ws.get(key)
+        if dv is not None:
+            return dv
+        L = self.cfg.max_seq_length
+        dv = type("DiverseWs", (), {})()
+        dv.B, dv.G, dv.bdash = B, G, bdash
+        dv.hist = torch.zeros(G, 2, B * bdash, L, dtype=torch.int32, device=self.dev)
+        dv.groups = []
+        for g in range(G):
+            ws = self._get_dec_ws(B, bdash, N, False, slot, tag=("diverse", G, g))
+            ws.state.seq = [dv.hist[g, 0], dv.hist[g, 1]]
+            dv.groups.append(ws)
+        dv.seq = torch.zeros(B, G * bdash, L, dtype=torch.int32, device=self.dev)
+        dv.lp = torch.zeros(B, G * bdash, L, device=self.dev)
+        dv.graph = None
+        dv.opt_key = None
+        self._dec_ws[key] = dv
+        return dv
+
+    def _diverse_body(self, dv, enc, opt):
+        """batch_beam_search with group_size G > 1 (caption_model.py:126-226): global step t = 0 .. L+G-2, group g decodes
+        and steps at its local step t - g while that lies in [0, L-1], groups in ascending order; finished beams stay per
+        group and are concatenated group by group (:221-225)."""
+        c = self.cfg
+        L, V = c.max_seq_length, c.vocab_size
+        G, bdash = dv.G, dv.bdash
+        _, _, lam = diverse_groups(opt)
+        kind, alpha = _parse_penalty(opt.get("length_penalty", ""))
+        pen_col = int(opt.get("penalized_col", -1))
+        bad_t = self._bad_endings(dv, opt)
+        temperature = float(opt.get("temperature", 1.0))
+        # fused generator + row pass: a group needs its bdash + g*bdash <= beam_size best raw candidates per row
+        fused = (all(ws.topk_part is not None for ws in dv.groups) and self._topk_ok(G * bdash) and temperature == 1.0
+                 and not opt.get("decoding_constraint", 0) and bad_t is None and pen_col < 0)
+        for ws in dv.groups:
+            ws.state.reset(c.bos_token_id, c.pad_token_id)
+        for t in range(L + G - 1):
+            for g in range(G):
+                tau = t - g
+                if not 0 <= tau <= L - 1:
+                    continue
+                ws = dv.groups[g]
+                st = ws.state
+                self._decode_step(ws, enc, tau, st.anc[tau & 1], fused_topk=fused, candidates=G * bdash)
+                div = (dv.hist, g, lam)
+                if fused:
+                    K.beam_step_partials(ws.topk_part, st, tau, B=dv.B, beam=bdash, V=V, L=L, eos=c.eos_token_id,
+                                         pad=c.pad_token_id, penalty_kind=kind, penalty_alpha=alpha, diverse=div)
+                else:
+                    K.beam_step(ws.logits, st, tau, B=dv.B, beam=bdash, V=V, L=L, eos=c.eos_token_id, pad=c.pad_token_id,
+                                temperature=temperature, constraint=opt.get("decoding_constraint", 0), penalty_kind=kind,
+                                penalty_alpha=alpha, suppress_tok=_suppress_bad(st, bad_t, tau), penalized_col=pen_col,
+                                diverse=div)
+        for g, ws in enumerate(dv.groups):
+            dv.seq[:, g * bdash:(g + 1) * bdash].copy_(ws.state.done_seq)
+            dv.lp[:, g * bdash:(g + 1) * bdash].copy_(ws.state.done_lp)
 
     def _greedy_body(self, ws, enc, opt):
         c = self.cfg
@@ -649,10 +718,9 @@ class OrtEngine:
         """Beam (beam_size > 1), greedy (beam_size == 1) or multinomial (num_random_sample > 0, models/transformer.py:
         507-561) decoding over an encoded batch.  Returns (seq int32 [B,b,L], lp [B,b,L]); b = num_random_sample when sampling.
         ``opt["sample_seed"]`` re-seeds the sampler (default: a counter), ``opt["sample_uniforms"]`` (fp32 [L, B*n], tests)
-        replaces the Philox draws."""
+        replaces the Philox draws.  ``group_size`` G > 1 with beam_size > 1: diverse beam search (``diversity_lambda``,
+        default 0.5), b = G * (beam_size // G) beams per image in group-major order."""
         beam = int(opt.get("beam_size", 1))
-        if opt.get("group_size", 1) != 1:
-            raise NotImplementedError("diverse beam search (group_size > 1) is out of scope (SURVEY.md section 2.1 #6)")
         n_rand = int(opt.get("num_random_sample", 0))
         if n_rand > 0:
             assert beam < 1, f"Beam size must be < 1, saw {beam}"  # transformer.py:509
@@ -678,22 +746,29 @@ class OrtEngine:
             return ws.state.seq.view(enc.B, n_rand, -1), ws.state.lp.view(enc.B, n_rand, -1)
         greedy = beam == 1
         assert beam <= self.cfg.vocab_size
-        ws = self._get_dec_ws(enc.B, beam, enc.N, greedy, enc.slot)
         opt_key = (id(enc), tuple(sorted((k, str(v)) for k, v in opt.items())))
-        if opt.get("bad_endings_ix"):
-            opt = dict(opt, _bad_t=torch.tensor(sorted(opt["bad_endings_ix"]), dtype=torch.int32, device=self.dev))
+        if not greedy and int(opt.get("group_size", 1)) > 1:
+            G, bdash, _ = diverse_groups(opt)
+            ws = self._get_diverse_ws(enc.B, enc.N, G, bdash, enc.slot)
+            self._run(ws, lambda: self._diverse_body(ws, enc, opt), opt_key)
+            return ws.seq, ws.lp
+        ws = self._get_dec_ws(enc.B, beam, enc.N, greedy, enc.slot)
         body = (lambda: self._greedy_body(ws, enc, opt)) if greedy else (lambda: self._beam_body(ws, enc, opt))
-        if not self.use_graphs:
-            body()
-        else:
-            if ws.graph is None or ws.opt_key != opt_key:
-                self._warm_and_capture(ws, body)
-                ws.opt_key = opt_key
-            ws.graph.replay()
+        self._run(ws, body, opt_key)
         st = ws.state
         if greedy:
             return st.seq.view(enc.B, 1, -1), st.lp.view(enc.B, 1, -1)
         return st.done_seq, st.done_lp
+
+    def _run(self, ws, body, opt_key):
+        """Runs a decode body eagerly, or as the workspace's CUDA graph (captured again when the options change)."""
+        if not self.use_graphs:
+            body()
+            return
+        if ws.graph is None or ws.opt_key != opt_key:
+            self._warm_and_capture(ws, body)
+            ws.opt_key = opt_key
+        ws.graph.replay()
 
     def teacher_force(self, enc, tokens, beam=1, out=None):
         """Incremental (KV-cached) decoding along GIVEN token paths: row r = image r // beam feeds BOS, tokens[r, 0], ...,
@@ -789,50 +864,65 @@ class OrtEngine:
         return out, caches
 
     def beam_search_stepwise(self, init_state, init_logprobs, args, opt, get_logprobs_state):
-        """``batch_beam_search`` (caption_model.py:30-226, group_size 1) driven step by step: sc_beam_step ranks the b*V
-        candidates, keeps the beam / finished-beam state on the device and yields the parent rows; the model state is reordered
-        with ``state[i][:, parents]`` and advanced through ``get_logprobs_state`` - the reference's own control flow.
-        Returns done_beams [B][beam] dicts."""
+        """``batch_beam_search`` (caption_model.py:30-226) driven step by step: sc_beam_step ranks the b*V candidates, keeps
+        the beam / finished-beam state on the device and yields the parent rows; the model state is reordered with
+        ``state[i][:, parents]`` and advanced through ``get_logprobs_state`` - the reference's own control flow.  With
+        group_size G > 1 (diverse beam search) every group has its own state list cloned from ``init_state``, its share of
+        ``args`` (row r of the B*b repeated rows goes to group r % G, model_utils.split_tensors) and its own staggered
+        steps (sc_beam_step_diverse).  Returns done_beams [B][G*bdash] dicts {seq, logps, unaug_p, p}, group-major."""
         c = self.cfg
         beam = int(opt.get("beam_size", 10))
+        G, bdash, lam = diverse_groups(opt) if int(opt.get("group_size", 1)) > 1 else (1, beam, 0.0)
         L, V = c.max_seq_length, c.vocab_size
         B = init_logprobs.shape[0]
-        st = BeamState(B, beam, L, self.dev)
-        st.reset(c.bos_token_id, c.pad_token_id)
+        hist = torch.zeros(G, 2, B * bdash, L, dtype=torch.int32, device=self.dev) if G > 1 else None
+        sts = []
+        for g in range(G):
+            st = BeamState(B, bdash, L, self.dev)
+            if hist is not None:
+                st.seq = [hist[g, 0], hist[g, 1]]
+            st.reset(c.bos_token_id, c.pad_token_id)
+            sts.append(st)
         kind, alpha = _parse_penalty(opt.get("length_penalty", ""))
         bad = opt.get("bad_endings_ix")
         bad_t = torch.tensor(sorted(bad), dtype=torch.int32, device=self.dev) if bad else None
         pen_col = int(opt.get("penalized_col", -1))
         temperature = float(opt.get("temperature", 1.0))
-        logits = torch.zeros(B * beam, V, device=self.dev)
-        logits.view(B, beam, V)[:, 0] = init_logprobs.float()   # t = 0: only beam 0 of an image is expanded
-        state = [x.clone() for x in init_state]
-        for t in range(L):
-            sup = None
-            if bad_t is not None and t > 0:
-                sup = torch.where(torch.isin(st.tokens, bad_t), 0, -1).to(torch.int32)
-            K.beam_step(logits, st, t, B=B, beam=beam, V=V, L=L, eos=c.eos_token_id, pad=c.pad_token_id, temperature=temperature,
-                        constraint=opt.get("decoding_constraint", 0), penalty_kind=kind, penalty_alpha=alpha, suppress_tok=sup,
-                        penalized_col=pen_col)
-            parents = st.anc[(t + 1) & 1][:, t].long()          # row each new beam descends from (b*beam + parent)
-            if t == 0:
-                parents = parents // beam                        # the first state holds one row per image
-            state = [x[:, parents] for x in state]
-            it = st.tokens.long()
-            logprobs, state = get_logprobs_state(it, *(list(args) + [state]))
-            logits = logprobs.contiguous()                       # (sc_beam_step re-normalises: log_softmax is idempotent)
-        done_seq, done_lp, done_p = st.done_seq.long().cpu(), st.done_lp.cpu(), st.done_p.cpu()
-        out = []
-        for b in range(B):
-            beams = []
-            for v in range(beam):
-                n = int((done_seq[b, v] != c.pad_token_id).sum())
-                eos = (done_seq[b, v] == c.eos_token_id).nonzero()
-                if eos.numel():
-                    n = int(eos[0]) + 1
-                beams.append({"seq": done_seq[b, v, :n].to(self.dev), "logps": done_lp[b, v, :n].to(self.dev),
-                              "unaug_p": float(done_lp[b, v, :n].sum()), "p": float(done_p[b, v])})
-            out.append(beams)
+        args = list(args)
+        group_args = [[None if a is None else a.reshape(a.shape[0] // G, G, *a.shape[1:])[:, g] for a in args] for g in range(G)]
+        logits, state = [], []
+        for g in range(G):
+            lg = torch.zeros(B * bdash, V, device=self.dev)
+            lg.view(B, bdash, V)[:, 0] = init_logprobs.float()   # local step 0: only beam 0 of an image is expanded
+            logits.append(lg)
+            state.append([x.clone() for x in init_state])
+        for t in range(L + G - 1):
+            for g in range(G):
+                tau = t - g
+                if not 0 <= tau <= L - 1:
+                    continue
+                st = sts[g]
+                K.beam_step(logits[g], st, tau, B=B, beam=bdash, V=V, L=L, eos=c.eos_token_id, pad=c.pad_token_id,
+                            temperature=temperature, constraint=opt.get("decoding_constraint", 0), penalty_kind=kind,
+                            penalty_alpha=alpha, suppress_tok=_suppress_bad(st, bad_t, tau), penalized_col=pen_col,
+                            diverse=None if hist is None else (hist, g, lam))
+                parents = st.anc[(tau + 1) & 1][:, tau].long()      # row each new beam descends from (b*bdash + parent)
+                if tau == 0:
+                    parents = parents // bdash                       # the first state holds one row per image
+                state[g] = [x[:, parents] for x in state[g]]
+                logprobs, state[g] = get_logprobs_state(st.tokens.long(), *(group_args[g] + [state[g]]))
+                logits[g] = logprobs.contiguous()                    # (sc_beam_step re-normalises: log_softmax is idempotent)
+        out = [[] for _ in range(B)]
+        for st in sts:
+            done_seq, done_lp, done_p = st.done_seq.long().cpu(), st.done_lp.cpu(), st.done_p.cpu()
+            for b in range(B):
+                for v in range(bdash):
+                    n = int((done_seq[b, v] != c.pad_token_id).sum())
+                    eos = (done_seq[b, v] == c.eos_token_id).nonzero()
+                    if eos.numel():
+                        n = int(eos[0]) + 1
+                    out[b].append({"seq": done_seq[b, v, :n].to(self.dev), "logps": done_lp[b, v, :n].to(self.dev),
+                                   "unaug_p": float(done_lp[b, v, :n].sum()), "p": float(done_p[b, v])})
         return out
 
     # ---- batch pipelining: slot s owns a stream + workspaces + graphs; batches in different slots overlap on the GPU
@@ -896,6 +986,31 @@ def decode_grid_hint(rows, n_out, d_model, dec_ctas):
     target = dec_ctas[1] if n_out <= d_model else dec_ctas[0]
     tpc = -(-tiles // max(1, target))
     return min(tpc, 200) * 10000000 + 3256 if tpc >= 2 else 0
+
+
+MAX_GROUP_BEAMS = 8  # beams per group: the beam-step kernel's per-image limit
+
+
+def diverse_groups(opt):
+    """(G, bdash, diversity_lambda) of a diverse beam search (caption_model.py:114-123: bdash = beam_size // group_size beams
+    per group, diversity_lambda default 0.5).  ValueError when a group would hold no beam or more than the kernel serves."""
+    beam, G = int(opt.get("beam_size", 10)), int(opt.get("group_size", 1))
+    bdash = beam // G if G > 0 else 0
+    if bdash < 1 or bdash > MAX_GROUP_BEAMS:
+        raise ValueError(f"diverse beam search: beam_size={beam} // group_size={G} = {bdash} beams per group; "
+                         f"it must lie in [1, {MAX_GROUP_BEAMS}]")
+    if (G - 1) * bdash > 256:
+        raise ValueError(f"diverse beam search: (group_size - 1) * (beam_size // group_size) = {(G - 1) * bdash} "
+                         f"earlier-group beams; at most 256")
+    return G, bdash, float(opt.get("diversity_lambda", 0.5))
+
+
+def _suppress_bad(st, bad_t, t):
+    """remove_bad_endings at step t > 0: int32 [rows], 0 where the row's previous token (the token just fed) is a bad ending
+    (token 0 may not follow it), -1 elsewhere; None when the option is off."""
+    if bad_t is None or t == 0:
+        return None
+    return torch.where(torch.isin(st.tokens, bad_t), 0, -1).to(torch.int32)
 
 
 def _parse_penalty(s):

@@ -375,17 +375,28 @@ def cross_attn_step(q, mem_k, mem_v, att_mask, out, *, B, beam, N, D, h, ldq, ld
 
 
 def beam_step(logits, st, t, *, B, beam, V, L, eos, pad, temperature=1.0, constraint=0, penalty_kind=0, penalty_alpha=0.0,
-              suppress_tok=None, penalized_col=-1):
+              suppress_tok=None, penalized_col=-1, diverse=None):
     """``st``: BeamState.  Reads buffers ``t % 2`` and writes ``(t+1) % 2``.  ``suppress_tok`` (int32 [B*beam], -1 = none):
     per-row token that cannot be chosen at this step (remove_bad_endings); ``penalized_col``: column whose log-prob is
-    lowered by 1000 (suppress_UNK)."""
+    lowered by 1000 (suppress_UNK).  ``diverse = (group_seq, group, diversity_lambda)``: the diverse-beam step of group
+    ``group`` at its local step ``t`` (sc_beam_step_diverse; group_seq int32 [G, 2, B*beam, L] holds every group's seq)."""
     i, o = t & 1, (t + 1) & 1
     assert suppress_tok is None or (suppress_tok.dtype == torch.int32 and suppress_tok.numel() == B * beam)
-    lib.call("sc_beam_step", lib.ptr(logits), B, beam, V, L, t, eos, pad, float(temperature), int(constraint),
-             int(penalty_kind), float(penalty_alpha), lib.ptr(suppress_tok), int(penalized_col), lib.ptr(st.seq[i]), lib.ptr(st.seq[o]), lib.ptr(st.lp[i]),
-             lib.ptr(st.lp[o]), lib.ptr(st.sum), lib.ptr(st.anc[i]), lib.ptr(st.anc[o]), lib.ptr(st.tokens),
-             lib.ptr(st.done_seq), lib.ptr(st.done_lp), lib.ptr(st.done_p), lib.ptr(st.done_count), lib.ptr(st.ws),
-             st.ws.numel(), lib.stream())
+    head = [lib.ptr(logits), B, beam, V, L, t, eos, pad, float(temperature), int(constraint), int(penalty_kind), float(penalty_alpha),
+            lib.ptr(suppress_tok), int(penalized_col)]
+    tail = [lib.ptr(st.seq[i]), lib.ptr(st.seq[o]), lib.ptr(st.lp[i]), lib.ptr(st.lp[o]), lib.ptr(st.sum), lib.ptr(st.anc[i]),
+            lib.ptr(st.anc[o]), lib.ptr(st.tokens), lib.ptr(st.done_seq), lib.ptr(st.done_lp), lib.ptr(st.done_p),
+            lib.ptr(st.done_count), lib.ptr(st.ws), st.ws.numel(), lib.stream()]
+    if diverse is None:
+        lib.call("sc_beam_step", *head, *tail)
+    else:
+        lib.call("sc_beam_step_diverse", *head, *_diverse_args(diverse, B, beam, L), *tail)
+
+
+def _diverse_args(diverse, B, beam, L):
+    hist, group, lam = diverse
+    assert hist.dtype == torch.int32 and hist.is_contiguous() and tuple(hist.shape[1:]) == (2, B * beam, L) and group < hist.shape[0]
+    return [lib.ptr(hist), int(group), float(lam)]
 
 
 def linear_hmask(x, w, h, out, *, scale=1.0, colsum=None):
@@ -419,13 +430,18 @@ def linear_topk(x, w, bias, partials, candidates=5):
     return partials
 
 
-def beam_step_partials(partials, st, t, *, B, beam, V, L, eos, pad, penalty_kind=0, penalty_alpha=0.0):
-    """Beam step from sc_linear_topk records (temperature 1, no decoding constraint, beam <= 5)."""
+def beam_step_partials(partials, st, t, *, B, beam, V, L, eos, pad, penalty_kind=0, penalty_alpha=0.0, diverse=None):
+    """Beam step from sc_linear_topk records (temperature 1, no decoding constraint, beam <= 5).  ``diverse``: as in
+    ``beam_step`` (the records must hold (group + 1) * beam candidates per row)."""
     i, o = t & 1, (t + 1) & 1
-    lib.call("sc_beam_step_partials", lib.ptr(partials), partials.shape[1], B, beam, V, L, t, eos, pad, int(penalty_kind),
-             float(penalty_alpha), lib.ptr(st.seq[i]), lib.ptr(st.seq[o]), lib.ptr(st.lp[i]), lib.ptr(st.lp[o]), lib.ptr(st.sum),
-             lib.ptr(st.anc[i]), lib.ptr(st.anc[o]), lib.ptr(st.tokens), lib.ptr(st.done_seq), lib.ptr(st.done_lp),
-             lib.ptr(st.done_p), lib.ptr(st.done_count), lib.ptr(st.ws), st.ws.numel(), lib.stream())
+    head = [lib.ptr(partials), partials.shape[1], B, beam, V, L, t, eos, pad, int(penalty_kind), float(penalty_alpha)]
+    tail = [lib.ptr(st.seq[i]), lib.ptr(st.seq[o]), lib.ptr(st.lp[i]), lib.ptr(st.lp[o]), lib.ptr(st.sum), lib.ptr(st.anc[i]),
+            lib.ptr(st.anc[o]), lib.ptr(st.tokens), lib.ptr(st.done_seq), lib.ptr(st.done_lp), lib.ptr(st.done_p),
+            lib.ptr(st.done_count), lib.ptr(st.ws), st.ws.numel(), lib.stream()]
+    if diverse is None:
+        lib.call("sc_beam_step_partials", *head, *tail)
+    else:
+        lib.call("sc_beam_step_partials_diverse", *head, *_diverse_args(diverse, B, beam, L), *tail)
 
 
 def beam_step_workspace_bytes(B, beam):

@@ -44,6 +44,10 @@ SIGNATURES = {
     "sc_linear_topk_parts": [_i],
     "sc_linear_topk": [_p, _p, _p, _i, _i, _i, _p, _i, _p],
     "sc_beam_step_partials": [_p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _f, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p],
+    "sc_beam_step_diverse": [_p, _i, _i, _i, _i, _i, _i, _i, _f, _i, _i, _f, _p, _i, _p, _i, _f, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p,
+                             _p, _p, _p, _sz, _p],
+    "sc_beam_step_partials_diverse": [_p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _f, _p, _i, _f, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p,
+                                      _p, _p, _p, _sz, _p],
     "sc_greedy_step": [_p, _i, _i, _i, _i, _i, _i, _p, _p, _p, _p, _p, _p],
     "sc_sample_step": [_p, _i, _i, _i, _i, _i, _i, _f, _p, _u64, _p, _p, _p, _p, _p, _p],
     "sc_cache_reorder": [_p, _p, _p, _l, _l, _p],

@@ -460,7 +460,6 @@ class _OrtBase(nn.Module):
         self._engine_key = None
         self._trainer = None
         self._trainer_key = None
-        self._step_t = 0
 
     def make_model(self, mask, dropout):
         c = self.cfg
@@ -593,26 +592,31 @@ class _OrtBase(nn.Module):
     @torch.no_grad()
     def get_logprobs_state(self, it, memory, mask, state):
         """One decoding step (relation_transformer.py:374-387): ``it`` [R] tokens, ``memory`` [R, N, d] encoder output,
-        ``mask`` [R, 1, N]; ``state`` None (first step) or the list returned by the previous call - [ys[None]] followed, per
-        unique decoder layer, by self K [slots, R, d], self V, and the cross K|V [1, R, N*ld] of the row's image, all with the
-        row dimension at dim 1 so that ``state[i][:, ix]`` reorders beams exactly as caption_model.py:106-110 does.
+        ``mask`` [R, 1, N]; ``state`` None (first step) or the list returned by the previous call - the tokens fed so far
+        [1, R, t] (ys[None]) followed, per unique decoder layer, by self K [slots, R, d], self V, and the cross K|V
+        [1, R, N*ld] of the row's image, all with the row dimension at dim 1 so that ``state[i][:, ix]`` reorders beams
+        exactly as caption_model.py:106-110 does.  The decode position is the length of that token history, so several
+        searches (the groups of a diverse beam search) may advance their own states in any interleaving.
         Returns (log-probs fp32 [R, V], new state)."""
         eng = self._get_engine() if (state is None or self._engine is None) else self._engine
+        ys = it.reshape(1, -1, 1)
         if state is None:
-            self._step_t = 0
-        caches = None if state is None else state[1:]
-        logprobs, caches = eng.logprobs_step(it, memory, mask, caches, self._step_t)
-        self._step_t += 1
-        return logprobs, [it.reshape(1, -1, 1)] + caches
+            t, caches = 0, None
+        else:
+            t, caches, prev = state[0].shape[-1], state[1:], state[0]
+            if prev.shape[1] != ys.shape[1]:  # first beam step: rows repeated `beam` times (transformer.py:240-252)
+                prev = prev.repeat_interleave(ys.shape[1] // prev.shape[1], 1)
+            ys = torch.cat([prev.to(ys.dtype), ys], -1)
+        logprobs, caches = eng.logprobs_step(it, memory, mask, caches, t)
+        return logprobs, [ys] + caches
 
     @torch.no_grad()
     def batch_beam_search(self, init_state, init_logprobs, *args, **kwargs):
-        """caption_model.py:30-226 with group_size 1: the per-step candidate ranking, beam bookkeeping and finished-beam
-        handling run in sc_beam_step on device state; ``get_logprobs_state`` advances the model.  Returns ``done_beams``:
-        per image a list of ``beam_size`` dicts {seq, logps (chosen-token log-probs [len]), unaug_p, p}, best first."""
+        """caption_model.py:30-226: the per-step candidate ranking, beam bookkeeping and finished-beam handling run in
+        sc_beam_step (sc_beam_step_diverse for group_size > 1) on device state; ``get_logprobs_state`` advances the model.
+        Returns ``done_beams``: per image a list of dicts {seq, logps (chosen-token log-probs [len]), unaug_p, p} - beam_size
+        of them best first, or with group_size G > 1 each group's beam_size // G best, groups in order."""
         opt = self._decode_opts(kwargs["opt"])
-        if opt.get("group_size", 1) != 1:
-            raise NotImplementedError("diverse beam search (group_size > 1) is out of scope (SURVEY.md section 2.1 #6)")
         eng = self._engine if self._engine is not None else self._get_engine()
         self.done_beams = eng.beam_search_stepwise(init_state, init_logprobs, list(args), opt, self.get_logprobs_state)
         return self.done_beams
