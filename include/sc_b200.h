@@ -345,6 +345,16 @@ int sc_ciderd_score(const int* hyp, int H, int L, const int* hyp_img, int eos, i
                     const double* df_log, long n_df, double ref_len, double sigma, const long* img_ref_off, const long* ref_ng_off,
                     const unsigned long long* ref_keys, const double* ref_vec, const double* ref_norm, const int* ref_length,
                     double* out, sc_stream_t stream);
+/* SCST rollout -> teacher-forcing inputs of the training step (utils/training.py:239-255 with RewardCriterion, utils/losses.py:10-29),
+ * one launch.  seq int32 [R = B*S, L]: the rollout (S samples per image, rows image-major).  score float64 [R]: the samples'
+ * CIDEr-D; base_score float64 [B] (the greedy baseline, one per image) or NULL (each sample's baseline is the mean of its image's
+ * other S - 1 samples, S >= 2).  reward[r] = cider_weight * (score[r] - baseline[r]), rounded to fp32.  Writes [R, L]:
+ * tokens = [bos, s_0 .. s_{L-2}], targets = s, key_valid = (tokens != pad), tok_w = reward * mask with mask[r, 0] = 1,
+ * mask[r, t] = (s_{t-1} != pad); mask_sum (optional) = sum of mask; inv_norm = 1 / (norm_in ? *norm_in : sum of mask)
+ * (norm_in: the data-parallel global count); mean_reward (optional) = mean of reward over the R rows. */
+int sc_scst_targets(const int* seq, int R, int L, int S, const double* score, const double* base_score, float cider_weight,
+                    int bos, int pad, int* tokens, int* targets, float* tok_w, float* key_valid, float* mask_sum, float* inv_norm,
+                    const float* norm_in, float* mean_reward, sc_stream_t stream);
 
 /* teacher-forcing attention with saved probabilities + backward (decoder self: causal_T = T; cross: groups = images with
  * S*T query rows; encoder box attention: additive bias): transformer.py:230-295, relation_transformer.py:258-293 */

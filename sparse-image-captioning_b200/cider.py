@@ -63,7 +63,8 @@ class CiderD:
         return self
 
     def set_refs(self, refs_per_image: Sequence[Sequence[Sequence[int]]]) -> None:
-        """tf-idf vectors / norms / lengths of the reference captions of a batch (counts2vec, ciderD_scorer.py:134-160)."""
+        """tf-idf vectors / norms / lengths of the reference captions (counts2vec, ciderD_scorer.py:134-160), per image: of a batch, or
+        of a whole split once (then ``score`` / ``scst_reward`` / ``scst_step`` take dataset image indices)."""
         img_off, ng_off, keys, vecs, norms, lens = [0], [0], [], [], [], []
         for refs in refs_per_image:
             for ref in refs:
@@ -107,15 +108,19 @@ class CiderD:
                  lib.ptr(r["norm"]), lib.ptr(r["length"]), lib.ptr(out), lib.stream())
         return out
 
-    def scst_reward(self, sample_seq: torch.Tensor, baseline_seq: Optional[torch.Tensor] = None, cider_weight: float = 1.0):
+    def scst_reward(self, sample_seq: torch.Tensor, baseline_seq: Optional[torch.Tensor] = None, cider_weight: float = 1.0,
+                    image_ids: Optional[torch.Tensor] = None):
         """CaptionScorer.__call__ (scorers.py:47-114): ``sample_seq`` [B, n, L] rollouts, ``baseline_seq`` [B, 1, L] greedy captions or
-        None (then each sample's baseline is the mean score of the image's OTHER samples).  Returns (sc_sample, sc_baseline), float64
-        [B * n] on the device; the SCST reward is their difference (training.py:252)."""
+        None (then each sample's baseline is the mean score of the image's OTHER samples).  ``image_ids`` [B]: the images' indices
+        into the references given to ``set_refs`` (default 0 .. B-1): ``set_refs`` can then take a whole split once instead of
+        every batch.  Returns (sc_sample, sc_baseline), float64 [B * n] on the device; the SCST reward is their difference
+        (training.py:252)."""
         B, n, L = sample_seq.shape
-        img = torch.arange(B, device=self.dev).repeat_interleave(n)
+        ids = torch.arange(B, device=self.dev) if image_ids is None else torch.as_tensor(image_ids).to(self.dev)
+        img = ids.repeat_interleave(n)
         sc_sample = self.score(sample_seq.reshape(B * n, L), img) * cider_weight
         if baseline_seq is not None:
-            sc_b = self.score(baseline_seq.reshape(B, -1)[:, :L], torch.arange(B, device=self.dev)) * cider_weight
+            sc_b = self.score(baseline_seq.reshape(B, -1)[:, :L], ids) * cider_weight
             return sc_sample, sc_b.repeat_interleave(n)
         tot = sc_sample.view(B, n).sum(-1)
         return sc_sample, (tot.repeat_interleave(n) - sc_sample) / (n - 1)

@@ -132,9 +132,84 @@ __global__ void __launch_bounds__(kThreads) ciderd_kernel(const CiderArgs a) {
   }
 }
 
+// SCST rollout -> teacher-forcing inputs of the training step (utils/training.py:239-255, RewardCriterion utils/losses.py:10-29).
+// One CTA: the token count and the mean reward are block reductions in a fixed order (bit-reproducible, no atomics), and
+// inv_norm can be written by the same launch that counts.
+constexpr int kTargetThreads = 1024;
+
+__device__ __forceinline__ double scst_reward(const double* score, const double* base, int r, int S, float w) {
+  double b;
+  if (base != nullptr) {
+    b = base[r / S];
+  } else {  // mean of the image's OTHER samples (scst/scorers.py:100-106): (sum - own) / (S - 1), summed in sample order
+    const int r0 = r - r % S;
+    double tot = 0.0;
+    for (int j = 0; j < S; ++j) tot += score[r0 + j];
+    b = (tot - score[r]) / (double)(S - 1);
+  }
+  return (double)w * (score[r] - b);
+}
+
+template <typename T>
+__device__ T block_sum(T v, T* red) {
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  if (lane == 0) red[warp] = v;
+  __syncthreads();
+  T s = T(0);
+  if (threadIdx.x == 0) {
+    for (int i = 0; i < (int)(blockDim.x >> 5); ++i) s += red[i];
+  }
+  __syncthreads();
+  return s;   // valid in thread 0
+}
+
+__global__ void __launch_bounds__(kTargetThreads) scst_targets_kernel(
+    const int* __restrict__ seq, int R, int L, int S, const double* __restrict__ score, const double* __restrict__ base,
+    float cider_weight, int bos, int pad, int* __restrict__ tokens, int* __restrict__ targets, float* __restrict__ tok_w,
+    float* __restrict__ key_valid, float* __restrict__ mask_sum, float* __restrict__ inv_norm, const float* __restrict__ norm_in,
+    float* __restrict__ mean_reward) {
+  __shared__ long long red_i[kTargetThreads / 32];
+  __shared__ double red_d[kTargetThreads / 32];
+  long long count = 0;
+  const long long n = (long long)R * L;
+  for (long long e = threadIdx.x; e < n; e += blockDim.x) {
+    const int r = (int)(e / L), t = (int)(e % L);
+    const int* s = seq + (size_t)r * L;
+    const int prev = t == 0 ? bos : s[t - 1];        // tokens = [BOS, s_0 .. s_{L-2}]
+    const int m = (t == 0 || prev != pad) ? 1 : 0;   // RewardCriterion's mask, shifted right by one, first column 1
+    tokens[e] = prev;
+    targets[e] = s[t];
+    key_valid[e] = prev != pad ? 1.f : 0.f;
+    tok_w[e] = m ? (float)scst_reward(score, base, r, S, cider_weight) : 0.f;   // (reward -> fp32 first, like .float())
+    count += m;
+  }
+  double rsum = 0.0;
+  for (int r = threadIdx.x; r < R; r += blockDim.x) rsum += scst_reward(score, base, r, S, cider_weight);
+  const long long c = block_sum(count, red_i);
+  const double rs = block_sum(rsum, red_d);
+  if (threadIdx.x == 0) {
+    if (mask_sum) *mask_sum = (float)c;
+    *inv_norm = 1.0f / (norm_in ? *norm_in : (float)c);
+    if (mean_reward) *mean_reward = (float)(rs / (double)R);
+  }
+}
+
 }  // namespace
 
 extern "C" {
+
+int sc_scst_targets(const int* seq, int R, int L, int S, const double* score, const double* base_score, float cider_weight,
+                    int bos, int pad, int* tokens, int* targets, float* tok_w, float* key_valid, float* mask_sum, float* inv_norm,
+                    const float* norm_in, float* mean_reward, cudaStream_t stream) {
+  SC_CHECK(R > 0 && L > 0 && S > 0 && R % S == 0, SC_ERR_SHAPE, "sc_scst_targets: R=%d L=%d S=%d", R, L, S);
+  SC_CHECK(base_score != nullptr || S >= 2, SC_ERR_SHAPE, "sc_scst_targets: the mean-of-others baseline needs S >= 2 samples (S=%d)", S);
+  SC_CHECK(seq && score && tokens && targets && tok_w && key_valid && inv_norm, SC_ERR_SHAPE, "sc_scst_targets: null argument");
+  scst_targets_kernel<<<1, kTargetThreads, 0, stream>>>(seq, R, L, S, score, base_score, cider_weight, bos, pad, tokens, targets,
+                                                        tok_w, key_valid, mask_sum, inv_norm, norm_in, mean_reward);
+  SC_LAUNCH_CHECK("sc_scst_targets");
+  return SC_OK;
+}
 
 int sc_ciderd_score(const int* hyp, int H, int L, const int* hyp_img, int eos, int pad, const unsigned long long* df_keys,
                     const double* df_log, long n_df, double ref_len, double sigma, const long* img_ref_off, const long* ref_ng_off,

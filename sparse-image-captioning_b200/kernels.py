@@ -607,6 +607,20 @@ def logsoftmax_nll(logits, target=None, weight=None, inv_norm=None, loss_sum=Non
              lib.stream())
 
 
+def scst_targets(seq, score, base_score, *, S, cider_weight, bos, pad, tokens, targets, tok_w, key_valid, inv_norm, mask_sum=None,
+                 norm_in=None, mean_reward=None):
+    """SCST rollout seq int32 [R, L] + CIDEr-D scores float64 [R] (+ greedy baseline scores float64 [R // S], or None: mean of
+    the image's other samples) -> the training step's tokens / targets / tok_w / key_valid [R * L] and inv_norm (sc_scst_targets)."""
+    R, L = seq.shape
+    assert seq.dtype == torch.int32 and seq.is_contiguous() and score.dtype == torch.float64 and score.numel() == R
+    assert base_score is None or (base_score.dtype == torch.float64 and base_score.numel() == R // S)
+    for t, dt in ((tokens, torch.int32), (targets, torch.int32), (tok_w, torch.float32), (key_valid, torch.float32)):
+        assert t.dtype == dt and t.numel() == R * L and t.is_contiguous()
+    lib.call("sc_scst_targets", lib.ptr(seq), R, L, int(S), lib.ptr(score), lib.ptr(base_score), float(cider_weight), int(bos), int(pad),
+             lib.ptr(tokens), lib.ptr(targets), lib.ptr(tok_w), lib.ptr(key_valid), lib.ptr(mask_sum), lib.ptr(inv_norm),
+             lib.ptr(norm_in), lib.ptr(mean_reward), lib.stream())
+
+
 def embedding_bwd(tokens, dy, dtable, scale):
     rows, D = dy.shape
     lib.call("sc_embedding_bwd", lib.ptr(tokens), lib.ptr(dy), lib.ptr(dtable), rows, D, dtable.shape[0], float(scale), lib.stream())

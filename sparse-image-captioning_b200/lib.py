@@ -78,6 +78,7 @@ SIGNATURES = {
     "sc_log_clamp": [_p, _p, _p, _sz, _f, _p],
     "sc_logsoftmax_bwd": [_p, _p, _p, _i, _i, _p],
     "sc_ciderd_score": [_p, _i, _i, _p, _i, _i, _p, _p, _l, C.c_double, C.c_double, _p, _p, _p, _p, _p, _p, _p, _p],
+    "sc_scst_targets": [_p, _i, _i, _i, _p, _p, _f, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p],
 }
 
 _lib = None

@@ -24,6 +24,34 @@ def _round_up(n, m):
     return (n + m - 1) // m * m
 
 
+def scst_samples(opt, baseline, bleu_weight=0.0):
+    """Captions per image S of an SCST rollout ``opt`` (beam_size b, G * (b // G) for diverse beam search, or num_random_sample);
+    ValueError for the options the device step does not support."""
+    from .engine import diverse_groups
+    if baseline not in ("greedy", "sample"):
+        raise ValueError(f"SCST baseline must be 'greedy' or 'sample', got {baseline!r}")
+    if bleu_weight:
+        raise ValueError("bleu_weight > 0: the BLEU scorer does not run on the device (CIDEr-D only)")
+    if float(opt.get("temperature", 1.0)) != 1.0:
+        raise ValueError("SCST re-scores the plain log-softmax of the sampled tokens: temperature must be 1")
+    beam, n_rand = int(opt.get("beam_size", 1)), int(opt.get("num_random_sample", 0))
+    if n_rand > 0:
+        assert beam < 1, f"Beam size must be < 1, saw {beam}"  # transformer.py:509
+        S = n_rand
+    elif beam == 1:
+        raise ValueError("beam_size == 1 is the greedy baseline, not a rollout: use beam_size > 1 or num_random_sample > 0")
+    elif beam < 1:
+        raise ValueError(f"SCST rollout needs beam_size > 1 or num_random_sample > 0 (got beam_size={beam})")
+    else:
+        S = beam
+        if int(opt.get("group_size", 1)) > 1:
+            G, bdash, _ = diverse_groups(opt)
+            S = G * bdash
+    if baseline == "sample" and S < 2:
+        raise ValueError(f"baseline='sample' averages the image's other samples: it needs at least 2 per image (got {S})")
+    return S
+
+
 class OrtTrainer:
     def __init__(self, state_dict: Dict[str, torch.Tensor], cfg: ModelCfg, *, mask_type: Optional[str] = "supermask",
                  precision="bf16", device="cuda", dropout=0.1 / 3, drop_prob_src=0.5, bypass_sigmoid_grad=False, seed=0,
@@ -169,6 +197,9 @@ class OrtTrainer:
         # decoder-side Adam on its own stream underneath the encoder backward: measured slower (5.42 vs 5.35 ms/step, the
         # HBM-bound update slows the backward kernels more than it hides) - off unless SC_OPT_OVERLAP=1
         self.overlap_opt = os.environ.get("SC_OPT_OVERLAP") == "1"
+        # SCST step in progress: its masks were applied before the rollouts (scst_step), the forward must reuse that sample
+        self._scst = False
+        self._rollout = self._baseline = None
 
     # ---------------------------------------------------------------------------------------------------------
     def _group(self, table, first, count):
@@ -533,7 +564,7 @@ class OrtTrainer:
         trig = not c.no_box_trigonometric_embedding
         if ws.att_a is not ws.att_in:
             K.cast_bf16(ws.att_in, out=ws.att_a)
-        if self.adt == torch.bfloat16 and self.premask and self.training:
+        if self.adt == torch.bfloat16 and self.premask and self.training and not self._scst:
             self._premask_all()
         self._lin("att_embed.0.weight", ws.att_a, ws.xe[0], relu=True, p=self.p_src, site=1)
         if ws.att_mask is not None:
@@ -994,7 +1025,8 @@ class OrtTrainer:
         self._dyn_dev.copy_(self._dyn_host, non_blocking=True)
 
     def _graph_body(self, ws, part, opt):
-        self._wm_step = {}  # every body (eager warm-up, capture) re-applies the masks
+        # every body (eager warm-up, capture) re-applies the masks - except an SCST body, whose masks the rollout already used
+        self._wm_step = {key: (self.step_id, self.training) for key in self._premask_keys()} if self._scst else {}
         if part == "all" and self.overlap_opt:
             # the decoder-side half of the optimizer (64 % of the parameters) runs on its own stream underneath the encoder's
             # backward: its gradients are final after phase 1 and nothing the remaining phases read is touched
@@ -1037,7 +1069,7 @@ class OrtTrainer:
                 h.wait()
 
     def _run_graphed(self, ws, part, opt):
-        key = (part, tuple(sorted((k, float(v)) for k, v in opt.items() if k in ("clip", "eps", "mask_eps", "weight_decay",
+        key = (part, self._scst, tuple(sorted((k, float(v)) for k, v in opt.items() if k in ("clip", "eps", "mask_eps", "weight_decay",
                                                                                 "grad_scale", "sparsity_target"))))
         graphs = ws.__dict__.setdefault("graphs", {})
         if key not in graphs:
@@ -1085,6 +1117,12 @@ class OrtTrainer:
             return ws.loss_sum * ws.inv_norm
         if self.use_graph and self.training:
             self._upload_step(lr=lr, **opt)
+        return self._fwd_bwd_opt(ws, lr, all_reduce, opt)
+
+    def _fwd_bwd_opt(self, ws, lr, all_reduce, opt):
+        """Forward, backward (+ bucketed gradient exchange) and optimizer of a loaded workspace; graph mode expects
+        ``_upload_step`` to have run for this step."""
+        if self.use_graph and self.training:
             opt = dict(opt, lr=lr)
             if all_reduce is None:
                 self._run_graphed(ws, "all", opt)
@@ -1115,6 +1153,162 @@ class OrtTrainer:
             return ws.loss_sum * ws.inv_norm
         self.optimizer_step(lr=lr, **opt)
         return ws.loss_sum * ws.inv_norm
+
+    # ---- self-critical sequence training -------------------------------------------------------------------
+    def rollout_engine(self, **engine_kw):
+        """The inference engine of the SCST rollouts, built once and bound to this trainer's memory: bf16 linears read the
+        step's pre-masked operands (``_wm``), biases and LayerNorm parameters are views of ``flat_w``; the masked embedding
+        table and geometry weights (and, in fp32, every masked linear) are engine-owned and refreshed from the step's mask
+        sample by ``_refresh_engine``.  The pointers never change, so its CUDA graphs replay across optimizer steps."""
+        if self._rollout is None:
+            self._rollout = self._bound_engine(eval_masks=False, **engine_kw)
+        return self._rollout
+
+    def _baseline_engine(self):
+        """Supermask only: the greedy baseline decodes with eval-mode weights rint(sigmoid(S)), a second bound operand set."""
+        if self._baseline is None:
+            self._baseline = self._bound_engine(eval_masks=True)
+        return self._baseline
+
+    def _bound_engine(self, *, eval_masks, **engine_kw):
+        from .engine import OrtEngine
+        if engine_kw.get("ln_fold") or engine_kw.get("sparse_backend", "dense") != "dense":
+            raise ValueError("the rollout engine reads the trainer's dense operands: ln_fold and the sparse backends are not supported")
+        c, L, h = self.cfg, self.cfg.num_layers, self.cfg.num_heads
+        sd = {k: self.p[k] for k in self.names}
+        sd["model.tgt_embed.1.pe"] = self.pe[None]
+        eng = OrtEngine(sd, c, precision="bf16" if self.adt == torch.bfloat16 else "fp32", device=self.dev, use_graphs=self.use_graph,
+                        **engine_kw)
+        lins = {("att_embed.0.weight", 1): eng.att_embed, ("model.generator.proj.weight", 1): eng.generator}
+        norms = [(eng.enc_norm, "model.encoder.norm"), (eng.dec_norm, "model.decoder.norm")]
+        for l in range(L):
+            p, e = f"model.encoder.layers.{l}", eng.enc[l]
+            lins.update({(f"{p}.self_attn.linears.0.weight", 3): e["qkv"], (f"{p}.self_attn.linears.3.weight", 1): e["o"],
+                         (f"{p}.feed_forward.w_1.weight", 1): e["ff1"], (f"{p}.feed_forward.w_2.weight", 1): e["ff2"]})
+            norms += [(e[f"n{j}"], f"{p}.sublayer.{j}.norm") for j in range(2)]
+            p, e = f"model.decoder.layers.{l}", eng.dec[l]
+            lins.update({(f"{p}.self_attn.linears.0.weight", 3): e["qkv"], (f"{p}.self_attn.linears.3.weight", 1): e["o"],
+                         (f"{p}.src_attn.linears.0.weight", 1): e["cq"], (f"{p}.src_attn.linears.1.weight", 2): e["ckv"],
+                         (f"{p}.src_attn.linears.3.weight", 1): e["co"], (f"{p}.feed_forward.w_1.weight", 1): e["ff1"],
+                         (f"{p}.feed_forward.w_2.weight", 1): e["ff2"]})
+            norms += [(e[f"n{j}"], f"{p}.sublayer.{j}.norm") for j in range(3)]
+        assert set(lins) == set(self._premask_keys())
+        # bf16 rollouts read the trainer's own pre-masked operands; everything else is refreshed into engine-owned buffers
+        share = self.adt == torch.bfloat16 and self.premask and not eval_masks
+        if share and self._premask_desc is None:
+            self._premask_all()   # (allocates _wm)
+        items = {torch.bfloat16: [], torch.float32: []}
+
+        def owned(wname, count, dtype):
+            W = self._group(self.p, wname, count)
+            out = torch.empty(W.shape, device=self.dev, dtype=dtype)
+            S = self._group(self.s, wname, count) if self.mask_type else None
+            items[dtype].append((W, S, self._u(wname, count), out, None, self.stream_of[wname]))
+            return out
+
+        for (wname, count), lin in lins.items():
+            op = self._wm[(wname, count)] if share else owned(wname, count, self.adt)
+            bias = self._group(self.p, wname.replace(".weight", ".bias"), count)
+            assert op.shape[0] >= lin.N and op.shape[1] == lin.K and bias.shape[0] >= lin.N
+            lin.w, lin.bias = op[: lin.N], bias[: lin.N]       # (generator: the first V rows of the padded operand)
+        for nrm, name in norms:
+            nrm.a, nrm.b = self.p[name + ".a_2"], self.p[name + ".b_2"]
+        eng.table = owned("model.tgt_embed.0.lut.weight", 1, torch.float32)
+        eng.wg_w_all = torch.empty_like(eng.wg_w_all)
+        b0 = self._offs_w["model.encoder.layers.0.self_attn.WGs.0.bias"]
+        if any(self._offs_w[f"model.encoder.layers.{l}.self_attn.WGs.{j}.bias"] != b0 + l * h + j for l in range(L) for j in range(h)):
+            raise ValueError(f"the rollout engine needs the geometry biases packed in the trainer's layout (num_heads % 4 == 0, got {h})")
+        eng.wg_b_all = self.flat_w[b0: b0 + L * h]
+        for l in range(L):
+            wname = f"model.encoder.layers.{l}.self_attn.WGs.0.weight"
+            W = self._group(self.p, wname, h)
+            out = eng.wg_w_all[l * h: (l + 1) * h]
+            items[torch.float32].append((W, self._group(self.s, wname, h) if self.mask_type else None, self._u(wname, h), out, None,
+                                         self.stream_of[wname]))
+            eng.enc[l]["wg_w"], eng.enc[l]["wg_b"] = out, eng.wg_b_all[l * h: (l + 1) * h]
+        eng.scst_refresh = [(K.mask_descriptors(it, self.dev), dt) for dt, it in items.items() if it]
+        eng.scst_eval = eval_masks
+        return eng
+
+    def _scst_masks(self, eng):
+        """Step 1 of an SCST step: the step's mask sample into the trainer's bf16 operands and the engine-owned ones (same seeds
+        and Philox streams, so the rollout and the teacher-forced re-score see one network)."""
+        if self.adt == torch.bfloat16 and self.premask:
+            self._premask_all()
+        self._refresh_engine(eng)
+
+    def _refresh_engine(self, eng):
+        """The engine-owned operands from the step's mask sample (the trainer's seeds and Philox streams), or from rint(sigmoid(S))
+        for the baseline engine: one sc_apply_mask_batched launch per operand dtype."""
+        mode = K.MASK_ROUND if eng.scst_eval else self.mask_mode()
+        for (desc, tiles), dt in eng.scst_refresh:
+            K.apply_mask_batched(desc, tiles, mode, seed=self._sd(0), stream_base=self._step_base(), out_dtype=dt)
+
+    def scst_step(self, att_feats, boxes, att_masks=None, *, scorer, image_ids=None, opt=None, baseline="greedy", cider_weight=1.0,
+                  bleu_weight=0.0, lr, all_reduce=None, **optim):
+        """One self-critical step (utils/training.py:202-255 + RewardCriterion + clip + Adam) without a host synchronisation:
+        premask the step's sample -> rollout (``opt``: {"beam_size": b[, "group_size": G]} or {"num_random_sample": n,
+        "beam_size": 0}) and greedy baseline on the bound engine -> CIDEr-D (``scorer``: cider.CiderD; ``image_ids`` [B]: rows of
+        its references, default 0 .. B-1) -> sc_scst_targets -> teacher-forcing forward / backward / optimizer (``optim``: the
+        keyword arguments of ``train_step``).  ``baseline``: "greedy" or "sample" (mean of the image's other samples).  The rollout
+        and the re-score share the step's ONE mask sample.  ``all_reduce``: data parallel as in ``train_step``; the token count
+        is summed over the ranks before the loss.  Returns (loss, mean reward, sample_seq int32 [B, S, L]) as device tensors."""
+        opt = dict(opt if opt is not None else {"beam_size": 5})
+        S = scst_samples(opt, baseline, bleu_weight)
+        c = self.cfg
+        B, N = att_feats.shape[:2]
+        L, R = c.max_seq_length, B * S
+        ws = self._get_ws(B, N, S, L, att_masks is not None)
+        if not hasattr(ws, "mask_sum"):
+            ws.mask_sum = torch.zeros(1, device=self.dev)
+            ws.mean_reward = torch.zeros(1, device=self.dev)
+        self.step_id += 1
+        if self.use_graph:
+            self._upload_step(lr=lr, **optim)
+        eng = self.rollout_engine()
+        self._scst_masks(eng)
+        # 2. rollouts; the sampler seed follows the trainer's step seed (a run is reproducible)
+        if int(opt.get("num_random_sample", 0)) > 0:
+            v = (self.seed + 3 + self.step_id * 0x9E3779B97F4A7C15) & 0xFFFFFFFFFFFFFFFF
+            opt["sample_seed"] = v - (1 << 64) if v >= (1 << 63) else v
+        greedy = {"beam_size": 1}
+        bseq = None
+        enc = eng.encode(att_feats, boxes, att_masks)
+        seq, _ = eng.decode(enc, opt)
+        if baseline == "greedy":
+            if self.mask_type == "supermask":
+                beng = self._baseline_engine()
+                self._refresh_engine(beng)
+                bseq, _ = beng.decode(beng.encode(att_feats, boxes, att_masks), greedy)
+            else:
+                bseq, _ = eng.decode(enc, greedy)
+        seq = seq.reshape(R, L)
+        # 3. CIDEr-D of the samples and the baseline
+        ids = (torch.arange(B, device=self.dev) if image_ids is None else torch.as_tensor(image_ids).to(self.dev)).to(torch.int32)
+        score = scorer.score(seq, ids.repeat_interleave(S))
+        bscore = scorer.score(bseq.reshape(B, L), ids) if bseq is not None else None
+        # 4. rewards, targets and the token count
+        targ = dict(S=S, cider_weight=cider_weight, bos=c.bos_token_id, pad=c.pad_token_id, tokens=ws.tokens, targets=ws.targets,
+                    tok_w=ws.tok_w, key_valid=ws.key_valid, inv_norm=ws.inv_norm, mean_reward=ws.mean_reward)
+        K.scst_targets(seq, score, bscore, mask_sum=ws.mask_sum, **targ)
+        if all_reduce is not None:
+            h = all_reduce(ws.mask_sum)
+            if h is not None:
+                h.wait()
+            K.scst_targets(seq, score, bscore, norm_in=ws.mask_sum, **targ)   # inv_norm = 1 / global count
+        ws.att_in.copy_(att_feats.reshape(B * N, -1), non_blocking=True)
+        ws.boxes.copy_(boxes, non_blocking=True)
+        if att_masks is not None:
+            ws.att_mask.copy_(att_masks.float(), non_blocking=True)
+        # 5. teacher-forcing forward on the step's operands, backward, clip + Adam
+        prev_pdl = K.set_pdl(self.pdl_mask)
+        self._scst = True
+        try:
+            loss = self._fwd_bwd_opt(ws, lr, all_reduce, optim)
+        finally:
+            self._scst = False
+            K.set_pdl(prev_pdl)
+        return loss, ws.mean_reward.clone(), seq.view(B, S, L).clone()
 
     def state_dict(self):
         sd = {k: v.clone() for k, v in self.p.items()}
@@ -1155,6 +1349,12 @@ class ModuleTrainer:
         if getattr(m, "MASKED", False) and m.mask_type == "supermask" and sparsity_target is not None and sparsity_weight:
             total = total + m.compute_sparsity_loss(sparsity_target, sparsity_weight, current_step, max_step)
         total.backward()
+        self._update(params, all_reduce, lr=lr, mask_lr=mask_lr, clip=clip, betas=betas, eps=eps, mask_eps=mask_eps,
+                     weight_decay=weight_decay, grad_scale=grad_scale)
+        return loss.detach()
+
+    def _update(self, params, all_reduce, *, lr, mask_lr=100.0, clip=0.1, betas=(0.9, 0.98), eps=1e-9, mask_eps=1e-2, weight_decay=0.0,
+                grad_scale=1.0):
         if all_reduce is not None:  # data parallel: sum the gradients of every rank (the loss is normalised by the global token count)
             flat = torch._utils._flatten_dense_tensors([p.grad for _, p in params])
             h = all_reduce(flat)
@@ -1173,7 +1373,59 @@ class ModuleTrainer:
                 K.adam_clip(p.data.view(-1), g, mom, var, lr=mask_lr if is_logit else lr, betas=betas, eps=mask_eps if is_logit else eps,
                             weight_decay=0.0 if is_logit else weight_decay, clip=clip, grad_scale=grad_scale, step=self.opt_step)
                 torch.autograd.graph.increment_version(p)  # (written through raw pointers: cached engines must notice)
-        return loss.detach()
+
+    def scst_step(self, att_feats, boxes, att_masks=None, *, scorer, image_ids=None, opt=None, baseline="greedy", cider_weight=1.0,
+                  bleu_weight=0.0, lr, all_reduce=None, **optim):
+        """``OrtTrainer.scst_step`` for ACORT through the module tree (correctness path): greedy baseline in eval mode, rollout in
+        train mode, CIDEr-D and sc_scst_targets on the device, RewardCriterion on the autograd teacher-forced log-probs, then the
+        update of ``train_step``.  The train-mode rollout and the re-score draw their own supermask samples (module path)."""
+        opt = dict(opt if opt is not None else {"beam_size": 5})
+        S = scst_samples(opt, baseline, bleu_weight)
+        m = self.model
+        dev = m._device()
+        c = m.cfg
+        att_feats, boxes = att_feats.to(dev), boxes.to(dev)
+        att_masks = None if att_masks is None else att_masks.to(dev)
+        B, L = att_feats.shape[0], c.max_seq_length
+        R = B * S
+        bseq = None
+        if baseline == "greedy":
+            m.eval()
+            bseq, _ = m(att_feats=att_feats, boxes=boxes, att_masks=att_masks, opt={"beam_size": 1}, mode="sample")
+        m.train()
+        seq, _ = m(att_feats=att_feats, boxes=boxes, att_masks=att_masks, opt=opt, mode="sample")
+        seq = seq.reshape(R, L).to(torch.int32).contiguous()
+        ids = (torch.arange(B, device=dev) if image_ids is None else torch.as_tensor(image_ids).to(dev)).to(torch.int32)
+        score = scorer.score(seq, ids.repeat_interleave(S))
+        bscore = scorer.score(bseq.reshape(B, L), ids) if bseq is not None else None
+        i32, f32 = dict(dtype=torch.int32, device=dev), dict(dtype=torch.float32, device=dev)
+        tokens, targets, tok_w, key_valid = (torch.empty(R * L, **i32), torch.empty(R * L, **i32), torch.empty(R * L, **f32),
+                                             torch.empty(R * L, **f32))
+        inv_norm, mask_sum, mean_reward = torch.empty(1, **f32), torch.empty(1, **f32), torch.empty(1, **f32)
+        targ = dict(S=S, cider_weight=cider_weight, bos=c.bos_token_id, pad=c.pad_token_id, tokens=tokens, targets=targets, tok_w=tok_w,
+                    key_valid=key_valid, inv_norm=inv_norm, mean_reward=mean_reward)
+        K.scst_targets(seq, score, bscore, mask_sum=mask_sum, **targ)
+        if all_reduce is not None:
+            h = all_reduce(mask_sum)
+            if h is not None:
+                h.wait()
+            K.scst_targets(seq, score, bscore, norm_in=mask_sum, **targ)
+        params = [(n, p) for n, p in m.named_parameters() if p.requires_grad]
+        for _, p in params:
+            p.grad = None
+        # teacher-forced log-probs of the sampled captions: input [BOS, s_0 .. s_{L-2}], target s (RewardCriterion)
+        seqs = torch.cat([tokens.view(R, L).long(), seq[:, L - 1:].long()], 1)
+        out = m(att_feats=att_feats, boxes=boxes, seqs=seqs, att_masks=att_masks)
+        lp = out.gather(2, targets.view(R, L, 1).long()).squeeze(2)
+        loss = -(lp * tok_w.view(R, L)).sum() * inv_norm[0]
+        total = loss
+        sp = {k: optim.pop(k) for k in ("sparsity_target", "sparsity_weight", "current_step", "max_step") if k in optim}
+        if getattr(m, "MASKED", False) and m.mask_type == "supermask" and sp.get("sparsity_target") is not None and sp.get("sparsity_weight"):
+            total = total + m.compute_sparsity_loss(sp["sparsity_target"], sp["sparsity_weight"], sp.get("current_step", 0),
+                                                    sp.get("max_step", 1))
+        total.backward()
+        self._update(params, all_reduce, lr=lr, **optim)
+        return loss.detach(), mean_reward, seq.view(B, S, L)
 
     def state_dict(self):
         return self.model.state_dict()
