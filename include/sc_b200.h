@@ -356,6 +356,30 @@ int sc_scst_targets(const int* seq, int R, int L, int S, const double* score, co
                     int bos, int pad, int* tokens, int* targets, float* tok_w, float* key_valid, float* mask_sum, float* inv_norm,
                     const float* norm_in, float* mean_reward, sc_stream_t stream);
 
+/* Magnitude / SNIP mask updates on flat buffers (PruningMixin.update_masks_once + compute_mask, pruning/prune.py:259-289 and the
+ * gradual schedule :375-433 that calls it).  descs: device int64 [n_desc][6] = {src_off, dst_off, n, group, pos_base, first_block}:
+ * segment i is one masked tensor, elements src[src_off + e] of the criterion source (weights, or the SNIP saliency) and
+ * mask_out[dst_off + e], e < n; `group` its selection group, pos_base + e its 32-bit position in that group (the tie-break);
+ * one CTA per sc_prune_chunk() elements, segment i owns CTAs [first_block_i, first_block_{i+1}).
+ * sc_prune_stats: sums [n_desc][2] (double) = per segment {sum x, sum x^2}, x = src, or rint(sigmoid(src)) when binarize
+ *   (the per-tensor counts of calculate_sparsities, prune.py:124-144); with center (optional, the sums of a first call) the second
+ *   column is sum (x - mean)^2 (two-pass variance: exactly 0 for a constant tensor).  partials: double [total_blocks][2] scratch.
+ *   Fixed summation order: bitwise reproducible.
+ * sc_prune_select: criterion SC_PRUNE_ABS |w| (mag_blind / mag_uniform), SC_PRUNE_DIST |(w - mean) / std| with the segment's mean
+ *   and population std from `sums` of the centred pass (mag_dist), SC_PRUNE_SNIP sal / (sum of the group's sal) from `sums` (snip), computed in fp32 on
+ *   the fly.  Per group the first group_k[g] elements in (criterion, position) order get 0, every other element 1 (the complete
+ *   mask is written: a weight pruned earlier can come back).  -0.0 sorts as +0.0, NaN above every number.  group_k (device int64
+ *   [n_groups]) in [0, group size).  workspace: 16-byte aligned, n_groups * 1056 + n_desc * 8 bytes. */
+#define SC_PRUNE_ABS 0
+#define SC_PRUNE_DIST 1
+#define SC_PRUNE_SNIP 2
+int sc_prune_chunk(void);
+int sc_prune_stats(const void* descs, int n_desc, long total_blocks, const float* src, int binarize, const double* center,
+                   double* partials, double* sums, sc_stream_t stream);
+int sc_prune_select(const void* descs, int n_desc, long total_blocks, int n_groups, const long long* group_k, int criterion,
+                    const float* src, const double* sums, float* mask_out, void* workspace, size_t workspace_bytes,
+                    sc_stream_t stream);
+
 /* teacher-forcing attention with saved probabilities + backward (decoder self: causal_T = T; cross: groups = images with
  * S*T query rows; encoder box attention: additive bias): transformer.py:230-295, relation_transformer.py:258-293 */
 int sc_attention_fwd(const void* q, const void* k, const void* v, int ldq, int ldk, int ldv, int dtype, const float* key_valid,

@@ -654,6 +654,60 @@ def adam_clip_st(desc, blocks, w, g, m_w, v_w, s, m_s, v_s, *, uniforms, mask_mo
              float(grad_scale), int(step), lib.ptr(sigmoid_grad_coeff), lib.ptr(dyn), lib.stream())
 
 
+PRUNE_ABS, PRUNE_DIST, PRUNE_SNIP = 0, 1, 2
+
+
+def prune_descriptors(segments, device):
+    """Descriptor table of sc_prune_stats / sc_prune_select.  segments: (src_off, dst_off, n, group, pos_base) in flat-buffer
+    elements.  Returns (int64 device tensor [n, 6], total blocks)."""
+    chunk = int(lib.load().sc_prune_chunk())
+    rows, start = [], 0
+    for src_off, dst_off, n, group, pos_base in segments:
+        assert n > 0 and 0 <= pos_base and pos_base + n <= 1 << 32, (n, pos_base)
+        rows.append([int(src_off), int(dst_off), int(n), int(group), int(pos_base), start])
+        start += (int(n) + chunk - 1) // chunk
+    return _to_device(torch.tensor(rows, dtype=torch.int64), device), start
+
+
+def _to_device(t, device):
+    """Host tensor -> device without a host synchronisation: staged in pinned memory, copied asynchronously on the current
+    stream (the caching host allocator keeps the staging block until the copy has run)."""
+    device = torch.device(device)
+    if device.type != "cuda":
+        return t.to(device)
+    return t.pin_memory().to(device, non_blocking=True)
+
+
+def prune_stats(desc, blocks, src, *, binarize=False, centered=False):
+    """Per-segment {sum x, sum x^2} (float64 [n_desc, 2]) of ``src`` (or of rint(sigmoid(src)) with ``binarize``); ``centered``:
+    {sum x, sum (x - mean)^2} from a second pass (the two-pass variance of mag_dist)."""
+    assert src.dtype == torch.float32 and src.is_contiguous()
+    partials = torch.empty(blocks, 2, dtype=torch.float64, device=src.device)
+
+    def run(center):
+        sums = torch.empty(desc.shape[0], 2, dtype=torch.float64, device=src.device)
+        lib.call("sc_prune_stats", lib.ptr(desc), desc.shape[0], blocks, lib.ptr(src), int(binarize), lib.ptr(center), lib.ptr(partials),
+                 lib.ptr(sums), lib.stream())
+        return sums
+
+    sums = run(None)
+    return run(sums) if centered else sums
+
+
+def prune_select(desc, blocks, group_k, criterion, src, mask_out, *, sums=None):
+    """0/1 masks into ``mask_out``: per group, the first group_k[g] elements in (criterion, position) order are pruned
+    (sc_prune_select).  group_k: a list of ints (uploaded without a host synchronisation) or a device int64 tensor.  ``sums``:
+    prune_stats of ``src`` for PRUNE_SNIP, prune_stats(centered=True) for PRUNE_DIST."""
+    if not torch.is_tensor(group_k):
+        group_k = _to_device(torch.tensor(group_k, dtype=torch.int64), src.device)
+    assert src.dtype == mask_out.dtype == torch.float32 and group_k.dtype == torch.int64 and group_k.is_cuda
+    n_groups = group_k.numel()
+    ws = torch.empty(n_groups * 1056 + desc.shape[0] * 8, dtype=torch.uint8, device=src.device)
+    lib.call("sc_prune_select", lib.ptr(desc), desc.shape[0], blocks, n_groups, lib.ptr(group_k), int(criterion), lib.ptr(src),
+             lib.ptr(sums), lib.ptr(mask_out), lib.ptr(ws), ws.numel(), lib.stream())
+    return mask_out
+
+
 def sparsity_coeff(count, total, target, scale, out3, scale_dev=None):
     """out3 = [|target - sparsity|, d(scaled loss)/d(nnz), sparsity] from the device-side binarized-mask count."""
     lib.call("sc_sparsity_coeff", lib.ptr(count), float(total), float(target), float(scale), lib.ptr(scale_dev), lib.ptr(out3),

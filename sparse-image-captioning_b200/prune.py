@@ -67,6 +67,19 @@ def fold_masks(state_dict, mask_type):
     return out
 
 
+def gradual_sparsity(sparsity_target, current_step, start_step, prune_steps, initial_sparsity=0.0, prune_frequency=1000):
+    """The sparsity that update_masks_gradual prunes to at `current_step` (cubic schedule, prune.py:375-433), or None when
+    no mask update is due at that step.  Shared by PruningMixin and trainer.OrtTrainer."""
+    assert prune_frequency > 0, f"Pruning frequency must be greater than zero, saw `{prune_frequency}`"
+    assert prune_steps > 0, f"Pruning steps must be greater than zero, saw `{prune_steps}`"
+    end_step = start_step + prune_frequency * prune_steps
+    in_range = current_step >= start_step and (current_step <= end_step or end_step < 0)
+    if in_range and (current_step - start_step) % prune_frequency == 0:
+        progress = min(1.0, max(0.0, (current_step - start_step) / (end_step - start_step)))
+        return sparsity_target + (initial_sparsity - sparsity_target) * (1.0 - progress) ** 3
+    return None
+
+
 class _SparsityLossFn(torch.autograd.Function):
     """|target - sparsity| with the straight-through gradient of rounding_sigmoid: d nnz / dS = sigmoid'(S)."""
 
@@ -293,13 +306,8 @@ class PruningMixin:
                              initial_sparsity: float = 0.0, prune_frequency: int = 1000):
         """Cubic sparsity schedule of Zhu & Gupta (arXiv:1710.01878), prune.py:375-433."""
         assert self.mask_type in MAG_ANNEAL
-        assert prune_frequency > 0, f"Pruning frequency must be greater than zero, saw `{prune_frequency}`"
-        assert prune_steps > 0, f"Pruning steps must be greater than zero, saw `{prune_steps}`"
-        end_step = start_step + prune_frequency * prune_steps
-        in_range = current_step >= start_step and (current_step <= end_step or end_step < 0)
-        if in_range and (current_step - start_step) % prune_frequency == 0:
-            progress = min(1.0, max(0.0, (current_step - start_step) / (end_step - start_step)))
-            now = sparsity_target + (initial_sparsity - sparsity_target) * (1.0 - progress) ** 3
+        now = gradual_sparsity(sparsity_target, current_step, start_step, prune_steps, initial_sparsity, prune_frequency)
+        if now is not None:
             self.update_masks_once(sparsity_target=now)
         return False  # the reference returns False on every path (prune.py:433)
 

@@ -558,6 +558,8 @@ class _OrtBase(nn.Module):
             return self._trainer
         key = self._param_key()
         if self._trainer is None or self._trainer_key != key:
+            if self.MASKED:
+                kw.setdefault("mask_freeze_scope", self.mask_freeze_scope)
             self._trainer = OrtTrainer(self.state_dict(), self.cfg, mask_type=self.mask_type if self.MASKED else None,
                                        precision=self.precision, device=self._device(), dropout=self.dropout_p,
                                        drop_prob_src=self.drop_prob_src, **kw)

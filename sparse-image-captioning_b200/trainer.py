@@ -55,13 +55,20 @@ def scst_samples(opt, baseline, bleu_weight=0.0):
 class OrtTrainer:
     def __init__(self, state_dict: Dict[str, torch.Tensor], cfg: ModelCfg, *, mask_type: Optional[str] = "supermask",
                  precision="bf16", device="cuda", dropout=0.1 / 3, drop_prob_src=0.5, bypass_sigmoid_grad=False, seed=0,
-                 mask_init_value=5.0, uniforms: Optional[Dict[str, torch.Tensor]] = None, use_graph=False, fused_st=True):
+                 mask_init_value=5.0, uniforms: Optional[Dict[str, torch.Tensor]] = None, use_graph=False, fused_st=True,
+                 mask_freeze_scope=None):
         assert cfg.share_att_encoder is None and cfg.share_att_decoder is None and not cfg.share_layer_encoder \
             and not cfg.share_layer_decoder, "the fused engine lays out the ORT stack; ACORT weight sharing trains through ModuleTrainer (model.trainer() picks it)"
         self.cfg = cfg
         self.dev = K.lib.resolve_device(device)
         self.adt = torch.bfloat16 if precision == "bf16" else torch.float32
         self.mask_type = mask_type
+        # prefixes of the frozen masks (PruningMixin.mask_freeze_scope: a list, or the comma-separated string of its constructor);
+        # magnitude / SNIP updates leave those masks alone
+        if isinstance(mask_freeze_scope, str):
+            mask_freeze_scope = [x for x in mask_freeze_scope.split(",") if x != ""] if mask_freeze_scope != "" else None
+        self.mask_freeze_scope = None if mask_freeze_scope is None else list(mask_freeze_scope)
+        self.sparsity_target = 0.0
         self.p_drop, self.p_src = float(dropout), float(drop_prob_src)
         self.bypass = bool(bypass_sigmoid_grad)
         self.seed = int(seed)
@@ -200,6 +207,10 @@ class OrtTrainer:
         # SCST step in progress: its masks were applied before the rollouts (scst_step), the forward must reuse that sample
         self._scst = False
         self._rollout = self._baseline = None
+        # magnitude / SNIP mask updates: cached sc_prune descriptor tables, the accumulated SNIP saliency (flat_s layout)
+        self._prune_desc = {}
+        self._saliency = None
+        self._has_saliency = False
 
     # ---------------------------------------------------------------------------------------------------------
     def _group(self, table, first, count):
@@ -1012,17 +1023,21 @@ class OrtTrainer:
     def _upload_step(self, *, lr, mask_lr=100.0, betas=(0.9, 0.98), sparsity_weight=0.0, current_step=0, max_step=1, **_):
         """Per-step scalars of the captured graph -> pinned host words -> device (two tiny async copies)."""
         self.opt_step += 1
-        golden = 0x9E3779B97F4A7C15
-        for i in range(3):
-            v = (self.seed + i + self.step_id * golden) & 0xFFFFFFFFFFFFFFFF
-            self._seeds_host[i] = v - (1 << 64) if v >= (1 << 63) else v
+        self._upload_seeds()
         bc1 = 1.0 - betas[0] ** self.opt_step
         bc2 = math.sqrt(1.0 - betas[1] ** self.opt_step)
         anneal = (1.0 + math.cos(min(1.0, current_step / max_step) * math.pi)) / 2.0
         h = self._dyn_host
         h[0], h[1], h[2], h[3], h[4], h[5], h[6] = lr, bc1, bc2, mask_lr, bc1, bc2, sparsity_weight * (1.0 - anneal)
-        self._seeds_dev.copy_(self._seeds_host, non_blocking=True)
         self._dyn_dev.copy_(self._dyn_host, non_blocking=True)
+
+    def _upload_seeds(self):
+        """The step's Philox seeds (masks, dropout, attention dropout) for the captured graphs."""
+        golden = 0x9E3779B97F4A7C15
+        for i in range(3):
+            v = (self.seed + i + self.step_id * golden) & 0xFFFFFFFFFFFFFFFF
+            self._seeds_host[i] = v - (1 << 64) if v >= (1 << 63) else v
+        self._seeds_dev.copy_(self._seeds_host, non_blocking=True)
 
     def _graph_body(self, ws, part, opt):
         # every body (eager warm-up, capture) re-applies the masks - except an SCST body, whose masks the rollout already used
@@ -1309,6 +1324,126 @@ class OrtTrainer:
             self._scst = False
             K.set_pdl(prev_pdl)
         return loss, ws.mean_reward.clone(), seq.view(B, S, L).clone()
+
+    # ---- magnitude / SNIP mask updates (PruningMixin.update_masks_*, pruning/prune.py:259-304) ------------------------------
+    # The masks of flat_s are rewritten in place by sc_prune_select; weights, Adam moments, opt_step, step_id, workspaces, captured
+    # graphs and the rollout engine are untouched (every step re-reads flat_s: premask / operand prologues / _refresh_engine).
+    def active_masked(self):
+        """Masked tensors a mask update rewrites, in module order: PruningMixin.active_pruning_masks (mask_freeze_scope)."""
+        scope = self.mask_freeze_scope
+        return [k for k in self.masked if scope is None or not any((k + "_pruning_mask").startswith(s) for s in scope)]
+
+    def _prune_table(self, from_saliency, per_tensor):
+        """(descriptors, blocks, sizes) of the active masks: one segment per tensor (the generator's V rows, not the padded Vp),
+        one selection group per tensor or one for all; position = index in the concatenation of the active masks (or in the
+        tensor).  The criterion source is flat_w, or the saliency buffer, which has flat_s's layout."""
+        key = (from_saliency, per_tensor)
+        if key not in self._prune_desc:
+            segs, pos = [], 0
+            for i, k in enumerate(self.active_masked()):
+                n = self.s[k].numel()
+                segs.append((self._offs_s[k] if from_saliency else self._offs_w[k], self._offs_s[k], n, i if per_tensor else 0,
+                             0 if per_tensor else pos))
+                pos += n
+            assert segs, "no active pruning masks (mask_freeze_scope freezes all of them)"
+            self._prune_desc[key] = K.prune_descriptors(segs, self.dev) + ([sg[2] for sg in segs],)
+        return self._prune_desc[key]
+
+    @torch.no_grad()
+    def update_masks_once(self, sparsity_target: float):
+        """PruningMixin.update_masks_once on the trainer's own buffers, on the device and without a host synchronisation: the
+        complete 0/1 mask of every active tensor from the exact k-th smallest criterion (sc_prune_select; ties in module order).
+        ``snip`` consumes (and clears) the saliency accumulated by ``snip_saliency``.  Returns True."""
+        from . import prune as P
+        assert self.mask_type in P.MAG_PRUNE_MASKS, f"Invalid mask_type: {self.mask_type}. Must be one of {P.MAG_PRUNE_MASKS}"
+        if self.mask_type == P.SNIP:
+            assert self._has_saliency, "SNIP needs the mask gradients: call snip_saliency() first"
+            crit, src = K.PRUNE_SNIP, self._saliency
+        elif self.mask_type in P._DIST:
+            crit, src = K.PRUNE_DIST, self.flat_w
+        elif self.mask_type in P._BLIND or self.mask_type in P._UNIFORM:
+            crit, src = K.PRUNE_ABS, self.flat_w
+        else:
+            raise ValueError(f"Unknown `self.mask_type`: {self.mask_type}")
+        assert isinstance(sparsity_target, float) and 0 <= sparsity_target < 1.0, \
+            f"`sparsity_target` must be a float >= 0 and < 1, saw {sparsity_target}"
+        per_tensor = self.mask_type in P._UNIFORM
+        desc, blocks, sizes = self._prune_table(crit == K.PRUNE_SNIP, per_tensor)
+        groups = sizes if per_tensor else [sum(sizes)]
+        ks = [int(sparsity_target * n) for n in groups]
+        assert all(0 <= k < n for k, n in zip(ks, groups))
+        sums = K.prune_stats(desc, blocks, src, centered=crit == K.PRUNE_DIST) if crit != K.PRUNE_ABS else None
+        K.prune_select(desc, blocks, ks, crit, src, self.flat_s, sums=sums)
+        if crit == K.PRUNE_SNIP:
+            self._saliency.zero_()
+            self._has_saliency = False
+        self._wm_step = {}   # (an eval-mode operand cached for the current step_id is stale now)
+        self.sparsity_target = sparsity_target
+        return True
+
+    def update_masks_gradual(self, sparsity_target: float, current_step: int, start_step: int, prune_steps: int,
+                             initial_sparsity: float = 0.0, prune_frequency: int = 1000):
+        """PruningMixin.update_masks_gradual (cubic schedule, prune.gradual_sparsity) through ``update_masks_once``.  Returns
+        False, like the reference."""
+        from . import prune as P
+        assert self.mask_type in P.MAG_ANNEAL
+        now = P.gradual_sparsity(sparsity_target, current_step, start_step, prune_steps, initial_sparsity, prune_frequency)
+        if now is not None:
+            self.update_masks_once(now)
+        return False
+
+    def snip_saliency(self, att_feats, boxes, seqs, masks, att_masks=None, *, seq_per_img, all_reduce=None, global_tokens=None):
+        """SNIP: adds dL/dm = dWm (.) W of every active mask to the saliency buffer (repeated calls accumulate, the reference's
+        ``prune_snip_grad_accum`` batches).  Teacher-forcing forward + backward of ``train_step`` (graph mode: the "fwdbwd"
+        graph), no optimizer step.  ``all_reduce``: data parallel, the gradient buffer is summed over the ranks first (the
+        weights are identical, so this sums the saliency).  Returns the batch loss (device scalar)."""
+        from . import prune as P
+        assert self.mask_type == P.SNIP, f"snip_saliency needs mask_type '{P.SNIP}', saw {self.mask_type!r}"
+        B, N = att_feats.shape[:2]
+        T = seqs.shape[1] - 1
+        ws = self._get_ws(B, N, seq_per_img, T, att_masks is not None)
+        self.step_id += 1
+        self.load_batch(ws, att_feats, boxes, seqs, masks, att_masks, global_tokens)
+        prev_pdl = K.set_pdl(self.pdl_mask)
+        try:
+            if self.use_graph:
+                self._upload_seeds()
+                self._run_graphed(ws, "fwdbwd", {})
+            else:
+                self.forward(ws)
+                self.loss_and_backward(ws)
+        finally:
+            K.set_pdl(prev_pdl)
+        grads = self.flat_gw if self.fused_st else self.flat_gs   # dWm (straight-through form) or dS = dWm (.) W (raw masks)
+        if all_reduce is not None:
+            h = all_reduce(grads)
+            if h is not None:
+                h.wait()
+        if self._saliency is None:
+            self._saliency = torch.zeros_like(self.flat_s)
+        for k in self.active_masked():
+            sal = self._saliency[self._offs_s[k]: self._offs_s[k] + self.s[k].numel()]
+            if self.fused_st:
+                K.mask_grad(self.g[k], self.p[k], self.s[k], K.MASK_RAW, None, sal, accumulate=True)
+            else:
+                sal.add_(self.gs[k].reshape(-1))
+        self._has_saliency = True
+        return ws.loss_sum * ws.inv_norm
+
+    def mask_sparsities(self):
+        """PruningMixin.all_mask_sparsities of the trainer's masks: (overall sparsity, nnz, per-tensor sparsities, mask names) as
+        Python numbers.  Counted on the device (rint(sigmoid(S)) for supermask, the raw mask values otherwise) with one copy to
+        the host."""
+        assert self.masked, "the trainer has no pruning masks (mask_type=None)"
+        if "count" not in self._prune_desc:
+            segs = [(self._offs_s[k], self._offs_s[k], self.s[k].numel(), 0, 0) for k in self.masked]
+            self._prune_desc["count"] = K.prune_descriptors(segs, self.dev)
+        desc, blocks = self._prune_desc["count"]
+        nnz = K.prune_stats(desc, blocks, self.flat_s, binarize=self.mask_type == "supermask")[:, 0].tolist()
+        sizes = [self.s[k].numel() for k in self.masked]
+        total = sum(nnz)
+        return (1.0 - total / sum(sizes), total, [1.0 - c / n for c, n in zip(nnz, sizes)],
+                tuple(k + "_pruning_mask" for k in self.masked))
 
     def state_dict(self):
         sd = {k: v.clone() for k, v in self.p.items()}
