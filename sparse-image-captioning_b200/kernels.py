@@ -3,6 +3,7 @@
 All tensors must be CUDA tensors; outputs are allocated by the caller or here with torch (plumbing only).
 Every function launches on torch's current stream, so calls are CUDA-graph capturable.
 """
+import contextlib
 import math
 
 import torch
@@ -66,6 +67,16 @@ def set_pdl(enabled):
 
 
 _pdl_mask = 7
+
+
+@contextlib.contextmanager
+def pdl(mask):
+    """``with pdl(mask):`` the block launches with set_pdl(mask), then the previous mask is restored."""
+    prev = set_pdl(mask)
+    try:
+        yield
+    finally:
+        set_pdl(prev)
 
 
 class CsrWeight:
@@ -307,10 +318,10 @@ def apply_mask(w, mask, mask_mode, *, uniforms=None, seed=0, stream_id=0, out_dt
     return out
 
 
-def mask_count(logits_list):
-    """sum over tensors of sum(rint(sigmoid(S))) -> int64 CUDA scalar tensor."""
+def mask_count(logits_list, out=None):
+    """sum over tensors of sum(rint(sigmoid(S))) -> int64 CUDA scalar tensor (``out``: zeroed, then counted into)."""
     dev = logits_list[0].device
-    cnt = torch.zeros(1, dtype=torch.int64, device=dev)
+    cnt = torch.zeros(1, dtype=torch.int64, device=dev) if out is None else out.zero_()
     for s in logits_list:
         _chk(s, "logits")
         lib.call("sc_mask_count", lib.ptr(s), s.numel(), lib.ptr(cnt), lib.stream())

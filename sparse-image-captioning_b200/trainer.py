@@ -24,6 +24,50 @@ def _round_up(n, m):
     return (n + m - 1) // m * m
 
 
+# A layer's linears in parameter order.  Each entry is one storage block - consecutive linears of a module, their weights then
+# their biases - and the fused groups the forward runs on it: (count, OrtEngine slot).  The cross-attention stores q, k, v like
+# the self-attention's [q;k;v] but projects q alone and [k;v] once from the memory.
+_ATT = (("self_attn.linears.0", (3, "qkv")), ("self_attn.linears.3", (1, "o")))
+_FF = (("feed_forward.w_1", (1, "ff1")), ("feed_forward.w_2", (1, "ff2")))
+_CROSS = (("src_attn.linears.0", (1, "cq"), (2, "ckv")), ("src_attn.linears.3", (1, "co")))
+_LINEARS = {"encoder": _ATT + _FF, "decoder": _ATT + _CROSS + _FF}
+
+# Philox dropout sites (_drop_stream): the backward regenerates each dropout mask of the forward from its site.  att_embed 1, the
+# target embedding 2, and per layer l: site + l of the dropout after a linear (by OrtEngine slot) or of an attention's probabilities
+_SITES = {"att_embed": 1, "embed": 2, "encoder": dict(attn=10, o=20, ff1=30, ff2=40),
+          "decoder": dict(attn=50, o=60, cattn=70, co=80, ff1=90, ff2=100)}
+_DEC0 = "model.decoder.layers.0.self_attn.linears.0.weight"   # first decoder parameter: the decoder / encoder cut of the layout
+
+
+def _member(first, i):
+    """Name of the i-th linear of a block that starts at `first` ("self_attn.linears.0", 2 -> "self_attn.linears.2")."""
+    stem, j = first.rsplit(".", 1)
+    return first if i == 0 else f"{stem}.{int(j) + i}"
+
+
+def _layer_linears(p, stack):
+    """(first weight name, fused count, OrtEngine slot) of every fused group of layer `p`, and its linears' parameter names."""
+    groups, names = [], []
+    for first, *fused in _LINEARS[stack]:
+        members = [f"{p}.{_member(first, i)}" for i in range(sum(n for n, _ in fused))]
+        names += [m + ".weight" for m in members] + [m + ".bias" for m in members]
+        i = 0
+        for n, slot in fused:
+            groups.append((f"{members[i]}.weight", n, slot))
+            i += n
+    return groups, names
+
+
+def _anneal(current_step, max_step):
+    """Cosine anneal of the sparsity-loss weight (prune.py:246): 1 at step 0, 0 from max_step on."""
+    return (1.0 + math.cos(min(1.0, current_step / max_step) * math.pi)) / 2.0
+
+
+def _part(n, cut, part):
+    """[lo, hi) of an optimizer `part` of a layout of n: "all", "hi" (decoder, embedding, generator: from `cut`) or "lo"."""
+    return {"all": (0, n), "hi": (cut, n), "lo": (0, cut)}[part]
+
+
 def scst_samples(opt, baseline, bleu_weight=0.0):
     """Captions per image S of an SCST rollout ``opt`` (beam_size b, G * (b // G) for diverse beam search, or num_random_sample);
     ValueError for the options the device step does not support."""
@@ -89,30 +133,24 @@ class OrtTrainer:
         self._seeds_dev = torch.zeros(3, dtype=torch.int64, device=self.dev)
         self._dyn_host = torch.zeros(8, dtype=torch.float32).pin_memory() if self.use_graph else None
         self._dyn_dev = torch.zeros(8, dtype=torch.float32, device=self.dev)
-        d, L = cfg.d_model, cfg.num_layers
+        d, L, h = cfg.d_model, cfg.num_layers, cfg.num_heads
         sd = state_dict
         # ---- parameter layout: fused groups are contiguous so that [q;k;v] / [k;v] / WG blocks are single views ----
         # the one-element WG biases of ALL encoder layers come first, contiguous: the geometry bias of every layer is then
         # one kernel (sc_box_bias_all) over a single [L*h] bias vector
-        order = [f"model.encoder.layers.{i}.self_attn.WGs.{j}.bias" for i in range(L) for j in range(cfg.num_heads)]
+        order = [f"model.encoder.layers.{i}.self_attn.WGs.{j}.bias" for i in range(L) for j in range(h)]
         order += ["att_embed.0.weight", "att_embed.0.bias"]
-        for i in range(L):
-            p = f"model.encoder.layers.{i}"
-            order += [f"{p}.self_attn.linears.{j}.weight" for j in range(3)] + [f"{p}.self_attn.linears.{j}.bias" for j in range(3)]
-            order += [f"{p}.self_attn.linears.3.weight", f"{p}.self_attn.linears.3.bias"]
-            order += [f"{p}.self_attn.WGs.{j}.weight" for j in range(cfg.num_heads)]
-            order += [f"{p}.feed_forward.w_1.weight", f"{p}.feed_forward.w_1.bias", f"{p}.feed_forward.w_2.weight", f"{p}.feed_forward.w_2.bias"]
-            order += [f"{p}.sublayer.{j}.norm.{ab}" for j in range(2) for ab in ("a_2", "b_2")]
-        order += ["model.encoder.norm.a_2", "model.encoder.norm.b_2"]
-        for i in range(L):
-            p = f"model.decoder.layers.{i}"
-            for att in ("self_attn", "src_attn"):
-                order += [f"{p}.{att}.linears.{j}.weight" for j in range(3)] + [f"{p}.{att}.linears.{j}.bias" for j in range(3)]
-                order += [f"{p}.{att}.linears.3.weight", f"{p}.{att}.linears.3.bias"]
-            order += [f"{p}.feed_forward.w_1.weight", f"{p}.feed_forward.w_1.bias", f"{p}.feed_forward.w_2.weight", f"{p}.feed_forward.w_2.bias"]
-            order += [f"{p}.sublayer.{j}.norm.{ab}" for j in range(3) for ab in ("a_2", "b_2")]
-        order += ["model.decoder.norm.a_2", "model.decoder.norm.b_2", "model.tgt_embed.0.lut.weight",
-                  "model.generator.proj.weight", "model.generator.proj.bias"]
+        self._groups = {}   # (stack, layer) -> [(first weight name, fused count, OrtEngine slot)] of its linears, in forward order
+        for stack, n_norms in (("encoder", 2), ("decoder", 3)):
+            for i in range(L):
+                p = f"model.{stack}.layers.{i}"
+                self._groups[stack, i], names = _layer_linears(p, stack)
+                if stack == "encoder":   # the geometry heads' weights follow the self-attention's linears
+                    at = names.index(f"{p}.self_attn.linears.3.bias") + 1
+                    names[at:at] = [f"{p}.self_attn.WGs.{j}.weight" for j in range(h)]
+                order += names + [f"{p}.sublayer.{j}.norm.{ab}" for j in range(n_norms) for ab in ("a_2", "b_2")]
+            order += [f"model.{stack}.norm.a_2", f"model.{stack}.norm.b_2"]
+        order += ["model.tgt_embed.0.lut.weight", "model.generator.proj.weight", "model.generator.proj.bias"]
         self.names = order
         # the generator is stored with its vocabulary padded to a multiple of 8 rows (zero weights, bias -1e9, masked
         # out) so that dlogits can be a 16-byte-aligned bf16 GEMM operand for any V (e.g. the 771-token radix vocab)
@@ -143,6 +181,10 @@ class OrtTrainer:
         for k in order:
             self.p[k].copy_(sd[k])
         self._offs_w = offs
+        # all WG biases as one [L*h] view when the layout packed them without padding (h % 4 == 0)
+        b0 = offs["model.encoder.layers.0.self_attn.WGs.0.bias"]
+        packed = all(offs[f"model.encoder.layers.{l}.self_attn.WGs.{j}.bias"] == b0 + l * h + j for l in range(L) for j in range(h))
+        self._wg_b_all = self.flat_w[b0: b0 + L * h] if packed else None
         if self.Vp != V:
             ob = offs["model.generator.proj.bias"]
             self.flat_w[ob + V: ob + self.Vp] = -1e9
@@ -161,6 +203,7 @@ class OrtTrainer:
             else:
                 self.s[k].fill_(mask_init_value)
         self._offs_s = offs_s
+        self._cut, self._cut_w, self._cut_s = order.index(_DEC0), offs[_DEC0], offs_s.get(_DEC0)
         # padding elements of flat_s must never count as "kept" in the sparsity statistics
         pad = torch.ones_like(self.flat_s, dtype=torch.bool)
         for k in self.masked:
@@ -213,26 +256,21 @@ class OrtTrainer:
         self._has_saliency = False
 
     # ---------------------------------------------------------------------------------------------------------
+    def _view(self, flat, offs, first, count):
+        """View of a flat buffer over `count` consecutive same-shape parameters starting at `first` (e.g. [q;k;v]); the
+        generator alone spans its padded Vp rows."""
+        shp = self.p[first].shape
+        rows = self._pad_rows.get(first, shp[0]) if count == 1 else shp[0] * count
+        return flat[offs[first]: offs[first] + self.p[first].numel() // shp[0] * rows].view((rows,) + tuple(shp[1:]))
+
     def _group(self, table, first, count):
-        """Contiguous view over `count` consecutive same-shape parameters starting at `first` (e.g. [q;k;v])."""
-        shp = table[first].shape
-        offs = self._offs_w if table is self.p or table is self.g else self._offs_s
-        flat = {id(self.p): self.flat_w, id(self.g): self.flat_gw, id(self.s): self.flat_s, id(self.gs): self.flat_gs}[id(table)]
-        n = table[first].numel()
-        if first in self._pad_rows and count == 1:
-            rows = self._pad_rows[first]
-            return flat[offs[first]: offs[first] + n // shp[0] * rows].view((rows,) + tuple(shp[1:]))
-        return flat[offs[first]: offs[first] + n * count].view((shp[0] * count,) + tuple(shp[1:]))
+        """_view of the flat buffer behind `table` (self.p, self.g, self.s or self.gs)."""
+        flat, offs = {id(self.p): (self.flat_w, self._offs_w), id(self.g): (self.flat_gw, self._offs_w),
+                      id(self.s): (self.flat_s, self._offs_s), id(self.gs): (self.flat_gs, self._offs_s)}[id(table)]
+        return self._view(flat, offs, first, count)
 
     def _u(self, first, count=1):
-        if self.flat_u is None:
-            return None
-        n = self.s[first].numel()
-        shp = self.s[first].shape
-        if first in self._pad_rows and count == 1:
-            rows = self._pad_rows[first]
-            return self.flat_u[self._offs_s[first]: self._offs_s[first] + n // shp[0] * rows].view((rows,) + tuple(shp[1:]))
-        return self.flat_u[self._offs_s[first]: self._offs_s[first] + n * count].view((shp[0] * count,) + tuple(shp[1:]))
+        return None if self.flat_u is None else self._view(self.flat_u, self._offs_s, first, count)
 
     def mask_mode(self):
         if not self.mask_type:
@@ -264,19 +302,11 @@ class OrtTrainer:
     def _premask_keys(self):
         """(first weight name, fused count) of every linear the teacher-forcing forward runs, in launch order."""
         L = self.cfg.num_layers
-        keys = [("att_embed.0.weight", 1)]
-        for l in range(L):
-            p = f"model.encoder.layers.{l}"
-            keys += [(f"{p}.self_attn.linears.0.weight", 3), (f"{p}.self_attn.linears.3.weight", 1),
-                     (f"{p}.feed_forward.w_1.weight", 1), (f"{p}.feed_forward.w_2.weight", 1)]
-        keys += [(f"model.decoder.layers.{l}.src_attn.linears.1.weight", 2) for l in range(L)]
-        for l in range(L):
-            p = f"model.decoder.layers.{l}"
-            keys += [(f"{p}.self_attn.linears.0.weight", 3), (f"{p}.self_attn.linears.3.weight", 1),
-                     (f"{p}.src_attn.linears.0.weight", 1), (f"{p}.src_attn.linears.3.weight", 1),
-                     (f"{p}.feed_forward.w_1.weight", 1), (f"{p}.feed_forward.w_2.weight", 1)]
-        keys.append(("model.generator.proj.weight", 1))
-        return keys
+        enc = [(w, n) for l in range(L) for w, n, _ in self._groups["encoder", l]]
+        dec = [(w, n, slot) for l in range(L) for w, n, slot in self._groups["decoder", l]]
+        # (the memory's [k;v] of every decoder layer is projected right after the encoder)
+        return ([("att_embed.0.weight", 1)] + enc + [(w, n) for w, n, slot in dec if slot == "ckv"]
+                + [(w, n) for w, n, slot in dec if slot != "ckv"] + [("model.generator.proj.weight", 1)])
 
     def _premask_all(self):
         """W (.) m (bf16) and its transpose for EVERY linear of the step in one launch (sc_apply_mask_batched): the forward
@@ -334,10 +364,7 @@ class OrtTrainer:
         dim_g = 64 if not c.no_box_trigonometric_embedding else 4
         ws.wg_eff_all = torch.zeros(L * h, dim_g, **f32)
         ws.wg_eff = [ws.wg_eff_all[l * h: (l + 1) * h] for l in range(L)]
-        # all WG biases as one [L*h] view when the layout packed them without padding (h % 4 == 0)
-        b0 = self._offs_w["model.encoder.layers.0.self_attn.WGs.0.bias"]
-        packed = all(self._offs_w[f"model.encoder.layers.{l}.self_attn.WGs.{j}.bias"] == b0 + l * h + j for l in range(L) for j in range(h))
-        ws.wg_b_all = self.flat_w[b0: b0 + L * h] if packed else None
+        ws.wg_b_all = self._wg_b_all
         ws.mem = torch.zeros(ME, d, **a)
         ws.memkv = [torch.zeros(ME, 2 * d, **a) for _ in range(L)]
         ws.y = [torch.zeros(MD, d, **f32) for _ in range(3 * L + 1)]
@@ -533,19 +560,22 @@ class OrtTrainer:
         return ws.gb_ring[slot][: M * N].view(M, N), slot
 
     def _ln_bwd(self, name, x, dy, dx, dres=None, nxt=None, ws=None):
-        """Backward of LayerNorm `name`.  ``nxt = (weight name, dropout p, site)``: the linear whose output gradient is dx
+        """Backward of LayerNorm `name`.  ``nxt = (weight name, dropout site)``: the linear whose output gradient is dx
         comes next in the backward chain - its bf16 gradient operand (dropout mask regenerated) and bias gradient are
         produced by the same kernel; returns ``pre`` for ``_lin_bwd`` (None when not fused)."""
         d = x.shape[1]
         if nxt is None or self.adt != torch.bfloat16 or d != 512 or len(ws.gb_ring) < 2:
             K.layernorm_bwd(x, self.p[name + ".a_2"], dy, dx, self.g[name + ".a_2"], self.g[name + ".b_2"], dres=dres)
             return None
-        wname, p, site = nxt
+        wname, site = nxt
         gb, slot = self._take_gb(ws, x.shape[0], d)
         gbias = self.g[wname.replace(".weight", ".bias")]
         K.layernorm_bwd(x, self.p[name + ".a_2"], dy, dx, self.g[name + ".a_2"], self.g[name + ".b_2"], dres=dres, next_gb=gb,
-                        next_colsum=gbias, next_p=p if self.training else 0.0, seed=self._sd(1), stream_id=self._drop_stream(site))
+                        next_colsum=gbias, next_p=self._pd(), seed=self._sd(1), stream_id=self._drop_stream(site))
         return gb, slot
+
+    def _pd(self):
+        return self.p_drop if self.training else 0.0
 
     # ---------------------------------------------------------------------------------------------------------
     def load_batch(self, ws, att_feats, boxes, seqs, masks, att_masks=None, global_tokens=None):
@@ -571,13 +601,14 @@ class OrtTrainer:
         B, N, S, T, ME, MD, R = ws.B, ws.N, ws.S, ws.T, ws.ME, ws.MD, ws.R
         d, h, L = c.d_model, c.num_heads, c.num_layers
         dk = d // h
-        pd = self.p_drop if self.training else 0.0
+        pd = self._pd()
         trig = not c.no_box_trigonometric_embedding
+        es, ds = _SITES["encoder"], _SITES["decoder"]
         if ws.att_a is not ws.att_in:
             K.cast_bf16(ws.att_in, out=ws.att_a)
         if self.adt == torch.bfloat16 and self.premask and self.training and not self._scst:
             self._premask_all()
-        self._lin("att_embed.0.weight", ws.att_a, ws.xe[0], relu=True, p=self.p_src, site=1)
+        self._lin("att_embed.0.weight", ws.att_a, ws.xe[0], relu=True, p=self.p_src, site=_SITES["att_embed"])
         if ws.att_mask is not None:
             K.mask_rows(ws.xe[0], ws.att_mask.view(-1))
         # effective (masked) WG weights of every layer, then the log-geometry bias of all layers and heads in ONE pass over
@@ -601,11 +632,11 @@ class OrtTrainer:
             q = ws.e_qkv[l]
             K.attention_fwd(q[:, 0:], q[:, d:], q[:, 2 * d:], ws.e_att[l], ws.e_probs[l], G=B, Tq=N, Tk=N, h=h, dk=dk, ldq=3 * d,
                             ldk=3 * d, ldv=3 * d, ldo=d, key_valid=ws.att_mask, bias=ws.e_bias[l], p=pd, seed=self._sd(2),
-                            stream_id=self._drop_stream(10 + l))
-            self._lin(f"{p}.self_attn.linears.3.weight", ws.e_att[l], x1, residual=x0, p=pd, site=20 + l)
+                            stream_id=self._drop_stream(es["attn"] + l))
+            self._lin(f"{p}.self_attn.linears.3.weight", ws.e_att[l], x1, residual=x0, p=pd, site=es["o"] + l)
             self._ln(f"{p}.sublayer.1.norm", x1, ws.e_xn2[l])
-            self._lin(f"{p}.feed_forward.w_1.weight", ws.e_xn2[l], ws.e_hid[l], relu=True, p=pd, site=30 + l)
-            self._lin(f"{p}.feed_forward.w_2.weight", ws.e_hid[l], x2, residual=x1, p=pd, site=40 + l)
+            self._lin(f"{p}.feed_forward.w_1.weight", ws.e_xn2[l], ws.e_hid[l], relu=True, p=pd, site=es["ff1"] + l)
+            self._lin(f"{p}.feed_forward.w_2.weight", ws.e_hid[l], x2, residual=x1, p=pd, site=es["ff2"] + l)
         self._ln("model.encoder.norm", ws.xe[2 * L], ws.mem)
         for l in range(L):
             self._lin(f"model.decoder.layers.{l}.src_attn.linears.1.weight", ws.mem, ws.memkv[l], count=2)
@@ -613,7 +644,7 @@ class OrtTrainer:
         W, S_, mode, U, seed, stream = self._mask_args("model.tgt_embed.0.lut.weight")
         K.embed_pe(ws.tokens, W, self.pe, T=T, pos0=0, mask=S_, mask_mode=mode, uniforms=U, seed=seed, stream_id=stream, out=ws.y[0])
         if pd > 0:
-            K.prep_grad(ws.y[0], out=ws.y[0], p=pd, seed=self._sd(1), stream_id=self._drop_stream(2))
+            K.prep_grad(ws.y[0], out=ws.y[0], p=pd, seed=self._sd(1), stream_id=self._drop_stream(_SITES["embed"]))
         for l in range(L):
             p = f"model.decoder.layers.{l}"
             y0, y1, y2, y3 = ws.y[3 * l], ws.y[3 * l + 1], ws.y[3 * l + 2], ws.y[3 * l + 3]
@@ -622,18 +653,18 @@ class OrtTrainer:
             q = ws.d_qkv[l]
             K.attention_fwd(q[:, 0:], q[:, d:], q[:, 2 * d:], ws.d_att[l], ws.d_probs[l], G=R, Tq=T, Tk=T, h=h, dk=dk, ldq=3 * d,
                             ldk=3 * d, ldv=3 * d, ldo=d, key_valid=ws.key_valid, causal_T=T, p=pd, seed=self._sd(2),
-                            stream_id=self._drop_stream(50 + l))
-            self._lin(f"{p}.self_attn.linears.3.weight", ws.d_att[l], y1, residual=y0, p=pd, site=60 + l)
+                            stream_id=self._drop_stream(ds["attn"] + l))
+            self._lin(f"{p}.self_attn.linears.3.weight", ws.d_att[l], y1, residual=y0, p=pd, site=ds["o"] + l)
             self._ln(f"{p}.sublayer.1.norm", y1, ws.d_yn2[l])
             self._lin(f"{p}.src_attn.linears.0.weight", ws.d_yn2[l], ws.d_qc[l])
             kv = ws.memkv[l]
             K.attention_fwd(ws.d_qc[l], kv[:, 0:], kv[:, d:], ws.d_catt[l], ws.c_probs[l], G=B, Tq=S * T, Tk=N, h=h, dk=dk, ldq=d,
                             ldk=2 * d, ldv=2 * d, ldo=d, key_valid=ws.att_mask, p=pd, seed=self._sd(2),
-                            stream_id=self._drop_stream(70 + l))
-            self._lin(f"{p}.src_attn.linears.3.weight", ws.d_catt[l], y2, residual=y1, p=pd, site=80 + l)
+                            stream_id=self._drop_stream(ds["cattn"] + l))
+            self._lin(f"{p}.src_attn.linears.3.weight", ws.d_catt[l], y2, residual=y1, p=pd, site=ds["co"] + l)
             self._ln(f"{p}.sublayer.2.norm", y2, ws.d_yn3[l])
-            self._lin(f"{p}.feed_forward.w_1.weight", ws.d_yn3[l], ws.d_hid[l], relu=True, p=pd, site=90 + l)
-            self._lin(f"{p}.feed_forward.w_2.weight", ws.d_hid[l], y3, residual=y2, p=pd, site=100 + l)
+            self._lin(f"{p}.feed_forward.w_1.weight", ws.d_yn3[l], ws.d_hid[l], relu=True, p=pd, site=ds["ff1"] + l)
+            self._lin(f"{p}.feed_forward.w_2.weight", ws.d_hid[l], y3, residual=y2, p=pd, site=ds["ff2"] + l)
         self._ln("model.decoder.norm", ws.y[3 * L], ws.yf)
         self._lin("model.generator.proj.weight", ws.yf, ws.logits)
         return ws.logits
@@ -665,7 +696,7 @@ class OrtTrainer:
                     i += 1
                 return offs[self.names[i]] if i < len(self.names) else None
             return at(first), at(last)
-        dec0, dech = "model.decoder.layers.0.self_attn.linears.0.weight", f"model.decoder.layers.{half}.self_attn.linears.0.weight"
+        dec0, dech = _DEC0, f"model.decoder.layers.{half}.self_attn.linears.0.weight"
         lut, gen = "model.tgt_embed.0.lut.weight", "model.generator.proj.weight"
         ench = f"model.encoder.layers.{half}.self_attn.linears.0.weight"
         spans = {0: [(dech, lut), (gen, None)], 1: [(dec0, dech), (lut, gen)], 2: [(ench, dec0)], 3: [(self.names[0], ench)]}[phase]
@@ -682,113 +713,50 @@ class OrtTrainer:
         return out
 
     def backward_phase(self, ws, phase):
-        c = self.cfg
-        B, N, S, T, ME, MD, R = ws.B, ws.N, ws.S, ws.T, ws.ME, ws.MD, ws.R
-        d, h, L, ff = c.d_model, c.num_heads, c.num_layers, c.dim_feedforward
-        dk = d // h
-        pd = self.p_drop if self.training else 0.0
-        trig = not c.no_box_trigonometric_embedding
+        d, L = self.cfg.d_model, self.cfg.num_layers
+        pd = self._pd()
         ws.gb_free = [None] * len(ws.gb_ring)
         ws.gb_next = 0
         ws.side_used = False
-        half = L // 2
+        stack = "decoder" if phase < 2 else "encoder"
+        last_ff2 = (f"model.{stack}.layers.{L - 1}.feed_forward.w_2.weight", _SITES[stack]["ff2"] + L - 1)
+        pre = None  # (a phase starts with a plain gradient preparation: the ring was reset)
         if phase == 0:
             self._materialized = False
             # norm and bias gradients accumulate through atomics: one memset of the flat buffer (weights are overwritten)
             self.flat_gw.zero_()
             ws.loss_sum.zero_()
             K.logsoftmax_nll(ws.logits, ws.targets, ws.tok_w, ws.inv_norm, ws.loss_sum, ws.dlogits)
-            ga_d = ws.ga.view(-1)[: MD * d].view(MD, d)
+            ga_d = ws.ga.view(-1)[: ws.MD * d].view(ws.MD, d)
             self._lin_bwd(ws, "model.generator.proj.weight", ws.yf, None, g_ready=ws.dlogits, dx=ga_d)
             ws.cur = 0
-            pre = self._ln_bwd("model.decoder.norm", ws.y[3 * L], ga_d, ws.dres[0][:MD], ws=ws,
-                               nxt=(f"model.decoder.layers.{L - 1}.feed_forward.w_2.weight", pd, 100 + L - 1))
+            pre = self._ln_bwd("model.decoder.norm", ws.y[3 * L], ga_d, ws.dres[0][:ws.MD], ws=ws, nxt=last_ff2)
             ws.dmem.zero_()
-        if phase >= 2:
-            self._backward_encoder(ws, phase - 2)
-            return
-        if phase != 0:
-            pre = None  # (a phase starts with a plain gradient preparation: the ring was reset)
-        first = half if phase == 0 else 0  # last layer this phase visits
-        cur, nxt = ws.dres[ws.cur][:MD], ws.dres[1 - ws.cur][:MD]
-        for l in (reversed(range(half, L)) if phase == 0 else reversed(range(half))):
-            p = f"model.decoder.layers.{l}"
-            y0, y1, y2 = ws.y[3 * l], ws.y[3 * l + 1], ws.y[3 * l + 2]
-            ga_ff = ws.ga.view(-1)[: MD * ff].view(MD, ff)
-            # feed-forward sublayer
-            pre1 = self._lin_bwd(ws, f"{p}.feed_forward.w_2.weight", ws.d_hid[l], cur, p=pd, site=100 + l, dx=ga_ff, pre=pre,
-                                 dx_next=(ws.d_hid[l], 1.0 / (1.0 - pd) if pd > 0 else 1.0, f"{p}.feed_forward.w_1.weight"))
-            ga_dd = ws.gq.view(-1)[: MD * d].view(MD, d)
-            self._lin_bwd(ws, f"{p}.feed_forward.w_1.weight", ws.d_yn3[l], ga_ff, h=ws.d_hid[l], p=pd, dx=ga_dd, pre=pre1)
-            pre = self._ln_bwd(f"{p}.sublayer.2.norm", y2, ga_dd, nxt, dres=cur, ws=ws, nxt=(f"{p}.src_attn.linears.3.weight", pd, 80 + l))
-            cur, nxt = nxt, cur
-            # cross-attention sublayer
-            ga_c = ws.ga.view(-1)[: MD * d].view(MD, d)
-            self._lin_bwd(ws, f"{p}.src_attn.linears.3.weight", ws.d_catt[l], cur, p=pd, site=80 + l, dx=ga_c, pre=pre)
-            kv = ws.memkv[l]
-            dqc = ws.gq.view(-1)[: MD * d].view(MD, d)
-            pre_q = pre_kv = None
-            if self._attn_fused(ws):
-                gbq, sq = self._take_gb(ws, MD, d)
-                gbkv, skv = self._take_gb(ws, ME, 2 * d)
-                bkv = self._group(self.g, f"{p}.src_attn.linears.1.bias", 2)
-                K.attention_bwd_bf16out(ws.d_qc[l], kv[:, 0:], kv[:, d:], ws.c_probs[l], ga_c, gbq, gbkv[:, 0:], gbkv[:, d:], G=B,
-                                        Tq=S * T, Tk=N, h=h, dk=dk, ldq=d, ldk=2 * d, ldv=2 * d, ldd=d, ldgq=d, ldgk=2 * d, ldgv=2 * d,
-                                        bq=self.g[f"{p}.src_attn.linears.0.bias"], bk=bkv[:d], bv=bkv[d:], p=pd, seed=self._sd(2),
-                                        stream_id=self._drop_stream(70 + l))
-                pre_q, pre_kv = (gbq, sq), (gbkv, skv)
+        elif phase == 2:
+            ws.cur = 0
+            pre = self._ln_bwd("model.encoder.norm", ws.xe[2 * L], ws.dmem, ws.dres[0][:ws.ME], ws=ws, nxt=last_ff2)
+        cur = self._backward_layers(ws, stack, range(L // 2, L) if phase % 2 == 0 else range(L // 2), pre)
+        if phase == 1:
+            # embedding: its dropout mask is regenerated from the forward's Philox stream (an exact zero in the saved output is
+            # not proof of a dropped element: sin(0) = 0 in the positional encoding, masked-out table entries)
+            W, S_, mode, U, seed, stream = self._mask_args("model.tgt_embed.0.lut.weight")
+            emb_g = ws.ga.view(-1)[: ws.MD * d].view(ws.MD, d)
+            if pd > 0:
+                K.prep_grad(cur, out=emb_g, p=pd, seed=self._sd(1), stream_id=self._drop_stream(_SITES["embed"]))
             else:
-                K.attention_bwd(ws.d_qc[l], kv[:, 0:], kv[:, d:], ws.c_probs[l], ga_c, dqc, ws.dmemkv[:, 0:], ws.dmemkv[:, d:],
-                                dtype=self.adt, G=B, Tq=S * T, Tk=N, h=h, dk=dk, ldq=d, ldk=2 * d, ldv=2 * d, ldd=d, ldgq=d, ldgk=2 * d,
-                                ldgv=2 * d, p=pd, seed=self._sd(2), stream_id=self._drop_stream(70 + l))
-            ga_c2 = ws.ga.view(-1)[: MD * d].view(MD, d)
-            self._lin_bwd(ws, f"{p}.src_attn.linears.0.weight", ws.d_yn2[l], dqc, dx=ga_c2, pre=pre_q)
-            pre = self._ln_bwd(f"{p}.sublayer.1.norm", y1, ga_c2, nxt, dres=cur, ws=ws, nxt=(f"{p}.self_attn.linears.3.weight", pd, 60 + l))
-            cur, nxt = nxt, cur
-            self._lin_bwd(ws, f"{p}.src_attn.linears.1.weight", ws.mem, ws.dmemkv, count=2, dx=ws.dmem, dx_residual=ws.dmem, pre=pre_kv)
-            # self-attention sublayer
-            ga_s = ws.ga.view(-1)[: MD * d].view(MD, d)
-            self._lin_bwd(ws, f"{p}.self_attn.linears.3.weight", ws.d_att[l], cur, p=pd, site=60 + l, dx=ga_s, pre=pre)
-            q = ws.d_qkv[l]
-            gq = ws.gq[:MD]
-            pre_qkv = None
-            if self._attn_fused(ws):
-                gb3, s3 = self._take_gb(ws, MD, 3 * d)
-                b3 = self._group(self.g, f"{p}.self_attn.linears.0.bias", 3)
-                K.attention_bwd_bf16out(q[:, 0:], q[:, d:], q[:, 2 * d:], ws.d_probs[l], ga_s, gb3[:, 0:], gb3[:, d:], gb3[:, 2 * d:], G=R,
-                                        Tq=T, Tk=T, h=h, dk=dk, ldq=3 * d, ldk=3 * d, ldv=3 * d, ldd=d, ldgq=3 * d, ldgk=3 * d,
-                                        ldgv=3 * d, bq=b3[:d], bk=b3[d: 2 * d], bv=b3[2 * d:], p=pd, seed=self._sd(2),
-                                        stream_id=self._drop_stream(50 + l))
-                pre_qkv = (gb3, s3)
+                emb_g = cur
+            if self.fused_st:
+                # (flat_gw was zeroed at the start of the backward: the scatter-add lands directly in the table's gradient view)
+                K.embedding_bwd(ws.tokens, emb_g, self.g["model.tgt_embed.0.lut.weight"], math.sqrt(d))
             else:
-                K.attention_bwd(q[:, 0:], q[:, d:], q[:, 2 * d:], ws.d_probs[l], ga_s, gq[:, 0:], gq[:, d:], gq[:, 2 * d:], dtype=self.adt,
-                                G=R, Tq=T, Tk=T, h=h, dk=dk, ldq=3 * d, ldk=3 * d, ldv=3 * d, ldd=d, ldgq=3 * d, ldgk=3 * d, ldgv=3 * d,
-                                p=pd, seed=self._sd(2), stream_id=self._drop_stream(50 + l))
-            ga_s2 = ws.ga.view(-1)[: MD * d].view(MD, d)
-            self._lin_bwd(ws, f"{p}.self_attn.linears.0.weight", ws.d_yn1[l], gq, count=3, dx=ga_s2, pre=pre_qkv)
-            pre = self._ln_bwd(f"{p}.sublayer.0.norm", y0, ga_s2, nxt, dres=cur, ws=ws,
-                               nxt=(f"model.decoder.layers.{l - 1}.feed_forward.w_2.weight", pd, 100 + l - 1) if l > first else None)
-            cur, nxt = nxt, cur
-        ws.cur = 0 if cur.data_ptr() == ws.dres[0].data_ptr() else 1
-        if phase == 0:
-            self._join_side(ws)
-            return
-        # embedding: its dropout mask is regenerated from the forward's Philox stream (an exact zero in the saved output is
-        # not proof of a dropped element: sin(0) = 0 in the positional encoding, masked-out table entries)
-        W, S_, mode, U, seed, stream = self._mask_args("model.tgt_embed.0.lut.weight")
-        emb_g = ws.ga.view(-1)[: MD * d].view(MD, d)
-        if pd > 0:
-            K.prep_grad(cur, out=emb_g, p=pd, seed=self._sd(1), stream_id=self._drop_stream(2))
-        else:
-            emb_g = cur
-        if self.fused_st:
-            # (flat_gw was zeroed at the start of the backward: the scatter-add lands directly in the table's gradient view)
-            K.embedding_bwd(ws.tokens, emb_g, self.g["model.tgt_embed.0.lut.weight"], math.sqrt(d))
-        else:
-            ws.dtable.zero_()
-            K.embedding_bwd(ws.tokens, emb_g, ws.dtable, math.sqrt(d))
-            K.mask_grad(ws.dtable, W, S_, mode, self.g["model.tgt_embed.0.lut.weight"],
-                        self.gs.get("model.tgt_embed.0.lut.weight"), uniforms=U, seed=seed, stream_id=stream, bypass=self.bypass)
+                ws.dtable.zero_()
+                K.embedding_bwd(ws.tokens, emb_g, ws.dtable, math.sqrt(d))
+                K.mask_grad(ws.dtable, W, S_, mode, self.g["model.tgt_embed.0.lut.weight"],
+                            self.gs.get("model.tgt_embed.0.lut.weight"), uniforms=U, seed=seed, stream_id=stream, bypass=self.bypass)
+        elif phase == 3:
+            if ws.att_mask is not None:
+                K.mask_rows(cur, ws.att_mask.view(-1))
+            self._lin_bwd(ws, "att_embed.0.weight", ws.att_a, cur, h=ws.xe[0], p=self.p_src if self.training else 0.0)
         self._join_side(ws)
 
     def _join_side(self, ws):
@@ -796,75 +764,108 @@ class OrtTrainer:
             torch.cuda.current_stream(self.dev).wait_stream(self._side_stream())
             ws.side_used = False
 
-    def _backward_encoder(self, ws, part):
-        """part 0: encoder norm + layers L-1 .. L/2 ; part 1: layers L/2-1 .. 0 + att_embed."""
-        c = self.cfg
-        B, N, S, T, ME, MD, R = ws.B, ws.N, ws.S, ws.T, ws.ME, ws.MD, ws.R
-        d, h, L, ff = c.d_model, c.num_heads, c.num_layers, c.dim_feedforward
-        dk = d // h
-        pd = self.p_drop if self.training else 0.0
-        trig = not c.no_box_trigonometric_embedding
-        half = L // 2
-        pre = None
-        if part == 0:
-            ws.cur = 0
-            pre = self._ln_bwd("model.encoder.norm", ws.xe[2 * L], ws.dmem, ws.dres[0][:ME], ws=ws,
-                               nxt=(f"model.encoder.layers.{L - 1}.feed_forward.w_2.weight", pd, 40 + L - 1))
-        first = half if part == 0 else 0
-        cur, nxt = ws.dres[ws.cur][:ME], ws.dres[1 - ws.cur][:ME]
-        for l in (reversed(range(half, L)) if part == 0 else reversed(range(half))):
-            p = f"model.encoder.layers.{l}"
-            x0, x1 = ws.xe[2 * l], ws.xe[2 * l + 1]
-            ga_ff = ws.ga.view(-1)[: ME * ff].view(ME, ff)
-            pre1 = self._lin_bwd(ws, f"{p}.feed_forward.w_2.weight", ws.e_hid[l], cur, p=pd, site=40 + l, dx=ga_ff, pre=pre,
-                                 dx_next=(ws.e_hid[l], 1.0 / (1.0 - pd) if pd > 0 else 1.0, f"{p}.feed_forward.w_1.weight"))
-            ga_dd = ws.gq.view(-1)[: ME * d].view(ME, d)
-            self._lin_bwd(ws, f"{p}.feed_forward.w_1.weight", ws.e_xn2[l], ga_ff, h=ws.e_hid[l], p=pd, dx=ga_dd, pre=pre1)
-            pre = self._ln_bwd(f"{p}.sublayer.1.norm", x1, ga_dd, nxt, dres=cur, ws=ws, nxt=(f"{p}.self_attn.linears.3.weight", pd, 20 + l))
+    def _backward_layers(self, ws, stack, layers, pre):
+        """Backward of `layers` of a stack, last first: each sublayer reads the residual-stream gradient from `cur`, its LayerNorm
+        backward writes it plus the sublayer's input gradient to `nxt` (ping-pong over ws.dres; ws.cur: the current one)."""
+        s, M = _SITES[stack], ws.MD if stack == "decoder" else ws.ME
+        cur, nxt = ws.dres[ws.cur][:M], ws.dres[1 - ws.cur][:M]
+        for l in reversed(layers):
+            p = f"model.{stack}.layers.{l}"
+            o = (f"{p}.self_attn.linears.3.weight", s["o"] + l)   # (an _ln_bwd hand-off: weight, dropout site)
+            if stack == "decoder":
+                pre = self._ff_bwd(ws, stack, l, cur, nxt, pre, (f"{p}.src_attn.linears.3.weight", s["co"] + l))
+                cur, nxt = nxt, cur
+                pre = self._cross_attn_bwd(ws, l, cur, nxt, pre, o)
+            else:
+                pre = self._ff_bwd(ws, stack, l, cur, nxt, pre, o)
             cur, nxt = nxt, cur
-            ga_a = ws.ga.view(-1)[: ME * d].view(ME, d)
-            self._lin_bwd(ws, f"{p}.self_attn.linears.3.weight", ws.e_att[l], cur, p=pd, site=20 + l, dx=ga_a, pre=pre)
-            q = ws.e_qkv[l]
-            gq = ws.gq[:ME]
-            pre_qkv = None
-            if self._attn_fused(ws):
-                gb3, s3 = self._take_gb(ws, ME, 3 * d)
-                b3 = self._group(self.g, f"{p}.self_attn.linears.0.bias", 3)
-                K.attention_bwd_bf16out(q[:, 0:], q[:, d:], q[:, 2 * d:], ws.e_probs[l], ga_a, gb3[:, 0:], gb3[:, d:], gb3[:, 2 * d:], G=B,
-                                        Tq=N, Tk=N, h=h, dk=dk, ldq=3 * d, ldk=3 * d, ldv=3 * d, ldd=d, ldgq=3 * d, ldgk=3 * d,
-                                        ldgv=3 * d, bq=b3[:d], bk=b3[d: 2 * d], bv=b3[2 * d:], dbias=ws.dbias, p=pd, seed=self._sd(2),
-                                        stream_id=self._drop_stream(10 + l))
-                pre_qkv = (gb3, s3)
-            else:
-                K.attention_bwd(q[:, 0:], q[:, d:], q[:, 2 * d:], ws.e_probs[l], ga_a, gq[:, 0:], gq[:, d:], gq[:, 2 * d:], dtype=self.adt,
-                                G=B, Tq=N, Tk=N, h=h, dk=dk, ldq=3 * d, ldk=3 * d, ldv=3 * d, ldd=d, ldgq=3 * d, ldgk=3 * d, ldgv=3 * d,
-                                dbias=ws.dbias, p=pd, seed=self._sd(2), stream_id=self._drop_stream(10 + l))
-            gb_wg = self._group(self.g, f"{p}.self_attn.WGs.0.bias", h)
-            gb_wg.zero_()
-            if self.fused_st:
-                gw_wg = self._group(self.g, f"{p}.self_attn.WGs.0.weight", h)
-                gw_wg.zero_()
-                K.box_bias_bwd(ws.boxes, ws.e_bias[l], ws.dbias, gw_wg, gb_wg, B=B, N=N, h=h, trig=trig)
-            else:
-                ws.dwg.zero_()
-                K.box_bias_bwd(ws.boxes, ws.e_bias[l], ws.dbias, ws.dwg, gb_wg, B=B, N=N, h=h, trig=trig)
-                Wg, Sg, mode, U, seed, stream = self._mask_args(f"{p}.self_attn.WGs.0.weight", h)
-                K.mask_grad(ws.dwg, Wg, Sg, mode, self._group(self.g, f"{p}.self_attn.WGs.0.weight", h),
-                            self._group(self.gs, f"{p}.self_attn.WGs.0.weight", h) if Sg is not None else None, uniforms=U, seed=seed,
-                            stream_id=stream, bypass=self.bypass)
-            ga_a2 = ws.ga.view(-1)[: ME * d].view(ME, d)
-            self._lin_bwd(ws, f"{p}.self_attn.linears.0.weight", ws.e_xn1[l], gq, count=3, dx=ga_a2, pre=pre_qkv)
-            pre = self._ln_bwd(f"{p}.sublayer.0.norm", x0, ga_a2, nxt, dres=cur, ws=ws,
-                               nxt=(f"model.encoder.layers.{l - 1}.feed_forward.w_2.weight", pd, 40 + l - 1) if l > first else None)
+            # (the previous layer's w_2 only within this phase: the next one starts with a reset ring)
+            ff2 = (f"model.{stack}.layers.{l - 1}.feed_forward.w_2.weight", s["ff2"] + l - 1) if l > layers[0] else None
+            pre = self._self_attn_bwd(ws, stack, l, cur, nxt, pre, ff2)
             cur, nxt = nxt, cur
         ws.cur = 0 if cur.data_ptr() == ws.dres[0].data_ptr() else 1
-        if part == 0:
-            self._join_side(ws)
-            return
-        if ws.att_mask is not None:
-            K.mask_rows(cur, ws.att_mask.view(-1))
-        self._lin_bwd(ws, "att_embed.0.weight", ws.att_a, cur, h=ws.xe[0], p=self.p_src if self.training else 0.0)
-        self._join_side(ws)
+        return cur
+
+    def _ff_bwd(self, ws, stack, l, cur, nxt, pre, then):
+        """Feed-forward sublayer: w_2 (its dX GEMM prepares w_1's gradient operand), w_1, LayerNorm (``then``: its _ln_bwd nxt)."""
+        p, pd = f"model.{stack}.layers.{l}", self._pd()
+        if stack == "decoder":
+            x, xn, hid, norm = ws.y[3 * l + 2], ws.d_yn3[l], ws.d_hid[l], f"{p}.sublayer.2.norm"
+        else:
+            x, xn, hid, norm = ws.xe[2 * l + 1], ws.e_xn2[l], ws.e_hid[l], f"{p}.sublayer.1.norm"
+        (M, ff), d = hid.shape, x.shape[1]
+        ga_ff = ws.ga.view(-1)[: M * ff].view(M, ff)
+        pre1 = self._lin_bwd(ws, f"{p}.feed_forward.w_2.weight", hid, cur, p=pd, site=_SITES[stack]["ff2"] + l, dx=ga_ff, pre=pre,
+                             dx_next=(hid, 1.0 / (1.0 - pd) if pd > 0 else 1.0, f"{p}.feed_forward.w_1.weight"))
+        ga = ws.gq.view(-1)[: M * d].view(M, d)
+        self._lin_bwd(ws, f"{p}.feed_forward.w_1.weight", xn, ga_ff, h=hid, p=pd, dx=ga, pre=pre1)
+        return self._ln_bwd(norm, x, ga, nxt, dres=cur, ws=ws, nxt=then)
+
+    def _self_attn_bwd(self, ws, stack, l, cur, nxt, pre, then):
+        """Self-attention sublayer: output linear, attention (encoder: + the geometry bias), [q;k;v], LayerNorm."""
+        p = f"model.{stack}.layers.{l}"
+        enc = stack == "encoder"
+        if enc:
+            x, xn, qkv, probs, att, G, T = ws.xe[2 * l], ws.e_xn1[l], ws.e_qkv[l], ws.e_probs[l], ws.e_att[l], ws.B, ws.N
+        else:
+            x, xn, qkv, probs, att, G, T = ws.y[3 * l], ws.d_yn1[l], ws.d_qkv[l], ws.d_probs[l], ws.d_att[l], ws.R, ws.T
+        M, d = x.shape
+        ga, gq = ws.ga.view(-1)[: M * d].view(M, d), ws.gq[:M]
+        self._lin_bwd(ws, f"{p}.self_attn.linears.3.weight", att, cur, p=self._pd(), site=_SITES[stack]["o"] + l, dx=ga, pre=pre)
+        pre_qkv, = self._attn_bwd(ws, f"{p}.self_attn", qkv, qkv[:, d:], probs, ga, gq, gq[:, d:], G=G, Tq=T, Tk=T,
+                                  site=_SITES[stack]["attn"] + l, dbias=ws.dbias if enc else None)
+        if enc:
+            self._box_bias_bwd(ws, l)
+        self._lin_bwd(ws, f"{p}.self_attn.linears.0.weight", xn, gq, count=3, dx=ga, pre=pre_qkv)
+        return self._ln_bwd(f"{p}.sublayer.0.norm", x, ga, nxt, dres=cur, ws=ws, nxt=then)
+
+    def _cross_attn_bwd(self, ws, l, cur, nxt, pre, then):
+        """Decoder cross-attention sublayer: output linear, attention, q, LayerNorm, then the memory's [k;v] (into ws.dmem)."""
+        p, MD, d = f"model.decoder.layers.{l}", ws.MD, self.cfg.d_model
+        ga, dq = ws.ga.view(-1)[: MD * d].view(MD, d), ws.gq.view(-1)[: MD * d].view(MD, d)
+        self._lin_bwd(ws, f"{p}.src_attn.linears.3.weight", ws.d_catt[l], cur, p=self._pd(), site=_SITES["decoder"]["co"] + l, dx=ga,
+                      pre=pre)
+        pre_q, pre_kv = self._attn_bwd(ws, f"{p}.src_attn", ws.d_qc[l], ws.memkv[l], ws.c_probs[l], ga, dq, ws.dmemkv, G=ws.B,
+                                       Tq=ws.S * ws.T, Tk=ws.N, site=_SITES["decoder"]["cattn"] + l)
+        self._lin_bwd(ws, f"{p}.src_attn.linears.0.weight", ws.d_yn2[l], dq, dx=ga, pre=pre_q)
+        pre = self._ln_bwd(f"{p}.sublayer.1.norm", ws.y[3 * l + 1], ga, nxt, dres=cur, ws=ws, nxt=then)
+        self._lin_bwd(ws, f"{p}.src_attn.linears.1.weight", ws.mem, ws.dmemkv, count=2, dx=ws.dmem, dx_residual=ws.dmem, pre=pre_kv)
+        return pre
+
+    def _attn_bwd(self, ws, pa, q, kv, probs, dout, dq, dkv, *, G, Tq, Tk, site, dbias=None):
+        """Attention backward of module `pa`: fp32 dq / d[k;v], or (_attn_fused) bf16 gradient operands with the bias gradients.
+        Returns the _lin_bwd ``pre`` of ([q;k;v],) (self-attention: kv is a view of q) or of (q, [k;v]) (cross-attention)."""
+        d, h = self.cfg.d_model, self.cfg.num_heads
+        packed = pa.endswith("self_attn")
+        kw = dict(G=G, Tq=Tq, Tk=Tk, h=h, dk=d // h, ldq=q.stride(0), ldk=kv.stride(0), ldv=kv.stride(0), ldd=d, dbias=dbias,
+                  p=self._pd(), seed=self._sd(2), stream_id=self._drop_stream(site))
+        if not self._attn_fused(ws):
+            K.attention_bwd(q[:, 0:], kv[:, 0:], kv[:, d:], probs, dout, dq[:, 0:], dkv[:, 0:], dkv[:, d:], dtype=self.adt,
+                            ldgq=dq.stride(0), ldgk=dkv.stride(0), ldgv=dkv.stride(0), **kw)
+            return (None,) if packed else (None, None)
+        if packed:
+            gb, slot = self._take_gb(ws, q.shape[0], 3 * d)
+            gq, gkv, pre = gb, gb[:, d:], ((gb, slot),)
+        else:
+            pre = self._take_gb(ws, q.shape[0], d), self._take_gb(ws, kv.shape[0], 2 * d)
+            (gq, _), (gkv, _) = pre
+        bkv = self._group(self.g, f"{pa}.linears.1.bias", 2)
+        K.attention_bwd_bf16out(q[:, 0:], kv[:, 0:], kv[:, d:], probs, dout, gq[:, 0:], gkv[:, 0:], gkv[:, d:], ldgq=gq.stride(0),
+                                ldgk=gkv.stride(0), ldgv=gkv.stride(0), bq=self.g[f"{pa}.linears.0.bias"], bk=bkv[:d], bv=bkv[d:], **kw)
+        return pre
+
+    def _box_bias_bwd(self, ws, l):
+        """Geometry-bias backward of encoder layer l: WG bias gradients and dWm (fused_st) or dW / dS (sc_mask_grad) of its heads."""
+        h, wg = self.cfg.num_heads, f"model.encoder.layers.{l}.self_attn.WGs.0.weight"
+        gb_wg = self._group(self.g, f"model.encoder.layers.{l}.self_attn.WGs.0.bias", h)
+        gb_wg.zero_()
+        dwg = self._group(self.g, wg, h) if self.fused_st else ws.dwg
+        dwg.zero_()
+        K.box_bias_bwd(ws.boxes, ws.e_bias[l], ws.dbias, dwg, gb_wg, B=ws.B, N=ws.N, h=h, trig=not self.cfg.no_box_trigonometric_embedding)
+        if not self.fused_st:
+            Wg, Sg, mode, U, seed, stream = self._mask_args(wg, h)
+            K.mask_grad(ws.dwg, Wg, Sg, mode, self._group(self.g, wg, h), self._group(self.gs, wg, h) if Sg is not None else None,
+                        uniforms=U, seed=seed, stream_id=stream, bypass=self.bypass)
 
     # ---------------------------------------------------------------------------------------------------------
     def optimizer_step(self, *, lr, mask_lr=100.0, clip=0.1, betas=(0.9, 0.98), eps=1e-9, mask_eps=1e-2, weight_decay=0.0,
@@ -882,23 +883,14 @@ class OrtTrainer:
             return self._optimizer_step_st(lr=lr, mask_lr=mask_lr, clip=clip, betas=betas, eps=eps, mask_eps=mask_eps,
                                            weight_decay=weight_decay, grad_scale=grad_scale, sparsity_target=sparsity_target,
                                            sparsity_weight=sparsity_weight, current_step=current_step, max_step=max_step, dyn=dyn, part=part)
-        cut_w = self._offs_w["model.decoder.layers.0.self_attn.linears.0.weight"]
-        lo_w, hi_w = {"all": (0, self.flat_w.numel()), "hi": (cut_w, self.flat_w.numel()), "lo": (0, cut_w)}[part]
+        lo_w, hi_w = _part(self.flat_w.numel(), self._cut_w, part)
         K.adam_clip(self.flat_w[lo_w:hi_w], self.flat_gw[lo_w:hi_w], self.m_w[lo_w:hi_w], self.v_w[lo_w:hi_w], lr=lr, betas=betas, eps=eps,
                     weight_decay=weight_decay, clip=clip, grad_scale=grad_scale, step=max(1, self.opt_step),
                     dyn=dyn[0:3] if _dyn else None)
         if self.masked and self.mask_type == "supermask":
-            coeff = None
-            if sparsity_target is not None and sparsity_weight:
-                if part != "lo":
-                    anneal = (1.0 + math.cos(min(1.0, current_step / max_step) * math.pi)) / 2.0
-                    self.sp_count.zero_()
-                    K.lib.call("sc_mask_count", K.lib.ptr(self.flat_s), self.flat_s.numel(), K.lib.ptr(self.sp_count), K.lib.stream())
-                    K.sparsity_coeff(self.sp_count, self.n_logits, sparsity_target, sparsity_weight * (1.0 - anneal), self.sp_out,
-                                     scale_dev=dyn[6:7] if _dyn else None)
-                coeff = self.sp_out[1:2]
-            cut_s = self._offs_s["model.decoder.layers.0.self_attn.linears.0.weight"]
-            lo_s, hi_s = {"all": (0, self.flat_s.numel()), "hi": (cut_s, self.flat_s.numel()), "lo": (0, cut_s)}[part]
+            coeff = self._sparsity_coeff(sparsity_target=sparsity_target, sparsity_weight=sparsity_weight, current_step=current_step,
+                                         max_step=max_step, scale_dev=dyn[6:7] if _dyn else None, part=part)
+            lo_s, hi_s = _part(self.flat_s.numel(), self._cut_s, part)
             K.adam_clip(self.flat_s[lo_s:hi_s], self.flat_gs[lo_s:hi_s], self.m_s[lo_s:hi_s], self.v_s[lo_s:hi_s], lr=mask_lr, betas=betas,
                         eps=mask_eps, weight_decay=0.0, clip=clip, grad_scale=grad_scale, step=max(1, self.opt_step),
                         sigmoid_grad_coeff=coeff, dyn=dyn[3:6] if _dyn else None)
@@ -923,8 +915,7 @@ class OrtTrainer:
                     first_of[wname] = count
                     i = self.names.index(wname)
                     member.update(self.names[i + 1: i + count])  # (the fused members are consecutive names: [q;k;v], [k;v], WG heads)
-            cut = self.names.index("model.decoder.layers.0.self_attn.linears.0.weight")
-            names = {"all": self.names, "hi": self.names[cut:], "lo": self.names[:cut]}[part]
+            names = self.names[slice(*_part(len(self.names), self._cut, part))]
             segs = []
             for k in names:
                 if k in member:
@@ -941,15 +932,8 @@ class OrtTrainer:
     def _optimizer_step_st(self, *, lr, mask_lr, clip, betas, eps, mask_eps, weight_decay, grad_scale, sparsity_target, sparsity_weight,
                            current_step, max_step, dyn, part):
         supermask = bool(self.masked) and self.mask_type == "supermask"
-        coeff = None
-        if supermask and sparsity_target is not None and sparsity_weight:
-            if part != "lo":
-                anneal = (1.0 + math.cos(min(1.0, current_step / max_step) * math.pi)) / 2.0
-                self.sp_count.zero_()
-                K.lib.call("sc_mask_count", K.lib.ptr(self.flat_s), self.flat_s.numel(), K.lib.ptr(self.sp_count), K.lib.stream())
-                K.sparsity_coeff(self.sp_count, self.n_logits, sparsity_target, sparsity_weight * (1.0 - anneal), self.sp_out,
-                                 scale_dev=dyn[6:7] if dyn is not None else None)
-            coeff = self.sp_out[1:2]
+        coeff = self._sparsity_coeff(sparsity_target=sparsity_target, sparsity_weight=sparsity_weight, current_step=current_step,
+                                     max_step=max_step, scale_dev=dyn[6:7] if dyn is not None else None, part=part)
         desc, blocks = self._st_table(part)
         mode = K.MASK_NONE  # the mask sample of the step being applied (train-mode forward)
         if self.masked:
@@ -973,14 +957,17 @@ class OrtTrainer:
             K.mask_grad(gW, W, S, mode, gW, self._group(self.gs, wname, count), uniforms=U, seed=seed, stream_id=stream, bypass=self.bypass)
         self._materialized = True
 
-    def _sparsity_coeff(self, *, sparsity_target=None, sparsity_weight=0.0, current_step=0, max_step=1, **_):
-        """Device scalar d(sparsity loss)/d(nnz) from the CURRENT logits (must run before any logit is updated)."""
+    def _sparsity_coeff(self, *, sparsity_target=None, sparsity_weight=0.0, current_step=0, max_step=1, scale_dev=None, part="all",
+                        **_):
+        """Device scalar d(sparsity loss)/d(nnz) from the CURRENT logits (must run before any logit is updated; the "lo" half of
+        an overlapped update reuses the one its "hi" half computed), None without a sparsity loss.  ``scale_dev``: graph mode,
+        the annealed loss weight is read from the device."""
         if not (self.masked and self.mask_type == "supermask") or sparsity_target is None or not sparsity_weight:
             return None
-        anneal = (1.0 + math.cos(min(1.0, current_step / max_step) * math.pi)) / 2.0
-        self.sp_count.zero_()
-        K.lib.call("sc_mask_count", K.lib.ptr(self.flat_s), self.flat_s.numel(), K.lib.ptr(self.sp_count), K.lib.stream())
-        K.sparsity_coeff(self.sp_count, self.n_logits, sparsity_target, sparsity_weight * (1.0 - anneal), self.sp_out)
+        if part != "lo":
+            K.mask_count([self.flat_s], out=self.sp_count)
+            K.sparsity_coeff(self.sp_count, self.n_logits, sparsity_target, sparsity_weight * (1.0 - _anneal(current_step, max_step)),
+                             self.sp_out, scale_dev=scale_dev)
         return self.sp_out[1:2]
 
     def _sharded_step(self, ws, exchange, opt, lr):
@@ -1026,18 +1013,21 @@ class OrtTrainer:
         self._upload_seeds()
         bc1 = 1.0 - betas[0] ** self.opt_step
         bc2 = math.sqrt(1.0 - betas[1] ** self.opt_step)
-        anneal = (1.0 + math.cos(min(1.0, current_step / max_step) * math.pi)) / 2.0
         h = self._dyn_host
-        h[0], h[1], h[2], h[3], h[4], h[5], h[6] = lr, bc1, bc2, mask_lr, bc1, bc2, sparsity_weight * (1.0 - anneal)
+        h[0], h[1], h[2], h[3], h[4], h[5], h[6] = lr, bc1, bc2, mask_lr, bc1, bc2, sparsity_weight * (1.0 - _anneal(current_step, max_step))
         self._dyn_dev.copy_(self._dyn_host, non_blocking=True)
 
     def _upload_seeds(self):
         """The step's Philox seeds (masks, dropout, attention dropout) for the captured graphs."""
-        golden = 0x9E3779B97F4A7C15
         for i in range(3):
-            v = (self.seed + i + self.step_id * golden) & 0xFFFFFFFFFFFFFFFF
-            self._seeds_host[i] = v - (1 << 64) if v >= (1 << 63) else v
+            self._seeds_host[i] = self._step_seed(i)
         self._seeds_dev.copy_(self._seeds_host, non_blocking=True)
+
+    def _step_seed(self, i):
+        """Seed i of the current step (0-2: _sd's in graph mode, 3: the SCST sampler): a golden-ratio hash of the trainer seed and
+        step_id, as a signed 64-bit word."""
+        v = (self.seed + i + self.step_id * 0x9E3779B97F4A7C15) & 0xFFFFFFFFFFFFFFFF
+        return v - (1 << 64) if v >= (1 << 63) else v
 
     def _graph_body(self, ws, part, opt):
         # every body (eager warm-up, capture) re-applies the masks - except an SCST body, whose masks the rollout already used
@@ -1108,31 +1098,23 @@ class OrtTrainer:
         """One full SMP step.  Data parallel: either ``all_reduce`` (callable applied to the gradient buckets, NCCL sum, every
         rank then runs the whole optimizer) or ``exchange`` (distributed.ShardedExchange: reduce-scatter -> Adam on the owned
         shard -> all-gather per bucket, overlapped with the backward)."""
-        # programmatic dependent launch, measured on this chain (ms/step): the GEMM's EARLY trigger (bit 2: dependents may start
-        # once its loads are issued) costs time here, PDL with the implicit trigger at exit helps: mask 2 5.42, 3 5.30, 7 5.36
-        prev_pdl = K.set_pdl(self.pdl_mask)
-        try:
-            return self._train_step(att_feats, boxes, seqs, masks, att_masks, seq_per_img=seq_per_img, lr=lr, all_reduce=all_reduce,
-                                    global_tokens=global_tokens, exchange=exchange, **opt)
-        finally:
-            K.set_pdl(prev_pdl)
-
-    def _train_step(self, att_feats, boxes, seqs, masks, att_masks=None, *, seq_per_img, lr, all_reduce=None, global_tokens=None,
-                    exchange=None, **opt):
         B, N = att_feats.shape[:2]
         T = seqs.shape[1] - 1
         ws = self._get_ws(B, N, seq_per_img, T, att_masks is not None)
         self.step_id += 1
-        self.load_batch(ws, att_feats, boxes, seqs, masks, att_masks, global_tokens)
-        if exchange is not None and self.training:
-            if self.use_graph:
+        # programmatic dependent launch, measured on this chain (ms/step): the GEMM's EARLY trigger (bit 2: dependents may start
+        # once its loads are issued) costs time here, PDL with the implicit trigger at exit helps: mask 2 5.42, 3 5.30, 7 5.36
+        with K.pdl(self.pdl_mask):
+            self.load_batch(ws, att_feats, boxes, seqs, masks, att_masks, global_tokens)
+            if exchange is not None and self.training:
+                if self.use_graph:
+                    self._upload_step(lr=lr, **opt)
+                    self.opt_step -= 1  # (_sharded_step counts the step itself)
+                self._sharded_step(ws, exchange, dict(opt, lr=lr) if self.use_graph else opt, lr)
+                return ws.loss_sum * ws.inv_norm
+            if self.use_graph and self.training:
                 self._upload_step(lr=lr, **opt)
-                self.opt_step -= 1  # (_sharded_step counts the step itself)
-            self._sharded_step(ws, exchange, dict(opt, lr=lr) if self.use_graph else opt, lr)
-            return ws.loss_sum * ws.inv_norm
-        if self.use_graph and self.training:
-            self._upload_step(lr=lr, **opt)
-        return self._fwd_bwd_opt(ws, lr, all_reduce, opt)
+            return self._fwd_bwd_opt(ws, lr, all_reduce, opt)
 
     def _fwd_bwd_opt(self, ws, lr, all_reduce, opt):
         """Forward, backward (+ bucketed gradient exchange) and optimizer of a loaded workspace; graph mode expects
@@ -1197,16 +1179,9 @@ class OrtTrainer:
         lins = {("att_embed.0.weight", 1): eng.att_embed, ("model.generator.proj.weight", 1): eng.generator}
         norms = [(eng.enc_norm, "model.encoder.norm"), (eng.dec_norm, "model.decoder.norm")]
         for l in range(L):
-            p, e = f"model.encoder.layers.{l}", eng.enc[l]
-            lins.update({(f"{p}.self_attn.linears.0.weight", 3): e["qkv"], (f"{p}.self_attn.linears.3.weight", 1): e["o"],
-                         (f"{p}.feed_forward.w_1.weight", 1): e["ff1"], (f"{p}.feed_forward.w_2.weight", 1): e["ff2"]})
-            norms += [(e[f"n{j}"], f"{p}.sublayer.{j}.norm") for j in range(2)]
-            p, e = f"model.decoder.layers.{l}", eng.dec[l]
-            lins.update({(f"{p}.self_attn.linears.0.weight", 3): e["qkv"], (f"{p}.self_attn.linears.3.weight", 1): e["o"],
-                         (f"{p}.src_attn.linears.0.weight", 1): e["cq"], (f"{p}.src_attn.linears.1.weight", 2): e["ckv"],
-                         (f"{p}.src_attn.linears.3.weight", 1): e["co"], (f"{p}.feed_forward.w_1.weight", 1): e["ff1"],
-                         (f"{p}.feed_forward.w_2.weight", 1): e["ff2"]})
-            norms += [(e[f"n{j}"], f"{p}.sublayer.{j}.norm") for j in range(3)]
+            for stack, e, n_norms in (("encoder", eng.enc[l], 2), ("decoder", eng.dec[l], 3)):
+                lins.update({(w, n): e[slot] for w, n, slot in self._groups[stack, l]})
+                norms += [(e[f"n{j}"], f"model.{stack}.layers.{l}.sublayer.{j}.norm") for j in range(n_norms)]
         assert set(lins) == set(self._premask_keys())
         # bf16 rollouts read the trainer's own pre-masked operands; everything else is refreshed into engine-owned buffers
         share = self.adt == torch.bfloat16 and self.premask and not eval_masks
@@ -1230,10 +1205,9 @@ class OrtTrainer:
             nrm.a, nrm.b = self.p[name + ".a_2"], self.p[name + ".b_2"]
         eng.table = owned("model.tgt_embed.0.lut.weight", 1, torch.float32)
         eng.wg_w_all = torch.empty_like(eng.wg_w_all)
-        b0 = self._offs_w["model.encoder.layers.0.self_attn.WGs.0.bias"]
-        if any(self._offs_w[f"model.encoder.layers.{l}.self_attn.WGs.{j}.bias"] != b0 + l * h + j for l in range(L) for j in range(h)):
+        if self._wg_b_all is None:
             raise ValueError(f"the rollout engine needs the geometry biases packed in the trainer's layout (num_heads % 4 == 0, got {h})")
-        eng.wg_b_all = self.flat_w[b0: b0 + L * h]
+        eng.wg_b_all = self._wg_b_all
         for l in range(L):
             wname = f"model.encoder.layers.{l}.self_attn.WGs.0.weight"
             W = self._group(self.p, wname, h)
@@ -1284,8 +1258,7 @@ class OrtTrainer:
         self._scst_masks(eng)
         # 2. rollouts; the sampler seed follows the trainer's step seed (a run is reproducible)
         if int(opt.get("num_random_sample", 0)) > 0:
-            v = (self.seed + 3 + self.step_id * 0x9E3779B97F4A7C15) & 0xFFFFFFFFFFFFFFFF
-            opt["sample_seed"] = v - (1 << 64) if v >= (1 << 63) else v
+            opt["sample_seed"] = self._step_seed(3)
         greedy = {"beam_size": 1}
         bseq = None
         enc = eng.encode(att_feats, boxes, att_masks)
@@ -1316,13 +1289,12 @@ class OrtTrainer:
         if att_masks is not None:
             ws.att_mask.copy_(att_masks.float(), non_blocking=True)
         # 5. teacher-forcing forward on the step's operands, backward, clip + Adam
-        prev_pdl = K.set_pdl(self.pdl_mask)
         self._scst = True
         try:
-            loss = self._fwd_bwd_opt(ws, lr, all_reduce, optim)
+            with K.pdl(self.pdl_mask):
+                loss = self._fwd_bwd_opt(ws, lr, all_reduce, optim)
         finally:
             self._scst = False
-            K.set_pdl(prev_pdl)
         return loss, ws.mean_reward.clone(), seq.view(B, S, L).clone()
 
     # ---- magnitude / SNIP mask updates (PruningMixin.update_masks_*, pruning/prune.py:259-304) ------------------------------
@@ -1404,16 +1376,13 @@ class OrtTrainer:
         ws = self._get_ws(B, N, seq_per_img, T, att_masks is not None)
         self.step_id += 1
         self.load_batch(ws, att_feats, boxes, seqs, masks, att_masks, global_tokens)
-        prev_pdl = K.set_pdl(self.pdl_mask)
-        try:
+        with K.pdl(self.pdl_mask):
             if self.use_graph:
                 self._upload_seeds()
                 self._run_graphed(ws, "fwdbwd", {})
             else:
                 self.forward(ws)
                 self.loss_and_backward(ws)
-        finally:
-            K.set_pdl(prev_pdl)
         grads = self.flat_gw if self.fused_st else self.flat_gs   # dWm (straight-through form) or dS = dWm (.) W (raw masks)
         if all_reduce is not None:
             h = all_reduce(grads)
