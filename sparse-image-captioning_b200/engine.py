@@ -11,6 +11,8 @@ Reference call stack replaced (SURVEY.md section 3.2):
   CaptionModel.batch_beam_search            sparse_caption/models/caption_model.py:30-226
 """
 import math
+import os
+import types
 from typing import Dict, Optional
 
 import torch
@@ -150,6 +152,17 @@ class BeamState:
         self.done_seq.fill_(pad)
         self.done_lp.zero_()
         self.done_p.zero_()
+        return self
+
+
+def shared_history(states):
+    """Points the seq ping-pong buffers of a diverse beam search's G group BeamStates into one int32 [G, 2, rows, L] tensor,
+    from which each group's beam step reads the earlier groups' tokens (sc_beam_step_diverse); returns it."""
+    seq = states[0].seq[0]
+    hist = torch.zeros(len(states), 2, *seq.shape, dtype=torch.int32, device=seq.device)
+    for g, st in enumerate(states):
+        st.seq = [hist[g, 0], hist[g, 1]]
+    return hist
 
 
 class GreedyState:
@@ -210,28 +223,31 @@ class OrtEngine:
             nrm = (sd[norm + ".a_2"], sd[norm + ".b_2"]) if (norm and self.ln_fold) else None
             return _Lin(ws, bs, adt, backend, csr_threshold, norm=nrm)
 
+        def layer(p, share_att, backend, n_norms):
+            """The entries both stacks share: self-attention projections (qkv fused per share mode, then o), feed-forward and
+            the sublayer LayerNorms n0 .. n{n_norms-1}; the last one feeds ff1."""
+            qi, ki, vi, oi = _att_parts(share_att)
+            parts = sorted(set((qi, ki, vi)))
+            e = {"qkv": lin([f"{p}.self_attn.linears.{j}" for j in parts], backend, norm=f"{p}.sublayer.0.norm"),
+                 "offs": tuple(parts.index(j) * d for j in (qi, ki, vi)),
+                 "ld": len(parts) * d,
+                 "o": lin([f"{p}.self_attn.linears.{oi}"], backend),
+                 "ff1": lin([f"{p}.feed_forward.w_1"], backend, norm=f"{p}.sublayer.{n_norms - 1}.norm"),
+                 "ff2": lin([f"{p}.feed_forward.w_2"], backend)}
+            e.update({f"n{j}": _Norm(sd, f"{p}.sublayer.{j}.norm") for j in range(n_norms)})
+            return e
+
         self.att_embed = lin(["att_embed.0"])
         # ---- encoder (unique modules only; shared layers re-use the pack) ----
         self.enc_uids = cfg.uids("enc")
         self.enc = {}
-        qi, ki, vi, oi = _att_parts(cfg.share_att_encoder)
         for pos, u in enumerate(self.enc_uids):
             if u in self.enc:
                 continue
             p = f"model.encoder.layers.{pos}"
-            parts = sorted(set((qi, ki, vi)))
-            e = {
-                "qkv": lin([f"{p}.self_attn.linears.{j}" for j in parts], norm=f"{p}.sublayer.0.norm"),
-                "offs": tuple(parts.index(j) * d for j in (qi, ki, vi)),
-                "ld": len(parts) * d,
-                "o": lin([f"{p}.self_attn.linears.{oi}"]),
-                "wg_w": torch.cat([sd[f"{p}.self_attn.WGs.{j}.weight"].float() for j in range(cfg.num_heads)], 0).contiguous(),
-                "wg_b": torch.cat([sd[f"{p}.self_attn.WGs.{j}.bias"].float() for j in range(cfg.num_heads)], 0).contiguous(),
-                "ff1": lin([f"{p}.feed_forward.w_1"], norm=f"{p}.sublayer.1.norm"),
-                "ff2": lin([f"{p}.feed_forward.w_2"]),
-                "n0": _Norm(sd, f"{p}.sublayer.0.norm"),
-                "n1": _Norm(sd, f"{p}.sublayer.1.norm"),
-            }
+            e = layer(p, cfg.share_att_encoder, "dense", 2)
+            e["wg_w"] = torch.cat([sd[f"{p}.self_attn.WGs.{j}.weight"].float() for j in range(cfg.num_heads)], 0).contiguous()
+            e["wg_b"] = torch.cat([sd[f"{p}.self_attn.WGs.{j}.bias"].float() for j in range(cfg.num_heads)], 0).contiguous()
             self.enc[u] = e
         self.enc_norm = _Norm(sd, "model.encoder.norm")
         # all unique encoder layers' WG rows stacked: the geometry bias of every layer comes from ONE pass over the boxes
@@ -240,7 +256,6 @@ class OrtEngine:
         self.wg_b_all = torch.cat([self.enc[u]["wg_b"] for u in self.enc], 0).contiguous()
         # tensor-path attention (mma tiles) serves bf16, d_k = 64, N <= 128; fp32 mode keeps the exact fused kernel
         self.split_box_attn = (adt == torch.bfloat16 and d // cfg.num_heads == 64)
-        import os
         # CTA-per-(image, head) encoder attention (the training forward kernel without saved probabilities): 43 vs 50 us per
         # launch, no difference on the whole step -> the warp-per-(image, head) kernel stays the default
         self.enc_attn_cta = os.environ.get("SC_ENC_ATTN_CTA") == "1"
@@ -258,28 +273,19 @@ class OrtEngine:
             if u in self.dec:
                 continue
             p = f"model.decoder.layers.{pos}"
-            parts = sorted(set((qi, ki, vi)))
             kv_parts = sorted(set((ki, vi)))
             if cfg.share_att_decoder == "qk":
                 # cross-attention: key = linears.0(memory), value = linears.1(memory)
                 kv_parts = [0, 1]
-            e = {
-                "qkv": lin([f"{p}.self_attn.linears.{j}" for j in parts], be, norm=f"{p}.sublayer.0.norm"),
-                "offs": tuple(parts.index(j) * d for j in (qi, ki, vi)),
-                "ld": len(parts) * d,
-                "o": lin([f"{p}.self_attn.linears.{oi}"], be),
+            e = layer(p, cfg.share_att_decoder, be, 3)
+            e.update({
                 "cq": lin([f"{p}.src_attn.linears.{qi}"], be, norm=f"{p}.sublayer.1.norm"),
                 "ckv": lin([f"{p}.src_attn.linears.{j}" for j in kv_parts], norm="model.encoder.norm"),
                 "ckv_offs": tuple(kv_parts.index(j) * d for j in (ki, vi)),
                 "ckv_ld": len(kv_parts) * d,
                 "co": lin([f"{p}.src_attn.linears.{oi}"], be),
-                "ff1": lin([f"{p}.feed_forward.w_1"], be, norm=f"{p}.sublayer.2.norm"),
-                "ff2": lin([f"{p}.feed_forward.w_2"], be),
-                "n0": _Norm(sd, f"{p}.sublayer.0.norm"),
-                "n1": _Norm(sd, f"{p}.sublayer.1.norm"),
-                "n2": _Norm(sd, f"{p}.sublayer.2.norm"),
                 "apps": self.dec_uids.count(u),
-            }
+            })
             self.dec[u] = e
         self.dec_norm = _Norm(sd, "model.decoder.norm")
         self.table = sd["model.tgt_embed.0.lut.weight"].float().contiguous()
@@ -287,13 +293,11 @@ class OrtEngine:
         pe = sd.get("model.tgt_embed.1.pe")
         self.pe = (pe[0, : L + 2] if pe is not None else _positional_encoding(d, L + 2, self.dev)).float().contiguous()
         self.generator = lin(["model.generator.proj"], be, norm="model.decoder.norm")
-        import os
         # the folded decode path needs every decoder linear on the dense tensor path
         self.fold_dec = self.ln_fold and os.environ.get("SC_LN_FOLD_ENC_ONLY") != "1" and all(
             e[k].w is not None for e in self.dec.values() for k in ("qkv", "o", "cq", "co", "ff1", "ff2")) and self.generator.w is not None
         # decode-GEMM tile hints {"o": 3256, ...} (1000 * stages + block_n).  With >= 8 batches in flight the wide tiles
         # give a little more aggregate throughput than the latency-oriented 64-wide default (scripts/gemm_concurrency.py)
-        import os
         hints = dict(dec_tiles or {})
         for kv in filter(None, os.environ.get("SC_DEC_TILES", "").split(",")):
             name, val = kv.split("=")
@@ -352,9 +356,36 @@ class OrtEngine:
             ws.stats = torch.zeros(M, d // 32, 2, device=dev)
         ws.box_bias = (torch.zeros(len(self.enc), B, c.num_heads, N, N, device=dev)
                        if self.split_box_attn and N <= 128 else None)
+        ws.tile = {}
         ws.graph = None
+        ws.opt_key = None
         self._enc_ws[key] = ws
         return ws
+
+    # ---- the pre-norm sublayers of both stacks: ``ws.fold`` selects the LayerNorm folded into the GEMMs (bf16 copy of the
+    # residual stream + its row statistics, written by the previous residual GEMM) or a LayerNorm kernel into ``ws.xn`` ----
+    @staticmethod
+    def _norm_linear(ws, u, e, norm, name, out, relu=False):
+        """out = act(LayerNorm(x) W^T + b) of linear ``e[name]`` behind LayerNorm ``e[norm]``."""
+        tile_n = ws.tile.get((u, name))
+        if ws.fold:
+            e[name].ln(ws.xb, ws.stats, out, relu=relu, tile_n=tile_n)
+        else:
+            e[norm](ws.x, ws.xn)
+            e[name](ws.xn, out, relu=relu, tile_n=tile_n)
+
+    @staticmethod
+    def _residual_linear(ws, u, e, name, src):
+        """x += src W^T + b of linear ``e[name]``."""
+        tile_n = ws.tile.get((u, name))
+        if ws.fold:
+            e[name].produce(src, ws.x, ws.xb, ws.stats, residual=ws.x, tile_n=tile_n)
+        else:
+            e[name](src, ws.x, residual=ws.x, tile_n=tile_n)
+
+    def _feed_forward(self, ws, u, e, norm):
+        self._norm_linear(ws, u, e, norm, "ff1", ws.hid, relu=True)
+        self._residual_linear(ws, u, e, "ff2", ws.hid)
 
     def _encode_body(self, ws):
         c = self.cfg
@@ -362,8 +393,7 @@ class OrtEngine:
         dk = d // h
         if ws.att_a is not ws.att_in and not ws.bf16_in:
             K.cast_bf16(ws.att_in, out=ws.att_a)
-        fold = ws.fold
-        if fold:
+        if ws.fold:
             self.att_embed.produce(ws.att_a, ws.x, ws.xb, ws.stats, relu=True)
         else:
             self.att_embed(ws.att_a, ws.x, relu=True)
@@ -377,11 +407,7 @@ class OrtEngine:
             e = self.enc[u]
             ld = e["ld"]
             qkv = ws.qkv.view(-1)[: B * N * ld].view(B * N, ld)
-            if fold:
-                e["qkv"].ln(ws.xb, ws.stats, qkv)
-            else:
-                e["n0"](ws.x, ws.xn)
-                e["qkv"](ws.xn, qkv)
+            self._norm_linear(ws, u, e, "n0", "qkv", qkv)
             qo, ko, vo = e["offs"]
             if ws.box_bias is not None and self.enc_attn_cta:
                 # CTA = (image, head) with one warp per 16-query tile sharing the staged K / V (sc_attention_fwd's tensor path
@@ -394,16 +420,9 @@ class OrtEngine:
             else:
                 K.box_attention(qkv[:, qo:], qkv[:, ko:], qkv[:, vo:], ws.boxes, e["wg_w"], e["wg_b"], ws.att_mask, ws.att,
                                 B=B, N=N, h=h, dk=dk, ldq=ld, ldk=ld, ldv=ld, ldo=d, trig=trig)
-            if fold:
-                e["o"].produce(ws.att, ws.x, ws.xb, ws.stats, residual=ws.x)
-                e["ff1"].ln(ws.xb, ws.stats, ws.hid, relu=True)
-                e["ff2"].produce(ws.hid, ws.x, ws.xb, ws.stats, residual=ws.x)
-            else:
-                e["o"](ws.att, ws.x, residual=ws.x)
-                e["n1"](ws.x, ws.xn)
-                e["ff1"](ws.xn, ws.hid, relu=True)
-                e["ff2"](ws.hid, ws.x, residual=ws.x)
-        if fold:
+            self._residual_linear(ws, u, e, "o", ws.att)
+            self._feed_forward(ws, u, e, "n1")
+        if ws.fold:
             for u, e in self.dec.items():
                 e["ckv"].ln(ws.xb, ws.stats, ws.memkv[u])
         else:
@@ -419,107 +438,119 @@ class OrtEngine:
         Measured SLOWER with 5-8 slots in flight (7.10 vs 6.85 ms/step end to end; a variant through staging buffers: 7.08): the
         other slots already hide the copy - off by default (bench.py --prefetch)."""
         B, N, F = att_feats.shape
-        bf16_in = att_feats.dtype == torch.bfloat16 and self.adt == torch.bfloat16
-        if (self.zero_copy_ingest and self.adt == torch.bfloat16 and att_feats.device.type == "cpu" and att_feats.dtype == torch.float32
+        masked = att_masks is not None
+        host = att_feats.device.type == "cpu"
+        if (self.zero_copy_ingest and self.adt == torch.bfloat16 and host and att_feats.dtype == torch.float32
                 and att_feats.is_pinned() and att_feats.is_contiguous() and (B * N * F) % 4 == 0):
             # fused ingest: one kernel reads the pinned fp32 features over PCIe and writes the bf16 operand (no fp32 staging, no cast)
-            ws = self._get_enc_ws(B, N, att_masks is not None, slot, True)
+            ws = self._get_enc_ws(B, N, masked, slot, True)
             # one engine-wide ingest stream: the ingest kernels of all slots queue FIFO on the PCIe link like DMA copies would
             # (launched on the slots' own streams they all share the link and every encoder starts late)
             if self._ingest_stream is None:
                 self._ingest_stream = torch.cuda.Stream(self.dev)
-            ist, cur = self._ingest_stream, torch.cuda.current_stream(self.dev)
-            ist.wait_stream(cur)  # the previous batch of this slot is done with the operand buffer
-            with torch.cuda.stream(ist):
-                K.ingest_f32_bf16(att_feats, ws.att_a.view(-1), ctas=self.zero_copy_ingest)
-                ready = torch.cuda.Event()
-                ready.record(ist)
-            cur.wait_event(ready)
-            ws.boxes.copy_(boxes, non_blocking=True)
-            if att_masks is not None:
-                ws.att_mask.copy_(att_masks.float(), non_blocking=True)
-            self.run_encoder(ws)
-            return ws
-        ws = self._get_enc_ws(B, N, att_masks is not None, slot, bf16_in)
-        dst = ws.att_a if ws.bf16_in else ws.att_in
-        src = att_feats.reshape(B * N, F)
-        if prefetch and src.device.type == "cpu" and boxes.device.type == "cpu" and att_masks is None:
-            # the input buffers are only read by the encoder graph: the next batch's H2D may start as soon as the previous
-            # ENCODER on this slot is done (event), on the slot's copy stream, underneath the previous batch's decode
-            if getattr(ws, "copy_stream", None) is None:
-                ws.copy_stream, ws.enc_done = torch.cuda.Stream(self.dev), None
-            cs, cur = ws.copy_stream, torch.cuda.current_stream(self.dev)
-            if ws.enc_done is not None:
-                cs.wait_event(ws.enc_done)
-            with torch.cuda.stream(cs):
-                dst.copy_(src, non_blocking=True)
-                ws.boxes.copy_(boxes, non_blocking=True)
-                ready = torch.cuda.Event()
-                ready.record(cs)
-            cur.wait_event(ready)
-            self.run_encoder(ws)
-            ws.enc_done = torch.cuda.Event()
-            ws.enc_done.record(cur)
-            return ws
+            # (after the current stream: the previous batch of this slot is done with the operand buffer)
+            self._fork_join(self._ingest_stream, lambda: K.ingest_f32_bf16(att_feats, ws.att_a.view(-1), ctas=self.zero_copy_ingest),
+                            after_stream=torch.cuda.current_stream(self.dev))
+            prefetch = False
         else:
-            dst.copy_(src, non_blocking=True)
+            bf16_in = att_feats.dtype == torch.bfloat16 and self.adt == torch.bfloat16
+            ws = self._get_enc_ws(B, N, masked, slot, bf16_in)
+            dst = ws.att_a if ws.bf16_in else ws.att_in
+            src = att_feats.reshape(B * N, F)
+            prefetch = prefetch and host and boxes.device.type == "cpu" and not masked
+            if prefetch:
+                # the input buffers are only read by the encoder graph: the next batch's H2D may start as soon as the previous
+                # ENCODER on this slot is done (event), on the slot's copy stream, underneath the previous batch's decode
+                if getattr(ws, "copy_stream", None) is None:
+                    ws.copy_stream, ws.enc_done = torch.cuda.Stream(self.dev), None
+                self._fork_join(ws.copy_stream, lambda: (dst.copy_(src, non_blocking=True), ws.boxes.copy_(boxes, non_blocking=True)),
+                                after_event=ws.enc_done)
+            else:
+                dst.copy_(src, non_blocking=True)
+        if not prefetch:
             ws.boxes.copy_(boxes, non_blocking=True)
-            if att_masks is not None:
-                ws.att_mask.copy_(att_masks.float(), non_blocking=True)
+        if masked:
+            ws.att_mask.copy_(att_masks.float(), non_blocking=True)
         self.run_encoder(ws)
+        if prefetch:
+            ws.enc_done = torch.cuda.Event()
+            ws.enc_done.record(torch.cuda.current_stream(self.dev))
         return ws
 
+    def _fork_join(self, side, work, after_stream=None, after_event=None):
+        """Runs ``work()`` on stream ``side`` once it has waited for ``after_stream`` / ``after_event`` (when given); the
+        current stream waits for it."""
+        cur = torch.cuda.current_stream(self.dev)
+        if after_stream is not None:
+            side.wait_stream(after_stream)
+        if after_event is not None:
+            side.wait_event(after_event)
+        with torch.cuda.stream(side):
+            work()
+            ready = torch.cuda.Event()
+            ready.record(side)
+        cur.wait_event(ready)
+
     def run_encoder(self, ws):
-        if not self.use_graphs:
-            self._encode_body(ws)
+        self._run(ws, lambda: self._encode_body(ws), None)
+
+    def _run(self, ws, body, key, eager=False):
+        """Runs a body eagerly, or as the workspace's CUDA graph (captured again when ``key`` changes)."""
+        if eager or not self.use_graphs:
+            body()
             return
-        if ws.graph is None:
-            self._warm_and_capture(ws, lambda: self._encode_body(ws))
+        if ws.graph is None or ws.opt_key != key:
+            # warm-up on a side stream (lazy module loading, cudaFuncSetAttribute) before capture
+            s = torch.cuda.Stream(self.dev)
+            s.wait_stream(torch.cuda.current_stream(self.dev))
+            with torch.cuda.stream(s):
+                body()
+            torch.cuda.current_stream(self.dev).wait_stream(s)
+            torch.cuda.synchronize(self.dev)
+            g = torch.cuda.CUDAGraph()
+            before = lib.launch_count
+            with torch.cuda.graph(g):
+                body()
+            ws.graph, ws.opt_key = g, key
+            ws.launches = lib.launch_count - before
         ws.graph.replay()
 
-    def _warm_and_capture(self, ws, body):
-        # warm-up on a side stream (lazy module loading, cudaFuncSetAttribute) before capture
-        s = torch.cuda.Stream(self.dev)
-        s.wait_stream(torch.cuda.current_stream(self.dev))
-        with torch.cuda.stream(s):
-            body()
-        torch.cuda.current_stream(self.dev).wait_stream(s)
-        torch.cuda.synchronize(self.dev)
-        g = torch.cuda.CUDAGraph()
-        before = lib.launch_count
-        with torch.cuda.graph(g):
-            body()
-        ws.graph = g
-        ws.launches = lib.launch_count - before
-
     # ------------------------------------------------------------------------------------------------
-    def _get_dec_ws(self, B, beam, N, greedy, slot=0, tag=None):
-        key = (B, beam, N, greedy, slot, tag)
-        if key in self._dec_ws:
-            return self._dec_ws[key]
+    def _new_dec_ws(self, key, kind, R, topk=False):
+        """A decode workspace (type name ``kind``) registered under ``key``: the step's activation buffers at R rows, the fused
+        generator's top-k records when ``topk``, and the folded LayerNorms' bf16 stream copy and row statistics."""
         c, dev, adt = self.cfg, self.dev, self.adt
-        d, ff, L, V = c.d_model, c.dim_feedforward, c.max_seq_length, c.vocab_size
-        R = B * beam
-        ws = type("DecWs", (), {})()
-        ws.B, ws.beam, ws.N, ws.R, ws.greedy = B, beam, N, R, greedy
+        d = c.d_model
+        ws = type(kind, (), {})()
+        ws.R, ws.fold, ws.tile = R, self.fold_dec, {}
         ws.x = torch.zeros(R, d, device=dev)
         ws.xn = torch.zeros(R, d, device=dev, dtype=adt)
         ws.qkv = torch.zeros(R, 3 * d, device=dev, dtype=adt)
         ws.att = torch.zeros(R, d, device=dev, dtype=adt)
         ws.qc = torch.zeros(R, d, device=dev, dtype=adt)
-        ws.hid = torch.zeros(R, ff, device=dev, dtype=adt)
-        ws.logits = torch.zeros(R, V, device=dev)
-        ws.topk_part = torch.zeros(R, K.linear_topk_parts(V), 12, device=dev) if (not greedy and self._topk_ok(beam)) else None
-        if self.fold_dec:
+        ws.hid = torch.zeros(R, c.dim_feedforward, device=dev, dtype=adt)
+        ws.logits = torch.zeros(R, c.vocab_size, device=dev)
+        ws.topk_part = torch.zeros(R, K.linear_topk_parts(c.vocab_size), 12, device=dev) if topk else None
+        if ws.fold:
             ws.xb = torch.zeros(R, d, device=dev, dtype=adt)
             ws.stats = torch.zeros(R, d // 32, 2, device=dev)
-        ws.cache = {u: (torch.zeros(L * e["apps"], R, d, device=dev, dtype=adt),
-                        torch.zeros(L * e["apps"], R, d, device=dev, dtype=adt)) for u, e in self.dec.items()}
+        self._dec_ws[key] = ws
+        return ws
+
+    def _get_dec_ws(self, B, beam, N, greedy, slot=0, tag=None):
+        key = (B, beam, N, greedy, slot, tag)
+        if key in self._dec_ws:
+            return self._dec_ws[key]
+        c, dev = self.cfg, self.dev
+        L, R = c.max_seq_length, B * beam
+        ws = self._new_dec_ws(key, "DecWs", R, topk=not greedy and self._topk_ok(beam))
+        ws.B, ws.beam, ws.N, ws.greedy = B, beam, N, greedy
+        ws.cache = {u: (torch.zeros(L * e["apps"], R, c.d_model, device=dev, dtype=self.adt),
+                        torch.zeros(L * e["apps"], R, c.d_model, device=dev, dtype=self.adt)) for u, e in self.dec.items()}
         ws.state = GreedyState(R, L, dev) if greedy else BeamState(B, beam, L, dev)
         ws.tile = self._dec_hints(R)
         ws.graph = None
         ws.opt_key = None
-        self._dec_ws[key] = ws
         return ws
 
     def _dec_hints(self, R):
@@ -543,26 +574,21 @@ class OrtEngine:
         return (self.fuse_topk and self.adt == torch.bfloat16 and g.w is not None and g.w.dtype == torch.bfloat16 and beam <= 5
                 and g.K % 8 == 0)
 
-    def _decode_step(self, ws, enc, t, anc, fused_topk=False, candidates=None):
+    def _decode_step(self, ws, enc, t, anc, topk=None):
+        """One decode step of every row; ``topk``: candidates per row of the fused generator + top-k records (None: the
+        generator writes the logits)."""
         c = self.cfg
         R, d, h, N = ws.R, c.d_model, c.num_heads, ws.N
-        fold = self.fold_dec
-        if fold:
+        if ws.fold:
             K.embed_pe_stats(ws.state.tokens, self.table, self.pe, ws.x, ws.xb, ws.stats, T=1, pos0=t)
         else:
             K.embed_pe(ws.state.tokens, self.table, self.pe, T=1, pos0=t, out=ws.x)
         used = {u: 0 for u in self.dec}
-        tiles = getattr(ws, "tile", None) or {}
         for u in self.dec_uids:
             e = self.dec[u]
-            tl = lambda name, u=u: tiles.get((u, name))   # per-workspace grid sizing of the decode GEMMs (dec_ctas)
             ld = e["ld"]
             qkv = ws.qkv.view(-1)[: R * ld].view(R, ld)
-            if fold:
-                e["qkv"].ln(ws.xb, ws.stats, qkv, tile_n=tl("qkv"))
-            else:
-                e["n0"](ws.x, ws.xn)
-                e["qkv"](ws.xn, qkv, tile_n=tl("qkv"))
+            self._norm_linear(ws, u, e, "n0", "qkv", qkv)
             qo, ko, vo = e["offs"]
             apps = e["apps"]
             slot = t * apps + used[u]
@@ -571,70 +597,46 @@ class OrtEngine:
             K.self_attn_step(qkv[:, qo:], qkv[:, ko:], qkv[:, vo:], ck, cv, anc, ws.att, R=R, D=d, h=h,
                              n_prev=0 if self.no_history else slot, write_slot=-1 if self.no_history else slot,
                              ldq=ld, ldk=ld, ldv=ld, ldo=d, anc_ld=anc.shape[1], slot_div=apps)
-            if fold:
-                e["o"].produce(ws.att, ws.x, ws.xb, ws.stats, residual=ws.x, tile_n=tl("o"))
-                e["cq"].ln(ws.xb, ws.stats, ws.qc, tile_n=tl("cq"))
-            else:
-                e["o"](ws.att, ws.x, residual=ws.x, tile_n=tl("o"))
-                e["n1"](ws.x, ws.xn)
-                e["cq"](ws.xn, ws.qc, tile_n=tl("cq"))
+            self._residual_linear(ws, u, e, "o", ws.att)
+            self._norm_linear(ws, u, e, "n1", "cq", ws.qc)
             mkv = enc.memkv[u]
             ko2, vo2 = e["ckv_offs"]
             K.cross_attn_step(ws.qc, mkv[:, ko2:], mkv[:, vo2:], enc.att_mask, ws.att, B=ws.B, beam=ws.beam, N=N, D=d, h=h,
                               ldq=d, ldm=e["ckv_ld"], ldo=d)
-            if fold:
-                e["co"].produce(ws.att, ws.x, ws.xb, ws.stats, residual=ws.x, tile_n=tl("co"))
-                e["ff1"].ln(ws.xb, ws.stats, ws.hid, relu=True, tile_n=tl("ff1"))
-                e["ff2"].produce(ws.hid, ws.x, ws.xb, ws.stats, residual=ws.x, tile_n=tl("ff2"))
-            else:
-                e["co"](ws.att, ws.x, residual=ws.x, tile_n=tl("co"))
-                e["n2"](ws.x, ws.xn)
-                e["ff1"](ws.xn, ws.hid, relu=True, tile_n=tl("ff1"))
-                e["ff2"](ws.hid, ws.x, residual=ws.x, tile_n=tl("ff2"))
+            self._residual_linear(ws, u, e, "co", ws.att)
+            self._feed_forward(ws, u, e, "n2")
         # (the final norm stays a kernel also when the layers' norms are folded: the fused generator + top-k epilogue has no
         # folded-LayerNorm variant, and one LayerNorm per step is 1/19 of them)
         self.dec_norm(ws.x, ws.xn)
-        if fused_topk:
-            K.linear_topk(ws.xn, self.generator.w, self.generator.bias, ws.topk_part, candidates=candidates or ws.beam)
+        if topk:
+            K.linear_topk(ws.xn, self.generator.w, self.generator.bias, ws.topk_part, candidates=topk)
         else:
             self.generator(ws.xn, ws.logits)
 
-    def _beam_body(self, ws, enc, opt):
-        c = self.cfg
-        L, V = c.max_seq_length, c.vocab_size
-        st = ws.state
-        st.reset(c.bos_token_id, c.pad_token_id)
-        kind, alpha = _parse_penalty(opt.get("length_penalty", ""))
-        pen_col = int(opt.get("penalized_col", -1))  # suppress_UNK (:169-170)
-        bad_t = self._bad_endings(ws, opt)
-        fused = (ws.topk_part is not None and float(opt.get("temperature", 1.0)) == 1.0 and not opt.get("decoding_constraint", 0)
-                 and bad_t is None and pen_col < 0)
-        for t in range(L):
-            self._decode_step(ws, enc, t, st.anc[t & 1], fused_topk=fused)
-            sup = _suppress_bad(st, bad_t, t)
-            if fused:
-                K.beam_step_partials(ws.topk_part, st, t, B=ws.B, beam=ws.beam, V=V, L=L, eos=c.eos_token_id, pad=c.pad_token_id,
-                                     penalty_kind=kind, penalty_alpha=alpha)
-            else:
-                K.beam_step(ws.logits, st, t, B=ws.B, beam=ws.beam, V=V, L=L, eos=c.eos_token_id, pad=c.pad_token_id,
-                            temperature=opt.get("temperature", 1.0), constraint=opt.get("decoding_constraint", 0),
-                            penalty_kind=kind, penalty_alpha=alpha, suppress_tok=sup, penalized_col=pen_col)
-
-    def _bad_endings(self, ws, opt):
+    def _bad_endings(self, ws, so):
         """remove_bad_endings (caption_model.py:161-168): the ids as a device tensor held by the workspace, made outside any
         graph capture, so that a captured decode reads live memory on every replay (None when the option is off)."""
-        bad = opt.get("bad_endings_ix")
-        if not bad:
+        if so.bad is None:
             return None
-        ids = sorted(int(i) for i in bad)
-        if getattr(ws, "bad_ids", None) != ids:
-            ws.bad_ids, ws.bad_t = ids, torch.tensor(ids, dtype=torch.int32, device=self.dev)
+        if getattr(ws, "bad_ids", None) != so.bad:
+            ws.bad_ids, ws.bad_t = so.bad, torch.tensor(so.bad, dtype=torch.int32, device=self.dev)
         return ws.bad_t
 
+    def _beam_step(self, scores, st, t, B, beam, so, bad_t, fused=False, diverse=None):
+        """sc_beam_step on one group's log-probs ``scores`` [B*beam, V], or (``fused``) sc_beam_step_partials on its top-k
+        records; ``diverse``: (hist, group, diversity_lambda) of a diverse beam search."""
+        c = self.cfg
+        kw = dict(B=B, beam=beam, V=c.vocab_size, L=c.max_seq_length, eos=c.eos_token_id, pad=c.pad_token_id,
+                  penalty_kind=so.kind, penalty_alpha=so.alpha, diverse=diverse)
+        if fused:
+            K.beam_step_partials(scores, st, t, **kw)
+        else:
+            K.beam_step(scores, st, t, temperature=so.temperature, constraint=so.constraint,
+                        suppress_tok=_suppress_bad(st, bad_t, t), penalized_col=so.pen_col, **kw)
+
     def _get_diverse_ws(self, B, N, G, bdash, slot):
-        """Diverse beam search: one decode workspace + BeamState per group (B*bdash rows each); the groups' seq ping-pong
-        buffers live in one int32 [G, 2, B*bdash, L] tensor, from which each group's beam step reads the earlier groups'
-        tokens (sc_beam_step_diverse)."""
+        """Diverse beam search: one decode workspace + BeamState per group (B*bdash rows each) over one seq history
+        (``shared_history``)."""
         key = (B, G * bdash, N, "diverse", G, slot)
         dv = self._dec_ws.get(key)
         if dv is not None:
@@ -642,12 +644,8 @@ class OrtEngine:
         L = self.cfg.max_seq_length
         dv = type("DiverseWs", (), {})()
         dv.B, dv.G, dv.bdash = B, G, bdash
-        dv.hist = torch.zeros(G, 2, B * bdash, L, dtype=torch.int32, device=self.dev)
-        dv.groups = []
-        for g in range(G):
-            ws = self._get_dec_ws(B, bdash, N, False, slot, tag=("diverse", G, g))
-            ws.state.seq = [dv.hist[g, 0], dv.hist[g, 1]]
-            dv.groups.append(ws)
+        dv.groups = [self._get_dec_ws(B, bdash, N, False, slot, tag=("diverse", G, g)) for g in range(G)]
+        dv.hist = shared_history([ws.state for ws in dv.groups])
         dv.seq = torch.zeros(B, G * bdash, L, dtype=torch.int32, device=self.dev)
         dv.lp = torch.zeros(B, G * bdash, L, device=self.dev)
         dv.graph = None
@@ -655,43 +653,33 @@ class OrtEngine:
         self._dec_ws[key] = dv
         return dv
 
-    def _diverse_body(self, dv, enc, opt):
-        """batch_beam_search with group_size G > 1 (caption_model.py:126-226): global step t = 0 .. L+G-2, group g decodes
-        and steps at its local step t - g while that lies in [0, L-1], groups in ascending order; finished beams stay per
-        group and are concatenated group by group (:221-225)."""
+    def _search_body(self, groups, enc, opt, dv=None):
+        """batch_beam_search (caption_model.py:30-226) over the workspaces of G = len(groups) groups of beams.  G > 1 (diverse
+        beam search, ``dv``, :126-226): global step t = 0 .. L+G-2, group g decodes and steps at its local step t - g while that
+        lies in [0, L-1], groups in ascending order; finished beams stay per group and are concatenated group by group into
+        ``dv.seq`` / ``dv.lp`` (:221-225)."""
         c = self.cfg
-        L, V = c.max_seq_length, c.vocab_size
-        G, bdash = dv.G, dv.bdash
-        _, _, lam = diverse_groups(opt)
-        kind, alpha = _parse_penalty(opt.get("length_penalty", ""))
-        pen_col = int(opt.get("penalized_col", -1))
-        bad_t = self._bad_endings(dv, opt)
-        temperature = float(opt.get("temperature", 1.0))
-        # fused generator + row pass: a group needs its bdash + g*bdash <= beam_size best raw candidates per row
-        fused = (all(ws.topk_part is not None for ws in dv.groups) and self._topk_ok(G * bdash) and temperature == 1.0
-                 and not opt.get("decoding_constraint", 0) and bad_t is None and pen_col < 0)
-        for ws in dv.groups:
+        L, G = c.max_seq_length, len(groups)
+        so = search_options(opt)
+        bad_t = self._bad_endings(dv or groups[0], so)
+        # fused generator + row pass: group g needs its bdash + g*bdash <= beam_size best raw candidates per row
+        cands = G * groups[0].beam
+        fused = so.fusable and all(ws.topk_part is not None for ws in groups) and self._topk_ok(cands)
+        for ws in groups:
             ws.state.reset(c.bos_token_id, c.pad_token_id)
         for t in range(L + G - 1):
-            for g in range(G):
+            for g, ws in enumerate(groups):
                 tau = t - g
                 if not 0 <= tau <= L - 1:
                     continue
-                ws = dv.groups[g]
                 st = ws.state
-                self._decode_step(ws, enc, tau, st.anc[tau & 1], fused_topk=fused, candidates=G * bdash)
-                div = (dv.hist, g, lam)
-                if fused:
-                    K.beam_step_partials(ws.topk_part, st, tau, B=dv.B, beam=bdash, V=V, L=L, eos=c.eos_token_id,
-                                         pad=c.pad_token_id, penalty_kind=kind, penalty_alpha=alpha, diverse=div)
-                else:
-                    K.beam_step(ws.logits, st, tau, B=dv.B, beam=bdash, V=V, L=L, eos=c.eos_token_id, pad=c.pad_token_id,
-                                temperature=temperature, constraint=opt.get("decoding_constraint", 0), penalty_kind=kind,
-                                penalty_alpha=alpha, suppress_tok=_suppress_bad(st, bad_t, tau), penalized_col=pen_col,
-                                diverse=div)
-        for g, ws in enumerate(dv.groups):
-            dv.seq[:, g * bdash:(g + 1) * bdash].copy_(ws.state.done_seq)
-            dv.lp[:, g * bdash:(g + 1) * bdash].copy_(ws.state.done_lp)
+                self._decode_step(ws, enc, tau, st.anc[tau & 1], topk=cands if fused else None)
+                self._beam_step(ws.topk_part if fused else ws.logits, st, tau, ws.B, ws.beam, so, bad_t, fused,
+                                None if dv is None else (dv.hist, g, so.lam))
+        if dv is not None:
+            for g, ws in enumerate(groups):
+                dv.seq[:, g * dv.bdash:(g + 1) * dv.bdash].copy_(ws.state.done_seq)
+                dv.lp[:, g * dv.bdash:(g + 1) * dv.bdash].copy_(ws.state.done_lp)
 
     def _greedy_body(self, ws, enc, opt):
         c = self.cfg
@@ -734,41 +722,23 @@ class OrtEngine:
             if uni is not None:
                 ws.uniforms = uni.to(self.dev, torch.float32).contiguous()
                 assert tuple(ws.uniforms.shape) == (self.cfg.max_seq_length, enc.B * n_rand)
-            body = lambda: self._sample_body(ws, enc, opt)
             opt_key = (id(enc), "sample", uni is not None, tuple(sorted((k, str(v)) for k, v in opt.items())))
-            if not self.use_graphs or uni is not None:
-                body()
-            else:
-                if ws.graph is None or ws.opt_key != opt_key:
-                    self._warm_and_capture(ws, body)
-                    ws.opt_key = opt_key
-                ws.graph.replay()
+            self._run(ws, lambda: self._sample_body(ws, enc, opt), opt_key, eager=uni is not None)
             return ws.state.seq.view(enc.B, n_rand, -1), ws.state.lp.view(enc.B, n_rand, -1)
-        greedy = beam == 1
         assert beam <= self.cfg.vocab_size
         opt_key = (id(enc), tuple(sorted((k, str(v)) for k, v in opt.items())))
-        if not greedy and int(opt.get("group_size", 1)) > 1:
+        if beam == 1:
+            ws = self._get_dec_ws(enc.B, beam, enc.N, True, enc.slot)
+            self._run(ws, lambda: self._greedy_body(ws, enc, opt), opt_key)
+            return ws.state.seq.view(enc.B, 1, -1), ws.state.lp.view(enc.B, 1, -1)
+        if int(opt.get("group_size", 1)) > 1:
             G, bdash, _ = diverse_groups(opt)
-            ws = self._get_diverse_ws(enc.B, enc.N, G, bdash, enc.slot)
-            self._run(ws, lambda: self._diverse_body(ws, enc, opt), opt_key)
-            return ws.seq, ws.lp
-        ws = self._get_dec_ws(enc.B, beam, enc.N, greedy, enc.slot)
-        body = (lambda: self._greedy_body(ws, enc, opt)) if greedy else (lambda: self._beam_body(ws, enc, opt))
-        self._run(ws, body, opt_key)
-        st = ws.state
-        if greedy:
-            return st.seq.view(enc.B, 1, -1), st.lp.view(enc.B, 1, -1)
-        return st.done_seq, st.done_lp
-
-    def _run(self, ws, body, opt_key):
-        """Runs a decode body eagerly, or as the workspace's CUDA graph (captured again when the options change)."""
-        if not self.use_graphs:
-            body()
-            return
-        if ws.graph is None or ws.opt_key != opt_key:
-            self._warm_and_capture(ws, body)
-            ws.opt_key = opt_key
-        ws.graph.replay()
+            dv = self._get_diverse_ws(enc.B, enc.N, G, bdash, enc.slot)
+            self._run(dv, lambda: self._search_body(dv.groups, enc, opt, dv), opt_key)
+            return dv.seq, dv.lp
+        ws = self._get_dec_ws(enc.B, beam, enc.N, False, enc.slot)
+        self._run(ws, lambda: self._search_body([ws], enc, opt), opt_key)
+        return ws.state.done_seq, ws.state.done_lp
 
     def teacher_force(self, enc, tokens, beam=1, out=None):
         """Incremental (KV-cached) decoding along GIVEN token paths: row r = image r // beam feeds BOS, tokens[r, 0], ...,
@@ -794,31 +764,6 @@ class OrtEngine:
         return out
 
     # ---- step-wise entry points (get_logprobs_state / batch_beam_search of the reference) over an explicit state ----
-    def _step_ws(self, R, N):
-        key = ("step", R, N)
-        ws = self._dec_ws.get(key)
-        if ws is None:
-            c, dev, adt = self.cfg, self.dev, self.adt
-            d, ff, L, V = c.d_model, c.dim_feedforward, c.max_seq_length, c.vocab_size
-            ws = type("StepWs", (), {})()
-            ws.B, ws.beam, ws.N, ws.R = R, 1, N, R   # every row carries its own memory K/V
-            ws.x = torch.zeros(R, d, device=dev)
-            ws.xn = torch.zeros(R, d, device=dev, dtype=adt)
-            ws.qkv = torch.zeros(R, 3 * d, device=dev, dtype=adt)
-            ws.att = torch.zeros(R, d, device=dev, dtype=adt)
-            ws.qc = torch.zeros(R, d, device=dev, dtype=adt)
-            ws.hid = torch.zeros(R, ff, device=dev, dtype=adt)
-            ws.logits = torch.zeros(R, V, device=dev)
-            ws.topk_part = None
-            if self.fold_dec:
-                ws.xb = torch.zeros(R, d, device=dev, dtype=adt)
-                ws.stats = torch.zeros(R, d // 32, 2, device=dev)
-            ws.state = type("Tok", (), {})()
-            ws.state.tokens = torch.zeros(R, dtype=torch.int32, device=dev)
-            ws.anc = torch.arange(R, dtype=torch.int32, device=dev).unsqueeze(1).expand(R, L * max(e["apps"] for e in self.dec.values())).contiguous()
-            self._dec_ws[key] = ws
-        return ws
-
     def logprobs_step(self, it, memory, att_mask, caches, t):
         """One ``get_logprobs_state`` step (relation_transformer.py:374-387).  ``it`` [R] tokens; ``memory`` [R, N, d] encoder
         output (final norm applied); ``att_mask`` [R, 1, N] / [R, N] / None; ``caches`` None at t = 0 or, per unique decoder
@@ -829,7 +774,13 @@ class OrtEngine:
         N = memory.shape[1]
         d, L = c.d_model, c.max_seq_length
         assert 0 <= t <= L, f"step {t} beyond max_seq_length {L}"
-        ws = self._step_ws(R, N)
+        ws = self._dec_ws.get(("step", R, N))
+        if ws is None:
+            ws = self._new_dec_ws(("step", R, N), "StepWs", R)
+            ws.B, ws.beam, ws.N = R, 1, N   # every row carries its own memory K/V
+            ws.state = type("Tok", (), {})()
+            ws.state.tokens = torch.zeros(R, dtype=torch.int32, device=self.dev)
+            ws.anc = torch.arange(R, dtype=torch.int32, device=self.dev).unsqueeze(1).expand(R, L * max(e["apps"] for e in self.dec.values())).contiguous()
         uids = list(self.dec)
         if caches is None:
             mem = memory.reshape(-1, d)
@@ -872,22 +823,13 @@ class OrtEngine:
         steps (sc_beam_step_diverse).  Returns done_beams [B][G*bdash] dicts {seq, logps, unaug_p, p}, group-major."""
         c = self.cfg
         beam = int(opt.get("beam_size", 10))
-        G, bdash, lam = diverse_groups(opt) if int(opt.get("group_size", 1)) > 1 else (1, beam, 0.0)
+        G, bdash, _ = diverse_groups(opt) if int(opt.get("group_size", 1)) > 1 else (1, beam, 0.0)
         L, V = c.max_seq_length, c.vocab_size
         B = init_logprobs.shape[0]
-        hist = torch.zeros(G, 2, B * bdash, L, dtype=torch.int32, device=self.dev) if G > 1 else None
-        sts = []
-        for g in range(G):
-            st = BeamState(B, bdash, L, self.dev)
-            if hist is not None:
-                st.seq = [hist[g, 0], hist[g, 1]]
-            st.reset(c.bos_token_id, c.pad_token_id)
-            sts.append(st)
-        kind, alpha = _parse_penalty(opt.get("length_penalty", ""))
-        bad = opt.get("bad_endings_ix")
-        bad_t = torch.tensor(sorted(bad), dtype=torch.int32, device=self.dev) if bad else None
-        pen_col = int(opt.get("penalized_col", -1))
-        temperature = float(opt.get("temperature", 1.0))
+        sts = [BeamState(B, bdash, L, self.dev).reset(c.bos_token_id, c.pad_token_id) for _ in range(G)]
+        hist = shared_history(sts) if G > 1 else None
+        so = search_options(opt)
+        bad_t = None if so.bad is None else torch.tensor(so.bad, dtype=torch.int32, device=self.dev)
         args = list(args)
         group_args = [[None if a is None else a.reshape(a.shape[0] // G, G, *a.shape[1:])[:, g] for a in args] for g in range(G)]
         logits, state = [], []
@@ -902,10 +844,7 @@ class OrtEngine:
                 if not 0 <= tau <= L - 1:
                     continue
                 st = sts[g]
-                K.beam_step(logits[g], st, tau, B=B, beam=bdash, V=V, L=L, eos=c.eos_token_id, pad=c.pad_token_id,
-                            temperature=temperature, constraint=opt.get("decoding_constraint", 0), penalty_kind=kind,
-                            penalty_alpha=alpha, suppress_tok=_suppress_bad(st, bad_t, tau), penalized_col=pen_col,
-                            diverse=None if hist is None else (hist, g, lam))
+                self._beam_step(logits[g], st, tau, B, bdash, so, bad_t, diverse=None if hist is None else (hist, g, so.lam))
                 parents = st.anc[(tau + 1) & 1][:, tau].long()      # row each new beam descends from (b*bdash + parent)
                 if tau == 0:
                     parents = parents // bdash                       # the first state holds one row per image
@@ -1011,6 +950,20 @@ def _suppress_bad(st, bad_t, t):
     if bad_t is None or t == 0:
         return None
     return torch.where(torch.isin(st.tokens, bad_t), 0, -1).to(torch.int32)
+
+
+def search_options(opt):
+    """The beam-step options of a search (caption_model.py:114-172): length penalty kind and alpha, the column suppressed by
+    suppress_UNK (``pen_col``), temperature, decoding constraint, the sorted bad-ending ids (None: off), the diversity lambda,
+    and whether the fused generator + top-k row pass can serve them (temperature 1, no constraint, no bad endings, no
+    suppressed column)."""
+    kind, alpha = _parse_penalty(opt.get("length_penalty", ""))
+    bad = opt.get("bad_endings_ix")
+    so = types.SimpleNamespace(kind=kind, alpha=alpha, pen_col=int(opt.get("penalized_col", -1)),
+                               temperature=float(opt.get("temperature", 1.0)), constraint=opt.get("decoding_constraint", 0),
+                               bad=sorted(int(i) for i in bad) if bad else None, lam=float(opt.get("diversity_lambda", 0.5)))
+    so.fusable = so.temperature == 1.0 and not so.constraint and so.bad is None and so.pen_col < 0
+    return so
 
 
 def _parse_penalty(s):
