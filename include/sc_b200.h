@@ -345,6 +345,33 @@ int sc_ciderd_score(const int* hyp, int H, int L, const int* hyp_img, int eos, i
                     const double* df_log, long n_df, double ref_len, double sigma, const long* img_ref_off, const long* ref_ng_off,
                     const unsigned long long* ref_keys, const double* ref_vec, const double* ref_norm, const int* ref_length,
                     double* out, sc_stream_t stream);
+/* coco-caption validation metrics on word ids (coco_caption/eval.py:15-86 as called by eval_on_split, utils/training.py:257-327),
+ * METEOR / SPICE / the PTB tokenizer excepted.  Hypotheses hyp int32 [H, L <= 64] (words = ids before the first <eos>, pads
+ * dropped), each scored against the references of image hyp_img[h] in [0, n_images) and written to that image's slot;
+ * hypotheses with an image index outside that range are skipped (sc_bleu_stats counts them in *bad_index).  References of image
+ * b are [img_ref_off[b], img_ref_off[b+1]).
+ * sc_cider_score: CIDEr of pycocoevalcap cider/cider_scorer.py (compute_cider: counts2vec + sim without the clip and the length
+ * penalty of CIDEr-D); the tables are those of sc_ciderd_score, out float64 [n_images]. */
+int sc_cider_score(const int* hyp, int H, int L, const int* hyp_img, int n_images, int eos, int pad, const unsigned long long* df_keys,
+                   const double* df_log, long n_df, double ref_len, const long* img_ref_off, const long* ref_ng_off,
+                   const unsigned long long* ref_keys, const double* ref_vec, const double* ref_norm, double* out, sc_stream_t stream);
+/* BLEU sufficient statistics of bleu/bleu_scorer.py (cook_test, n = 4, option "closest"): stats int64 [n_images, 10] =
+ * correct_1..4 (sum over n-grams of min(hypothesis count, largest count in one reference)), guess_1..4 = max(0, |h| - k + 1),
+ * testlen = |h|, reflen = the reference length l minimising (|l - |h||, l).  Per image b: n-gram keys ascending in
+ * keys[img_key_off[b] .. img_key_off[b+1]) with their max_count; reference r has length ref_tok_off[r+1] - ref_tok_off[r].
+ * hyp_count[b] += 1 per hypothesis of image b. */
+int sc_bleu_stats(const int* hyp, int H, int L, const int* hyp_img, int n_images, int eos, int pad, const long* img_key_off,
+                  const unsigned long long* keys, const int* max_count, const long* img_ref_off, const long* ref_tok_off,
+                  long long* stats, int* hyp_count, int* bad_index, sc_stream_t stream);
+/* ROUGE-L of rouge/rouge.py (beta = 1.2) from the exact LCS with every reference (bit-parallel over the hypothesis positions):
+ * out float64 [n_images].  Reference r's tokens are ref_tok[ref_tok_off[r] .. ref_tok_off[r+1]), any length. */
+int sc_rouge_l(const int* hyp, int H, int L, const int* hyp_img, int n_images, int eos, int pad, const long* img_ref_off,
+               const long* ref_tok_off, const int* ref_tok, double* out, sc_stream_t stream);
+/* One launch, fixed order (bitwise reproducible): out float64 [9 + 6 n_images] = corpus Bleu_1..4 (bleu_scorer.py compute_score
+ * on the summed statistics), mean ROUGE_L, mean CIDEr, #images without a hypothesis, #images with more than one, *bad_index;
+ * then per image {Bleu_1..4 (compute_score's bleu_list), ROUGE_L, CIDEr} (coco-caption's imgToEval). */
+int sc_caption_metrics_reduce(const long long* bleu_stats, const double* rouge, const double* cider, const int* hyp_count,
+                              const int* bad_index, int n_images, double* out, sc_stream_t stream);
 /* SCST rollout -> teacher-forcing inputs of the training step (utils/training.py:239-255 with RewardCriterion, utils/losses.py:10-29),
  * one launch.  seq int32 [R = B*S, L]: the rollout (S samples per image, rows image-major).  score float64 [R]: the samples'
  * CIDEr-D; base_score float64 [B] (the greedy baseline, one per image) or NULL (each sample's baseline is the mean of its image's

@@ -1,14 +1,17 @@
-// CIDEr-D reward of self-critical sequence training on the device (SURVEY.md section 8f.4).
-// Reference: sparse_caption/scst/cider/pyciderevalcap/ciderD/ciderD_scorer.py:133-212 (compute_cider: counts2vec + sim) as
-// called by CaptionScorer (sparse_caption/scst/scorers.py:47-114) on decoded sample / baseline captions.
+// Caption scores on the device, on word ids: the CIDEr-D reward of self-critical sequence training (SURVEY.md section 8f.4) and
+// the coco-caption validation metrics BLEU-1..4, ROUGE-L and CIDEr.
+// CIDEr-D reference: sparse_caption/scst/cider/pyciderevalcap/ciderD/ciderD_scorer.py:133-212 (compute_cider: counts2vec + sim)
+// as called by CaptionScorer (sparse_caption/scst/scorers.py:47-114) on decoded sample / baseline captions.  Validation
+// metrics reference: pycocoevalcap bleu/bleu_scorer.py (cook_test, compute_score), rouge/rouge.py and cider/cider_scorer.py as
+// called by coco_caption/eval.py:15-86 from eval_on_split (utils/training.py:257-327).
 //
-// The reference detokenises every rollout to a string on the host, splits it into words and scores it in Python dictionaries
-// (B x (samples + 1) captions per step).  Here the rollouts stay on the device as word ids: an n-gram (n <= 4) of ids below
-// 65536 is packed exactly into one 64-bit key; the document-frequency table (coco-train-words.p in the reference) and the
-// tf-idf vectors of the reference captions - both static over training - are uploaded once as sorted key arrays.
+// The reference detokenises every caption to a string on the host, splits it into words and scores it in Python dictionaries.
+// Here the captions stay on the device as word ids: an n-gram (n <= 4) of ids below 65536 is packed exactly into one 64-bit
+// key; the document-frequency table (coco-train-words.p in the reference, or the split's own references) and the tf-idf
+// vectors / BLEU max counts / token arrays of the reference captions - static over a split - are uploaded once.
 // One CTA scores one hypothesis against the references of its image.  All arithmetic is double precision in the reference's
 // own summation order (reductions are sequential in first-occurrence n-gram order, like the dict iteration of the reference),
-// so scores agree with the Python scorer to the last bits.
+// so scores agree with the Python scorers to the last bits.
 #include "sc_common.cuh"
 
 namespace {
@@ -28,7 +31,7 @@ struct CiderArgs {
   const unsigned long long* ref_keys; const double* ref_vec;   // per reference: keys ascending, tf-idf weights
   const double* ref_norm;       // [R, 4]
   const int* ref_length;        // [R]   (the reference scorer's `length`: its bigram count)
-  double* out;                  // [H]
+  double* out;                  // [H] (CIDEr-D) or [n_img] indexed by hyp_img (CIDEr)
 };
 
 __device__ __forceinline__ long lower_bound(const unsigned long long* a, long n, unsigned long long key) {
@@ -40,17 +43,45 @@ __device__ __forceinline__ long lower_bound(const unsigned long long* a, long n,
   return lo;
 }
 
-__global__ void __launch_bounds__(kThreads) ciderd_kernel(const CiderArgs a) {
+struct BleuArgs {
+  const long* img_key_off;                 // [n_img + 1] -> the image's entries of keys / max_count
+  const unsigned long long* keys;          // per image: n-gram keys ascending
+  const int* max_count;                    // the n-gram's largest count in any one reference of the image
+  const long* img_ref_off;                 // [n_img + 1] -> references of an image
+  const long* ref_tok_off;                 // [R + 1] -> tokens of a reference (its length is all BLEU needs)
+  long long* stats;                        // [n_img, 10]: correct_1..4, guess_1..4, testlen, reflen
+  int* hyp_count;                          // [n_img] hypotheses scored per image
+  int* bad_index;                          // hypotheses whose image index is outside [0, n_img)
+};
+
+enum Metric { kCiderD, kCider, kBleu };
+
+// One CTA per hypothesis.  All three metrics share the n-gram entries of the hypothesis: its words (ids before the first <eos>,
+// pads dropped: what tokenizer.decode + str.split leave), one 64-bit key per entry in the reference's dict insertion order
+// (k = 1..4, position ascending) and each n-gram's count at its first occurrence.  They are one template rather than a shared
+// helper function because an out-of-line helper changes the register allocation of the CIDEr-D instantiation.
+//   kCiderD: CIDEr-D (ciderD_scorer.py: clipped hypothesis tf-idf, Gaussian length penalty), out[h].
+//   kCider:  coco-caption CIDEr (cider_scorer.py: plain cosine, no penalty), out[hyp_img[h]].
+//   kBleu:   the sufficient statistics of bleu_scorer.py cook_test (n = 4, "closest" reference length), b.stats[hyp_img[h]].
+// kCider / kBleu skip hypotheses whose image is outside [0, n_img); kBleu counts them and the hypotheses of every image.
+template <Metric M>
+__global__ void __launch_bounds__(kThreads) ngram_score_kernel(const CiderArgs a, const BleuArgs b, int n_img) {
   __shared__ int s_words[kMaxWords];
   __shared__ unsigned long long s_key[kMaxNgrams];
-  __shared__ int s_tf[kMaxNgrams];      // 0 = not the first occurrence of its n-gram
+  __shared__ int s_tf[kMaxNgrams];      // 0 = not the first occurrence of its n-gram (kBleu: the clipped count)
   __shared__ int s_ord[kMaxNgrams];     // n-gram order - 1
   __shared__ double s_vec[kMaxNgrams], s_ref[kMaxNgrams];
   __shared__ double s_norm[4], s_score[4];
   __shared__ int s_nw, s_T;
   const int hI = blockIdx.x, tid = threadIdx.x;
+  if constexpr (M != kCiderD) {
+    const int img = a.hyp_img[hI];
+    if (img < 0 || img >= n_img) {
+      if (M == kBleu && tid == 0) atomicAdd(b.bad_index, 1);
+      return;
+    }
+  }
   if (tid == 0) {
-    // words of the caption: ids before the first <eos>, pads dropped (what tokenizer.decode + str.split leave)
     int n = 0;
     for (int i = 0; i < a.L && n < kMaxWords; ++i) {
       const int t = a.hyp[(size_t)hI * a.L + i];
@@ -65,7 +96,6 @@ __global__ void __launch_bounds__(kThreads) ciderd_kernel(const CiderArgs a) {
   }
   __syncthreads();
   const int nw = s_nw, T = s_T;
-  // entries in the reference's dict insertion order: k = 1..4, position ascending
   for (int e = tid; e < T; e += kThreads) {
     int k = 1, base = 0;
     while (e >= base + (nw - k + 1)) { base += nw - k + 1; ++k; }
@@ -80,16 +110,46 @@ __global__ void __launch_bounds__(kThreads) ciderd_kernel(const CiderArgs a) {
     const unsigned long long key = s_key[e];
     int tf = 0; bool first = true;
     for (int j = 0; j < T; ++j) if (s_key[j] == key) { ++tf; if (j < e) first = false; }
-    s_tf[e] = first ? tf : 0;
-    double v = 0.0;
-    if (first) {
-      const long p = lower_bound(a.df_keys, a.n_df, key);
-      const double dl = (p < a.n_df && a.df_keys[p] == key) ? a.df_log[p] : 0.0;
-      v = (double)tf * (a.ref_len - dl);
+    if constexpr (M == kBleu) {   // min(count_h, max over the references of count_r)
+      int c = 0;
+      if (first) {
+        const int img = a.hyp_img[hI];
+        const long k0 = b.img_key_off[img], kn = b.img_key_off[img + 1] - k0;
+        const long p = lower_bound(b.keys + k0, kn, key);
+        if (p < kn && b.keys[k0 + p] == key) c = min(tf, b.max_count[k0 + p]);
+      }
+      s_tf[e] = c;
+    } else {
+      s_tf[e] = first ? tf : 0;
+      double v = 0.0;
+      if (first) {
+        const long p = lower_bound(a.df_keys, a.n_df, key);
+        const double dl = (p < a.n_df && a.df_keys[p] == key) ? a.df_log[p] : 0.0;
+        v = (double)tf * (a.ref_len - dl);
+      }
+      s_vec[e] = v;
     }
-    s_vec[e] = v;
   }
   __syncthreads();
+  if constexpr (M == kBleu) {
+    if (tid == 0) {
+      const int img = a.hyp_img[hI];
+      long long st[10] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+      for (int e = 0; e < T; ++e) st[s_ord[e]] += s_tf[e];
+      for (int k = 0; k < 4; ++k) st[4 + k] = max(0, nw - k);
+      st[8] = nw;
+      // the reference length l minimising (|l - testlen|, l): a tie goes to the shorter reference
+      long best = -1, best_d = 0;
+      for (long r = b.img_ref_off[img]; r < b.img_ref_off[img + 1]; ++r) {
+        const long l = b.ref_tok_off[r + 1] - b.ref_tok_off[r], d = l > nw ? l - nw : nw - l;
+        if (best < 0 || d < best_d || (d == best_d && l < best)) { best = l; best_d = d; }
+      }
+      st[9] = best;
+      for (int i = 0; i < 10; ++i) b.stats[(size_t)img * 10 + i] = st[i];
+      atomicAdd(b.hyp_count + img, 1);
+    }
+    return;
+  }
   if (tid == 0) {
     for (int e = 0; e < T; ++e) if (s_tf[e]) s_norm[s_ord[e]] += s_vec[e] * s_vec[e];
     for (int k = 0; k < 4; ++k) s_norm[k] = sqrt(s_norm[k]);
@@ -111,13 +171,16 @@ __global__ void __launch_bounds__(kThreads) ciderd_kernel(const CiderArgs a) {
     __syncthreads();
     if (tid == 0) {
       double val[4] = {0.0, 0.0, 0.0, 0.0};
-      for (int e = 0; e < T; ++e) if (s_tf[e]) val[s_ord[e]] += fmin(s_vec[e], s_ref[e]) * s_ref[e];
-      const double delta = (double)(len_h - a.ref_length[r]);
-      const double pen = pow(2.718281828459045, -(delta * delta) / (2.0 * a.sigma * a.sigma));
+      for (int e = 0; e < T; ++e) if (s_tf[e]) val[s_ord[e]] += (M == kCiderD ? fmin(s_vec[e], s_ref[e]) : s_vec[e]) * s_ref[e];
+      double pen = 1.0;
+      if (M == kCiderD) {
+        const double delta = (double)(len_h - a.ref_length[r]);
+        pen = pow(2.718281828459045, -(delta * delta) / (2.0 * a.sigma * a.sigma));
+      }
       for (int k = 0; k < 4; ++k) {
         const double nr = a.ref_norm[r * 4 + k];
         if (s_norm[k] != 0.0 && nr != 0.0) val[k] /= s_norm[k] * nr;
-        val[k] *= pen;
+        if (M == kCiderD) val[k] *= pen;
         s_score[k] += val[k];
       }
     }
@@ -128,7 +191,7 @@ __global__ void __launch_bounds__(kThreads) ciderd_kernel(const CiderArgs a) {
     s /= 4.0;
     s /= (double)(r1 - r0);
     s *= 10.0;
-    a.out[hI] = s;
+    a.out[M == kCiderD ? hI : img] = s;
   }
 }
 
@@ -221,8 +284,38 @@ int sc_ciderd_score(const int* hyp, int H, int L, const int* hyp_img, int eos, i
   a.hyp = hyp; a.L = L; a.H = H; a.hyp_img = hyp_img; a.eos = eos; a.pad = pad; a.df_keys = df_keys; a.df_log = df_log; a.n_df = n_df;
   a.ref_len = ref_len; a.sigma = sigma; a.img_ref_off = img_ref_off; a.ref_ng_off = ref_ng_off; a.ref_keys = ref_keys;
   a.ref_vec = ref_vec; a.ref_norm = ref_norm; a.ref_length = ref_length; a.out = out;
-  ciderd_kernel<<<H, kThreads, 0, stream>>>(a);
+  ngram_score_kernel<kCiderD><<<H, kThreads, 0, stream>>>(a, BleuArgs{}, 0);
   SC_LAUNCH_CHECK("sc_ciderd_score");
+  return SC_OK;
+}
+
+int sc_cider_score(const int* hyp, int H, int L, const int* hyp_img, int n_images, int eos, int pad, const unsigned long long* df_keys,
+                   const double* df_log, long n_df, double ref_len, const long* img_ref_off, const long* ref_ng_off,
+                   const unsigned long long* ref_keys, const double* ref_vec, const double* ref_norm, double* out, cudaStream_t stream) {
+  SC_CHECK(H > 0 && L > 0 && L <= kMaxWords && n_images > 0, SC_ERR_SHAPE, "sc_cider_score: H=%d L=%d (L <= %d) n_images=%d", H, L,
+           kMaxWords, n_images);
+  SC_CHECK(hyp && hyp_img && img_ref_off && ref_ng_off && ref_norm && out, SC_ERR_SHAPE, "sc_cider_score: null argument");
+  CiderArgs a = {};
+  a.hyp = hyp; a.L = L; a.H = H; a.hyp_img = hyp_img; a.eos = eos; a.pad = pad; a.df_keys = df_keys; a.df_log = df_log; a.n_df = n_df;
+  a.ref_len = ref_len; a.img_ref_off = img_ref_off; a.ref_ng_off = ref_ng_off; a.ref_keys = ref_keys; a.ref_vec = ref_vec;
+  a.ref_norm = ref_norm; a.out = out;
+  ngram_score_kernel<kCider><<<H, kThreads, 0, stream>>>(a, BleuArgs{}, n_images);
+  SC_LAUNCH_CHECK("sc_cider_score");
+  return SC_OK;
+}
+
+int sc_bleu_stats(const int* hyp, int H, int L, const int* hyp_img, int n_images, int eos, int pad, const long* img_key_off,
+                  const unsigned long long* keys, const int* max_count, const long* img_ref_off, const long* ref_tok_off,
+                  long long* stats, int* hyp_count, int* bad_index, cudaStream_t stream) {
+  SC_CHECK(H > 0 && L > 0 && L <= kMaxWords && n_images > 0, SC_ERR_SHAPE, "sc_bleu_stats: H=%d L=%d (L <= %d) n_images=%d", H, L,
+           kMaxWords, n_images);
+  SC_CHECK(hyp && hyp_img && img_key_off && keys && max_count && img_ref_off && ref_tok_off && stats && hyp_count && bad_index,
+           SC_ERR_SHAPE, "sc_bleu_stats: null argument");
+  CiderArgs a = {};
+  a.hyp = hyp; a.L = L; a.H = H; a.hyp_img = hyp_img; a.eos = eos; a.pad = pad;
+  const BleuArgs b = {img_key_off, keys, max_count, img_ref_off, ref_tok_off, stats, hyp_count, bad_index};
+  ngram_score_kernel<kBleu><<<H, kThreads, 0, stream>>>(a, b, n_images);
+  SC_LAUNCH_CHECK("sc_bleu_stats");
   return SC_OK;
 }
 

@@ -1,6 +1,7 @@
 """The caller after the path (SURVEY.md section 8f.1): ``TrainingModule.eval_on_split`` (utils/training.py:257-327) up to the
 caption JSON - batches -> ``mode="sample"`` -> token ids on the host -> detokenisation -> COCO-caption result file
-(data/karpathy.py:193-221).  The COCO metrics themselves (Java METEOR / SPICE / PTBTokenizer) are out of scope.
+(data/karpathy.py:193-221), and optionally coco-caption's BLEU-1..4 / ROUGE-L / CIDEr on the device (``metrics.CaptionMetrics``,
+fed the best captions as word ids before they leave the GPU).  METEOR / SPICE / PTBTokenizer (Java) are out of scope.
 
 Detokenisation: word-level tokenizers call ``tokenizer.decode`` per caption (SentencePiece, C++); radix tokenizers (ACORT) first
 map the radix digits to word ids for the WHOLE batch in one vectorised pass on the device (detok.radix_to_word_ids), so the
@@ -61,8 +62,13 @@ def coco_caption_json_dump(image_ids_and_captions: Iterable[Tuple[int, str]], ou
 
 def eval_on_split(engine_or_model, batches: Iterable[dict], opt: dict, *, decode_words: Callable[[List[int]], str],
                   radix: Optional[Tuple[int, int]] = None, vocab_len: Optional[int] = None, json_fpath: Optional[str] = None,
-                  eos_id: int = 3):
-    """``batches`` yield {"att_feats", "boxes", "att_masks" (optional), "image_ids"}.  Returns (predictions, images / s, json path)."""
+                  eos_id: int = 3, metrics=None):
+    """``batches`` yield {"att_feats", "boxes", "att_masks" (optional), "image_ids"}.  Returns (predictions, images / s, json path).
+
+    ``metrics``: a ``CaptionMetrics`` whose ``set_refs`` holds the split's references; every batch then also yields "image_idx",
+    the images' indices into those references (not the COCO image ids of the JSON), and its best captions are added to it as word
+    ids on the device (radix models: ``radix_to_word_ids``, ids beyond ``vocab_len`` -> <unk> as in ``detokenize``).  The
+    caller reads ``metrics.compute()``."""
     t0 = time.perf_counter()
     ids, preds = [], []
     for data in batches:
@@ -70,7 +76,15 @@ def eval_on_split(engine_or_model, batches: Iterable[dict], opt: dict, *, decode
             seq, _ = engine_or_model.sample(data["att_feats"], data["boxes"], data.get("att_masks"), opt)
         else:
             seq, _ = engine_or_model(att_feats=data["att_feats"], boxes=data["boxes"], att_masks=data.get("att_masks"), opt=opt, mode="sample")
-        preds += detokenize(best_captions(seq), decode_words=decode_words, radix=radix, vocab_len=vocab_len, eos_id=eos_id)
+        best = best_captions(seq)
+        if metrics is not None:
+            words = best
+            if radix is not None:
+                words, _ = radix_to_word_ids(best, *radix)
+                if vocab_len is not None:
+                    words = torch.where(words < vocab_len, words, torch.ones_like(words))
+            metrics.add(words, data["image_idx"])
+        preds += detokenize(best, decode_words=decode_words, radix=radix, vocab_len=vocab_len, eos_id=eos_id)
         ids += list(data["image_ids"])
     speed = len(ids) / max(time.perf_counter() - t0, 1e-9)
     path = coco_caption_json_dump(zip(ids, preds), json_fpath) if json_fpath else None

@@ -78,6 +78,10 @@ SIGNATURES = {
     "sc_log_clamp": [_p, _p, _p, _sz, _f, _p],
     "sc_logsoftmax_bwd": [_p, _p, _p, _i, _i, _p],
     "sc_ciderd_score": [_p, _i, _i, _p, _i, _i, _p, _p, _l, C.c_double, C.c_double, _p, _p, _p, _p, _p, _p, _p, _p],
+    "sc_cider_score": [_p, _i, _i, _p, _i, _i, _i, _p, _p, _l, C.c_double, _p, _p, _p, _p, _p, _p, _p],
+    "sc_bleu_stats": [_p, _i, _i, _p, _i, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p],
+    "sc_rouge_l": [_p, _i, _i, _p, _i, _i, _i, _p, _p, _p, _p, _p],
+    "sc_caption_metrics_reduce": [_p, _p, _p, _p, _p, _i, _p, _p],
     "sc_scst_targets": [_p, _i, _i, _i, _p, _p, _f, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p, _p],
     "sc_prune_chunk": [],
     "sc_prune_stats": [_p, _i, _l, _p, _i, _p, _p, _p, _p],
