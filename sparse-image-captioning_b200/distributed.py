@@ -96,14 +96,20 @@ class ShardedExchange:
             update(lo, hi)
         if b > mid:
             update(mid, b)
-        if n > 0:
-            own = param[lo:hi].clone()
+        self.gather(param, a, b)
+
+    def gather(self, buf, a, b):
+        """All-gather of ``buf[a, mid)`` in place from the owners of its shards (``shard(a, b)``); the tail ``[mid, b)`` is the same
+        on every rank already.  The updated parameters of a bucket, or the optimizer state a rank keeps for its shards only."""
+        lo, hi, mid = self.shard(a, b)
+        if hi > lo:
+            own = buf[lo:hi].clone()
             if self.nccl:
-                dist.all_gather_into_tensor(param[a:mid], own, group=self.group)
+                dist.all_gather_into_tensor(buf[a:mid], own, group=self.group)
             else:
                 parts = [torch.empty_like(own) for _ in range(self.world)]
                 dist.all_gather(parts, own, group=self.group)
-                param[a:mid].copy_(torch.cat(parts))
+                buf[a:mid].copy_(torch.cat(parts))
 
     def finish(self):
         """Order the caller's stream after every bucket's chain."""

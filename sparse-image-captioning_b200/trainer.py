@@ -68,6 +68,72 @@ def _part(n, cut, part):
     return {"all": (0, n), "hi": (cut, n), "lo": (0, cut)}[part]
 
 
+# ---- optimizer state in the layout of torch.optim.Adam.state_dict() (train_n_prune_transformer.py:67-82: group 0 the weights, group 1
+# the mask logits with their own lr / eps, "pruning_mask": True) ------------------------------------------------------------------------
+_ADAM = dict(mask_lr=100.0, betas=(0.9, 0.98), eps=1e-9, mask_eps=1e-2, weight_decay=0.0)
+
+
+def _adam_hyper(lr, opt):
+    """The Adam hyper-parameters of a step (its optimizer keywords, defaults filled in): the param_groups of the exported state."""
+    return dict(_ADAM, **{k: opt[k] for k in _ADAM if k in opt}, lr=float(lr))
+
+
+def _export_adam(groups, hyper, step, trainer):
+    """torch.optim.Adam.state_dict() of ``groups`` = [[(name, (exp_avg, exp_avg_sq) or None)]]: parameter indices run over the groups
+    in order, a parameter without moments gets no state entry, every entry's step is ``float(step)``.  ``trainer``: the extra
+    top-level key (Adam.load_state_dict ignores it)."""
+    state, param_groups, i = {}, [], 0
+    for gi, entries in enumerate(groups):
+        ids = []
+        for _, mv in entries:
+            if mv is not None:
+                state[i] = {"step": torch.tensor(float(step), dtype=torch.float32), "exp_avg": mv[0], "exp_avg_sq": mv[1]}
+            ids.append(i)
+            i += 1
+        g = dict(lr=hyper["lr"], betas=tuple(hyper["betas"]), eps=hyper["eps"], weight_decay=hyper["weight_decay"], amsgrad=False,
+                 maximize=False)
+        if gi == 1:
+            g.update(lr=hyper["mask_lr"], eps=hyper["mask_eps"], weight_decay=0.0, pruning_mask=True)
+        param_groups.append(dict(g, params=ids))
+    return {"state": state, "param_groups": param_groups, "trainer": trainer}
+
+
+def _import_adam(sd, groups, mask_type):
+    """Checks an Adam state dict against ``groups`` = [[(name, shape, has_state)]] (``has_state``: the trainer updates it, so its
+    entry must be there).  Returns ({name: (exp_avg, exp_avg_sq)}, step, hyper-parameters, the "trainer" key or None); ValueError,
+    naming the parameter, for a different parameter count or shape, a missing entry, unequal steps or another mask type."""
+    pgs, state, extra = sd["param_groups"], sd["state"], sd.get("trainer")
+    if extra is not None and extra.get("mask_type") != mask_type:
+        raise ValueError(f"the state was saved by a trainer with mask_type {extra.get('mask_type')!r}, this one has {mask_type!r}")
+    if len(pgs) != len(groups):
+        raise ValueError(f"the state has {len(pgs)} parameter groups, the trainer {len(groups)}")
+    moments, step, first = {}, None, None
+    for gi, (pg, entries) in enumerate(zip(pgs, groups)):
+        if len(pg["params"]) != len(entries):
+            raise ValueError(f"parameter group {gi} has {len(pg['params'])} parameters in the state, {len(entries)} in the trainer "
+                             f"(first of them: {entries[0][0] if entries else None})")
+        for idx, (name, shape, has_state) in zip(pg["params"], entries):
+            st = state.get(idx)
+            if st is None:
+                if has_state:
+                    raise ValueError(f"{name}: no optimizer state entry (parameter {idx})")
+                continue
+            for key in ("exp_avg", "exp_avg_sq"):
+                if tuple(st[key].shape) != tuple(shape):
+                    raise ValueError(f"{name}: {key} has shape {tuple(st[key].shape)}, the parameter {tuple(shape)}")
+            s = float(st["step"])
+            if step is None:
+                step, first = s, name
+            elif s != step:
+                raise ValueError(f"{name}: step {s} differs from the step {step} of {first}")
+            moments[name] = (st["exp_avg"], st["exp_avg_sq"])
+    g0 = pgs[0]
+    hyper = dict(lr=g0["lr"], betas=tuple(g0["betas"]), eps=g0["eps"], weight_decay=g0["weight_decay"])
+    if len(pgs) > 1:
+        hyper.update(mask_lr=pgs[1]["lr"], mask_eps=pgs[1]["eps"])
+    return moments, int(step or 0), hyper, extra
+
+
 def scst_samples(opt, baseline, bleu_weight=0.0):
     """Captions per image S of an SCST rollout ``opt`` (beam_size b, G * (b // G) for diverse beam search, or num_random_sample);
     ValueError for the options the device step does not support."""
@@ -203,6 +269,11 @@ class OrtTrainer:
             else:
                 self.s[k].fill_(mask_init_value)
         self._offs_s = offs_s
+        # parameter order of optimizer_state_dict: the key order of `state_dict` (named_parameters() order for the drop-in module); a
+        # mask logit sits where its "_pruning_mask" key is, or where its weight is when the logit was initialised here
+        pos = {k: i for i, k in enumerate(sd)}
+        self._adam_order = sorted(order, key=pos.__getitem__)
+        self._adam_masks = sorted(self.masked, key=lambda k: pos.get(k + "_pruning_mask", pos[k]))
         self._cut, self._cut_w, self._cut_s = order.index(_DEC0), offs[_DEC0], offs_s.get(_DEC0)
         # padding elements of flat_s must never count as "kept" in the sparsity statistics
         pad = torch.ones_like(self.flat_s, dtype=torch.bool)
@@ -226,6 +297,7 @@ class OrtTrainer:
         self.m_w, self.v_w = torch.zeros_like(self.flat_w), torch.zeros_like(self.flat_w)
         self.m_s, self.v_s = torch.zeros_like(self.flat_s), torch.zeros_like(self.flat_s)
         self.opt_step = 0
+        self._hyper = _adam_hyper(0.0, {})   # hyper-parameters of the last optimizer step (optimizer_state_dict's param_groups)
         self.sp_out = torch.zeros(3, device=self.dev)
         self.sp_count = torch.zeros(1, dtype=torch.int64, device=self.dev)
         self._ws = {}
@@ -878,6 +950,7 @@ class OrtTrainer:
         "lo" = att_embed + encoder (after the last phase; also re-pins the padding logits)."""
         if not _dyn and part != "lo":
             self.opt_step += 1
+            self._hyper = _adam_hyper(lr, dict(mask_lr=mask_lr, betas=betas, eps=eps, mask_eps=mask_eps, weight_decay=weight_decay))
         dyn = self._dyn_dev if _dyn else None
         if self.fused_st and not self._materialized:
             return self._optimizer_step_st(lr=lr, mask_lr=mask_lr, clip=clip, betas=betas, eps=eps, mask_eps=mask_eps,
@@ -1102,6 +1175,7 @@ class OrtTrainer:
         T = seqs.shape[1] - 1
         ws = self._get_ws(B, N, seq_per_img, T, att_masks is not None)
         self.step_id += 1
+        self._hyper = _adam_hyper(lr, opt)   # (graph mode and the sharded update do not go through optimizer_step's bookkeeping)
         # programmatic dependent launch, measured on this chain (ms/step): the GEMM's EARLY trigger (bit 2: dependents may start
         # once its loads are issued) costs time here, PDL with the implicit trigger at exit helps: mask 2 5.42, 3 5.30, 7 5.36
         with K.pdl(self.pdl_mask):
@@ -1252,6 +1326,7 @@ class OrtTrainer:
             ws.mask_sum = torch.zeros(1, device=self.dev)
             ws.mean_reward = torch.zeros(1, device=self.dev)
         self.step_id += 1
+        self._hyper = _adam_hyper(lr, optim)
         if self.use_graph:
             self._upload_step(lr=lr, **optim)
         eng = self.rollout_engine()
@@ -1419,6 +1494,84 @@ class OrtTrainer:
         sd.update({k + "_pruning_mask": v.clone() for k, v in self.s.items()})
         return sd
 
+    # ---- resumable optimizer state ------------------------------------------------------------------------------------------------
+    def _adam_groups(self):
+        """[[(parameter name, flat moment buffers' layout, tensor name)]] of the two Adam groups: every trained weight, then (with
+        masks) every mask logit, in the order of the state dict the trainer was built from."""
+        groups = [[(k, self._offs_w, k) for k in self._adam_order]]
+        if self.masked:
+            groups.append([(k + "_pruning_mask", self._offs_s, k) for k in self._adam_masks])
+        return groups
+
+    @torch.no_grad()
+    def optimizer_state_dict(self, exchange=None):
+        """The optimizer state as ``torch.optim.Adam.state_dict()`` of the reference's two parameter groups: group 0 every trained
+        weight, group 1 (with masks) every ``*_pruning_mask`` logit, both in the key order of the state dict the trainer was built
+        from, so a ``torch.optim.Adam`` built over the drop-in module's parameters that way loads it.  Logits have moments only when
+        the trainer updates them (supermask).  CPU tensors of exactly each parameter's shape (no padding); every ``step`` is
+        ``opt_step``; ``param_groups`` carry the hyper-parameters of the last step.  The extra key ``"trainer"`` holds ``step_id``,
+        ``seed``, ``mask_type`` and ``sparsity_target``.  ``exchange``: the ``distributed.ShardedExchange`` the steps ran with -
+        the moments are all-gathered from the shard owners (a collective: every rank calls it and gets the full state).  With
+        ``all_reduce`` every rank already holds the whole state.  ValueError while a SNIP saliency is pending."""
+        if self._has_saliency:
+            raise ValueError("a SNIP saliency accumulation is pending (snip_saliency without update_masks_once): it is consumed before "
+                             "training and is not part of the resumable state")
+        bufs = {"w": (self.m_w, self.v_w), "s": (self.m_s, self.v_s)}
+        if exchange is not None:
+            bufs = {"w": (self.m_w.clone(), self.v_w.clone()), "s": (self.m_s.clone(), self.v_s.clone())}
+            for phase in range(self.N_PHASES):
+                for flat, a, b in self.grad_buckets(phase):
+                    if flat is self.flat_gw or self.mask_type == "supermask":   # (the update's buckets: _sharded_step)
+                        for buf in bufs["w" if flat is self.flat_gw else "s"]:
+                            exchange.gather(buf, a, b)
+        host = {key: (m.cpu(), v.cpu()) for key, (m, v) in bufs.items()}   # (one copy per buffer, then one clone per parameter)
+        groups = []
+        for gi, entries in enumerate(self._adam_groups()):
+            m, v = host["w" if gi == 0 else "s"]
+            out = []
+            for name, offs, k in entries:
+                n, shp = self.p[k].numel(), self.p[k].shape
+                has = gi == 0 or self.mask_type == "supermask"
+                out.append((name, (m[offs[k]: offs[k] + n].view(shp).clone(), v[offs[k]: offs[k] + n].view(shp).clone()) if has else None))
+            groups.append(out)
+        # the host-side fields a later step reads: the Philox position and seed, the last mask update's target
+        trainer = {"step_id": self.step_id, "seed": self.seed, "mask_type": self.mask_type, "sparsity_target": self.sparsity_target}
+        return _export_adam(groups, self._hyper, self.opt_step, trainer)
+
+    @torch.no_grad()
+    def load_optimizer_state_dict(self, sd):
+        """Loads ``optimizer_state_dict()`` - or a ``torch.optim.Adam`` state dict in that layout - in place into ``m_w`` / ``v_w``
+        / ``m_s`` / ``v_s`` (operand pointers, rollout engines and captured graphs stay valid; the padding is zero - its moments
+        only ever move padding logits, which every update resets) and sets
+        ``opt_step``, the Adam hyper-parameters of ``optimizer_state_dict`` and, from the ``"trainer"`` key, ``step_id``, ``seed``
+        and ``sparsity_target``.  A state without that key (one saved by ``torch.optim.Adam``) continues the Philox streams of
+        masks, dropout and SCST sampling at ``step_id = opt_step``.  Every data-parallel rank loads the same file.  ValueError,
+        naming the parameter, for a different parameter count or shape, a missing state entry of an updated parameter, unequal
+        ``step`` values or another ``mask_type``."""
+        logits = self.mask_type == "supermask"
+        groups = [[(name, self.p[k].shape, gi == 0 or logits) for name, _, k in entries] for gi, entries in enumerate(self._adam_groups())]
+        moments, step, hyper, extra = _import_adam(sd, groups, self.mask_type)
+        host = {"w": (torch.zeros(self.m_w.numel()), torch.zeros(self.v_w.numel())),
+                "s": (torch.zeros(self.m_s.numel()), torch.zeros(self.v_s.numel()))}
+        for gi, entries in enumerate(self._adam_groups()):
+            m, v = host["w" if gi == 0 else "s"]
+            for name, offs, k in entries:
+                if name in moments and (gi == 0 or logits):
+                    n = self.p[k].numel()
+                    m[offs[k]: offs[k] + n].copy_(moments[name][0].reshape(-1))
+                    v[offs[k]: offs[k] + n].copy_(moments[name][1].reshape(-1))
+        for (dm, dv), key in (((self.m_w, self.v_w), "w"), ((self.m_s, self.v_s), "s")):
+            dm.copy_(host[key][0])
+            dv.copy_(host[key][1])
+        self.opt_step = step
+        self._hyper.update(hyper)
+        if extra is not None:
+            self.step_id, self.seed = int(extra["step_id"]), int(extra["seed"])
+            self.sparsity_target = extra.get("sparsity_target", self.sparsity_target)
+        else:
+            self.step_id = step
+        self._wm_step = {}   # (operands cached for a step_id)
+
 
 class ModuleTrainer:
     """``train_step`` for the configurations the fused engine does not lay out - ACORT weight sharing (``share_att_*`` /
@@ -1432,6 +1585,7 @@ class ModuleTrainer:
         self.model = model
         self.opt_step = 0
         self._mv = {}
+        self._hyper = _adam_hyper(0.0, {})
 
     def train_step(self, att_feats, boxes, seqs, masks, att_masks=None, *, seq_per_img, lr, all_reduce=None, global_tokens=None,
                    mask_lr=100.0, clip=0.1, betas=(0.9, 0.98), eps=1e-9, mask_eps=1e-2, weight_decay=0.0, grad_scale=1.0,
@@ -1467,6 +1621,7 @@ class ModuleTrainer:
             for (_, p), g in zip(params, torch._utils._unflatten_dense_tensors(flat, [p.grad for _, p in params])):
                 p.grad.copy_(g)
         self.opt_step += 1
+        self._hyper = _adam_hyper(lr, dict(mask_lr=mask_lr, betas=betas, eps=eps, mask_eps=mask_eps, weight_decay=weight_decay))
         with torch.no_grad():
             for n, p in params:
                 is_logit = n.endswith("_pruning_mask")
@@ -1533,4 +1688,48 @@ class ModuleTrainer:
 
     def state_dict(self):
         return self.model.state_dict()
+
+    # ---- resumable optimizer state (OrtTrainer.optimizer_state_dict) --------------------------------------------------------------
+    def _adam_groups(self):
+        """[[(name, parameter)]]: the trained parameters in ``named_parameters()`` order, weights, then (if any) mask logits."""
+        params = [(n, p) for n, p in self.model.named_parameters() if p.requires_grad]
+        logits = [(n, p) for n, p in params if n.endswith("_pruning_mask")]
+        return [[(n, p) for n, p in params if not n.endswith("_pruning_mask")]] + ([logits] if logits else [])
+
+    def _mask_type(self):
+        return self.model.mask_type if getattr(self.model, "MASKED", False) else None
+
+    @torch.no_grad()
+    def optimizer_state_dict(self):
+        """``OrtTrainer.optimizer_state_dict`` of the module's trained parameters: the moments of ``_mv`` in each parameter's shape
+        (zeros before the first step), ``step`` = ``opt_step``.  The ``"trainer"`` key holds the mask type and the position of the
+        process-wide Philox streams (``sampler._state`` seed, mask stream and dropout stream), so that the per-application
+        Bernoulli masks and dropout continue where they stopped."""
+        from .sampler import _state
+        groups = []
+        for entries in self._adam_groups():
+            out = []
+            for n, p in entries:
+                m, v = self._mv.get(n, (torch.zeros(p.numel()), torch.zeros(p.numel())))
+                out.append((n, (m.view(p.shape).cpu().clone(), v.view(p.shape).cpu().clone())))
+            groups.append(out)
+        trainer = {"mask_type": self._mask_type(), "seed": _state["seed"], "stream": _state["stream"], "drop": _state["drop"]}
+        return _export_adam(groups, self._hyper, self.opt_step, trainer)
+
+    @torch.no_grad()
+    def load_optimizer_state_dict(self, sd):
+        """Loads an ``optimizer_state_dict()`` (or a ``torch.optim.Adam`` state dict in that layout): the moments into ``_mv``,
+        ``opt_step``, the hyper-parameters, and the sampler's stream position from the ``"trainer"`` key.  ValueError as for
+        ``OrtTrainer.load_optimizer_state_dict``."""
+        from .sampler import _state
+        groups = self._adam_groups()
+        moments, step, hyper, extra = _import_adam(sd, [[(n, p.shape, True) for n, p in entries] for entries in groups],
+                                                   self._mask_type())
+        for entries in groups:
+            for n, p in entries:
+                self._mv[n] = tuple(t.to(device=p.device, dtype=torch.float32).reshape(-1).clone() for t in moments[n])
+        self.opt_step = step
+        self._hyper.update(hyper)
+        if extra is not None:
+            _state.update(seed=int(extra["seed"]), stream=int(extra["stream"]), drop=int(extra["drop"]))
 
