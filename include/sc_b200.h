@@ -160,7 +160,8 @@ int sc_decode_self_attn_step(const void* q, const void* k, const void* v, int ld
                              void* cache_k, void* cache_v, const int* anc, int anc_ld, int slot_div, void* out, int ldo,
                              int R, int D, int h, int n_prev, int write_slot, sc_stream_t stream);
 
-/* K6 — decoder cross-attention step over the per-image memory K/V [B*N, ldm] (models/transformer.py:255-256). */
+/* K6 — decoder cross-attention step over the per-image memory K/V [B*N, ldm] (models/transformer.py:255-256).
+ * beam <= 32 query rows per image (SC_ERR_UNSUPPORTED above); the memory K/V are read once per image at every width. */
 int sc_decode_cross_attn_step(const void* q, int ldq, const void* mem_k, const void* mem_v, int ldm, int dtype,
                               const float* att_mask, void* out, int ldo, int B, int beam, int N, int D, int h,
                               sc_stream_t stream);
@@ -170,6 +171,8 @@ int sc_decode_cross_attn_step(const void* q, int ldq, const void* mem_k, const v
  * penalty_kind: 0 "", 1 "wu_<alpha>", 2 "avg_<alpha>".  seq/lp/anc are ping-pong buffers [B*beam, L].
  * Two launches: one CTA per (image, beam) row reads its logits row once (log-softmax statistics + the row's top-`beam`
  * candidates by final score), then one small CTA per image merges the rows and does the bookkeeping.
+ * beam <= 32 (SC_ERR_UNSUPPORTED above); beams 9-32 select with a block radix select on 64-bit (score, ~index) keys, with
+ * the same tie rule (equal scores: the smaller flat index beam*V + word wins).
  * workspace: sc_beam_step_workspace_bytes(B, beam) bytes of device scratch, 16-byte aligned.
  * suppress_tok (optional int32 [B*beam], -1 = none): per-row token whose log-prob is -inf at this step (remove_bad_endings,
  * caption_model.py:161-168); penalized_col (>= 0): column whose log-prob is lowered by 1000 (suppress_UNK, :169-170);
@@ -203,7 +206,7 @@ int sc_beam_step(const float* logits, int B, int beam, int V, int L, int t, int 
  * unpenalised one.  group_seq: every group's seq ping-pong buffers as one int32 [G][2][B*beam][L] tensor (seq_in / seq_out
  * are two of them); the groups are staggered in time, so group p has run its local step min(t + group - p, L-1) already and
  * its current history is buffer (that step + 1) % 2.  Everything else as sc_beam_step / sc_beam_step_partials; group * beam
- * <= 256, and for the records path (group + 1) * beam <= 5 with sc_linear_topk candidates >= (group + 1) * beam. */
+ * <= 256, beam <= 8, and for the records path (group + 1) * beam <= 5 with sc_linear_topk candidates >= (group + 1) * beam. */
 int sc_beam_step_diverse(const float* logits, int B, int beam, int V, int L, int t, int eos, int pad, float temperature,
                          int decoding_constraint, int penalty_kind, float penalty_alpha, const int* suppress_tok, int penalized_col,
                          const int* group_seq, int group, float diversity_lambda, const int* seq_in, int* seq_out,

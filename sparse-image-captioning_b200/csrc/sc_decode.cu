@@ -286,10 +286,138 @@ __global__ void __launch_bounds__(256) cross_attn_step_kernel(const T* __restric
   }
 }
 
+// kWideChunk query rows (q rows row0 .. row0 + kWideChunk - 1, of which the first nq exist) of cross_attn_step_wide_kernel
+// against the K/V slice staged at sk / sv: the scores, softmax and PV of cross_attn_step_kernel<T, kWideChunk>, rows n < nq
+// written to out.  (A copy rather than a helper shared with that kernel: sharing changed the register allocation of the
+// <= 8-beam instantiations.)
+constexpr int kWideChunk = 8;
+template <typename T>
+__device__ __forceinline__ void cross_attn_rows(const T* __restrict__ q, int ldq, const float* __restrict__ att_mask,
+                                                T* __restrict__ out, int ldo, size_t row0, int nq, const unsigned char* sk,
+                                                const unsigned char* sv, float* sq, int rbk, int rbv, int b, int N, int hh,
+                                                int dk, int lane) {
+  constexpr int NB = kWideChunk;
+  for (int e = lane; e < NB * dk; e += 32) {
+    const int n = e / dk, d = e - n * dk;
+    sq[e] = n < nq ? sc::to_f32<T>(q[(row0 + n) * ldq + hh * dk + d]) : 0.f;
+  }
+  __syncwarp();
+  const float scale_div = sqrtf((float)dk);
+  float sc_[kMaxKeyPass][NB];
+  float mx[NB];
+#pragma unroll
+  for (int n = 0; n < NB; ++n) mx[n] = -INFINITY;
+#pragma unroll
+  for (int ps = 0; ps < kMaxKeyPass; ++ps) {
+    const int j = ps * 32 + lane;
+    float dot[NB];
+#pragma unroll
+    for (int n = 0; n < NB; ++n) dot[n] = 0.f;
+    if (ps * 32 < N && j < N) {
+      const T* kr = (const T*)(sk + (size_t)j * rbk);
+      for (int c = 0; c < dk; c += 8) {
+        Vec8<T> kk;
+        kk.load(kr + c);
+#pragma unroll
+        for (int n = 0; n < NB; ++n) {
+          const float4 q0 = *(const float4*)(sq + n * dk + c), q1 = *(const float4*)(sq + n * dk + c + 4);
+          dot[n] = fmaf(q0.x, kk.v[0], dot[n]); dot[n] = fmaf(q0.y, kk.v[1], dot[n]);
+          dot[n] = fmaf(q0.z, kk.v[2], dot[n]); dot[n] = fmaf(q0.w, kk.v[3], dot[n]);
+          dot[n] = fmaf(q1.x, kk.v[4], dot[n]); dot[n] = fmaf(q1.y, kk.v[5], dot[n]);
+          dot[n] = fmaf(q1.z, kk.v[6], dot[n]); dot[n] = fmaf(q1.w, kk.v[7], dot[n]);
+        }
+      }
+      const bool masked = att_mask && att_mask[(size_t)b * N + j] == 0.f;
+#pragma unroll
+      for (int n = 0; n < NB; ++n) {
+        float sv_ = dot[n] / scale_div;
+        if (masked) sv_ = -1e9f;
+        sc_[ps][n] = sv_;
+        mx[n] = fmaxf(mx[n], sv_);
+      }
+    } else {
+#pragma unroll
+      for (int n = 0; n < NB; ++n) sc_[ps][n] = -INFINITY;
+    }
+  }
+  float inv[NB];
+#pragma unroll
+  for (int n = 0; n < NB; ++n) {
+    const float m = sc::warp_max(mx[n]);
+    float sum = 0.f;
+#pragma unroll
+    for (int ps = 0; ps < kMaxKeyPass; ++ps) {
+      const float e = (ps * 32 + lane < N) ? expf(sc_[ps][n] - m) : 0.f;
+      sc_[ps][n] = e;
+      sum += e;
+    }
+    inv[n] = 1.f / sc::warp_sum(sum);
+  }
+  // PV: lane owns dims lane, lane+32 (d_k <= 64); V rows come from shared memory
+  float o0[NB], o1[NB];
+#pragma unroll
+  for (int n = 0; n < NB; ++n) { o0[n] = 0.f; o1[n] = 0.f; }
+  const bool d0 = lane < dk, d1 = lane + 32 < dk;
+#pragma unroll
+  for (int ps = 0; ps < kMaxKeyPass; ++ps) {
+    if (ps * 32 >= N) break;
+    const int lim = min(32, N - ps * 32);
+    for (int l = 0; l < lim; ++l) {
+      const T* vr = (const T*)(sv + (size_t)(ps * 32 + l) * rbv);
+      const float v0 = d0 ? sc::to_f32<T>(vr[lane]) : 0.f;
+      const float v1 = d1 ? sc::to_f32<T>(vr[lane + 32]) : 0.f;
+#pragma unroll
+      for (int n = 0; n < NB; ++n) {
+        const float p = __shfl_sync(0xffffffffu, sc_[ps][n], l);
+        o0[n] = fmaf(p, v0, o0[n]);
+        o1[n] = fmaf(p, v1, o1[n]);
+      }
+    }
+  }
+#pragma unroll
+  for (int n = 0; n < NB; ++n) {
+    if (n >= nq) break;
+    T* orow = out + (row0 + n) * ldo + hh * dk;
+    if (d0) orow[lane] = sc::from_f32<T>(o0[n] * inv[n]);
+    if (d1) orow[lane + 32] = sc::from_f32<T>(o1[n] * inv[n]);
+  }
+}
+
+// 9 .. 32 beams: the same per-warp staging of the (image, head) K/V slice, then kWideChunk query rows at a time, so the
+// memory K/V are still read from HBM once per image.
+template <typename T>
+__global__ void __launch_bounds__(256) cross_attn_step_wide_kernel(const T* __restrict__ q, int ldq, const T* __restrict__ mk,
+                                                                   const T* __restrict__ mv, int ldm,
+                                                                   const float* __restrict__ att_mask, T* __restrict__ out,
+                                                                   int ldo, int B, int beam, int N, int h, int dk, int warps) {
+  extern __shared__ __align__(16) unsigned char smem_x[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int w = blockIdx.x * warps + warp;
+  sc::pdl_launch();
+  sc::pdl_wait();
+  if (w >= B * h) return;
+  const int b = w / h, hh = w - b * h;
+  const int rbk = dk * (int)sizeof(T) + 16;
+  const int rbv = dk * (int)sizeof(T);
+  const int per_warp = N * (rbk + rbv) + kWideChunk * dk * 4;
+  unsigned char* base = smem_x + (size_t)warp * per_warp;
+  unsigned char* sk = base;
+  unsigned char* sv = base + (size_t)N * rbk;
+  float* sq = (float*)(sv + (size_t)N * rbv);
+  stage_rows<T>(mk + (size_t)b * N * ldm + hh * dk, ldm, sk, rbk, N, dk, lane);
+  stage_rows<T>(mv + (size_t)b * N * ldm + hh * dk, ldm, sv, rbv, N, dk, lane);
+  for (int c = 0; c < beam; c += kWideChunk) {
+    __syncwarp();  // the previous chunk's query rows have been read
+    cross_attn_rows<T>(q, ldq, att_mask, out, ldo, (size_t)b * beam + c, min(kWideChunk, beam - c), sk, sv, sq,
+                                   rbk, rbv, b, N, hh, dk, lane);
+  }
+}
+
 // ---------------------------------------------------------------------------------------------------------
 // K7 beam step.  One CTA per image.
 // ---------------------------------------------------------------------------------------------------------
-constexpr int kMaxBeam = 8;
+constexpr int kMaxBeam = 8;       // beams served by the per-thread candidate lists below
+constexpr int kMaxWideBeam = 32;  // beams served by the radix-select row pass and merge (beam > kMaxBeam)
 constexpr int kBeamThreads = 256;
 constexpr int kBeamWarps = kBeamThreads / 32;
 constexpr int kBeamRegs = 40;  // logits of one row live in registers when V <= 256*40 = 10240
@@ -822,6 +950,315 @@ __global__ void __launch_bounds__(kMergeThreads) beam_merge_kernel(const BeamArg
   if (tid == 0) a.done_count[b] = cnt;
 }
 
+
+// ---------------------------------------------------------------------------------------------------------
+// Wide beams (kMaxBeam < beam <= kMaxWideBeam).  A per-thread insertion list of `beam` candidates does not fit in
+// registers, so both phases select with a block-wide radix select on 64-bit keys (order-preserving uint32 of the final
+// score << 32 | ~flat index): the keys are all distinct and a larger key is a better candidate under `better`, so "every
+// key whose digits >= the k-th largest key's" is the exact top-k even with ties and -inf scores.
+// ---------------------------------------------------------------------------------------------------------
+__device__ __forceinline__ unsigned long long cand_key(float s, int idx) {
+  uint32_t u = __float_as_uint(s);
+  if ((u << 1) == 0u) u = 0u;  // -0.0 keyed as +0.0: equal scores tie on the index
+  u = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+  return ((unsigned long long)u << 32) | (unsigned long long)(~(uint32_t)idx);
+}
+
+struct RadixSmem {
+  unsigned hist[256];
+  unsigned wsum[kBeamWarps];
+  int bin, rem, cnt;
+};
+
+// Block-wide (kBeamThreads threads) selection of the k largest of a set of distinct keys; each(f) calls f(key) for every
+// key of the calling thread.  A key is among the k largest iff (key & mask) >= prefix.  8-bit digits from the top; the
+// passes stop once every key left under the prefix is needed.
+struct RadixCut { unsigned long long prefix, mask; };
+template <typename Each>
+__device__ __forceinline__ RadixCut radix_top(Each each, int k, RadixSmem& sm) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  unsigned long long prefix = 0ull, mask = 0ull;
+  int rem = k;
+  for (int shift = 56; shift >= 0; shift -= 8) {
+    sm.hist[tid] = 0u;
+    __syncthreads();
+    each([&](unsigned long long key) {
+      if ((key & mask) == prefix) atomicAdd(&sm.hist[(unsigned)(key >> shift) & 255u], 1u);
+    });
+    __syncthreads();
+    // inclusive scan from the top digit down: incl = keys under the prefix whose digit >= 255 - tid
+    const unsigned c = sm.hist[255 - tid];
+    unsigned incl = c;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const unsigned n = __shfl_up_sync(0xffffffffu, incl, o);
+      if (lane >= o) incl += n;
+    }
+    if (lane == 31) sm.wsum[warp] = incl;
+    __syncthreads();
+    for (int w = 0; w < warp; ++w) incl += sm.wsum[w];
+    const unsigned excl = incl - c;
+    if (excl < (unsigned)rem && incl >= (unsigned)rem) { sm.bin = 255 - tid; sm.rem = rem - (int)excl; sm.cnt = (int)c; }
+    __syncthreads();
+    prefix |= (unsigned long long)sm.bin << shift;
+    mask |= 0xffull << shift;
+    rem = sm.rem;
+    if (sm.cnt == rem) break;  // block-uniform
+  }
+  RadixCut cut;
+  cut.prefix = prefix; cut.mask = mask;
+  return cut;
+}
+
+// Phase A for wide beams — one CTA per row, as beam_row_kernel: the row is read once (registers when V <= 256*40,
+// otherwise re-read through L2 on every pass), the log-softmax statistics, then the exact final score of every column.
+// The `beam`-th largest of the threads' best keys bounds the row's `beam`-th largest key from below, so only the keys above
+// it (a few times `beam` in practice) enter the radix passes.  The row's top-`beam` candidates go to the workspace unsorted.
+template <bool kRegs>
+__global__ void __launch_bounds__(kBeamThreads, 4) beam_row_wide_kernel(const BeamArgs a, float* __restrict__ ws_stats,
+                                                                       Cand* __restrict__ ws_cand) {
+  const int beam = a.beam;
+  const int r = blockIdx.x;  // row = b*beam + k
+  const int k = r % beam;
+  sc::pdl_wait();
+  if (a.t == 0 && k != 0) return;  // first step: every beam holds BOS, only beam 0 is expanded
+  const int tid = threadIdx.x;
+  const int V = a.V;
+  __shared__ float s_red[kBeamWarps];
+  __shared__ RadixSmem s_rs;
+  __shared__ unsigned long long s_best[kBeamThreads];
+  __shared__ unsigned long long s_floor;
+  __shared__ int s_n;
+  const float T = (a.t == 0) ? 1.0f : a.temperature;
+  const float* x = a.logits + (size_t)r * V;
+  const float base = a.sum[r];
+  const int prev = (a.constraint && a.t > 0) ? a.seq_in[(size_t)r * a.L + a.t - 1] : -1;
+  const int sup = (a.suppress_tok && a.t > 0) ? a.suppress_tok[r] : -1;
+  const int pen = a.penalized_col;
+  const int flat0 = k * V;
+  float mx = -INFINITY, ls, mx2 = 0.f, ls2 = 0.f;
+  // final score of column col (the order of operations of beam_row_kernel's L2 path)
+  auto score = [&](float v, int col) {
+    float lp = (v - mx) - ls;
+    if (T != 1.0f) lp = (lp / T - mx2) - ls2;
+    if (col == prev || col == sup) lp = -INFINITY;
+    if (col == pen) lp -= 1000.f;
+    return base + lp;
+  };
+  float4 xr[kRegs ? kBeamRegs / 4 : 1];
+  if constexpr (kRegs) {
+    const float4* x4 = (const float4*)x;
+    const int V4 = V >> 2;
+#pragma unroll
+    for (int i = 0; i < kBeamRegs / 4; ++i) {
+      const int c4 = tid + i * kBeamThreads;
+      xr[i] = c4 < V4 ? __ldg(x4 + c4) : make_float4(-INFINITY, -INFINITY, -INFINITY, -INFINITY);
+      mx = fmaxf(mx, fmaxf(fmaxf(xr[i].x, xr[i].y), fmaxf(xr[i].z, xr[i].w)));
+    }
+    mx = block_max(mx, s_red);
+    sc::pdl_launch();  // the row is in registers: the merge kernel's CTAs may be scheduled
+    float se = 0.f;
+#pragma unroll
+    for (int i = 0; i < kBeamRegs / 4; ++i)
+      se += __expf(xr[i].x - mx) + __expf(xr[i].y - mx) + __expf(xr[i].z - mx) + __expf(xr[i].w - mx);
+    ls = logf(block_sum(se, s_red));
+    if (T != 1.0f) {
+      mx2 = (0.f - ls) / T;
+      float se2 = 0.f;
+#pragma unroll
+      for (int i = 0; i < kBeamRegs / 4; ++i) {
+        se2 += __expf(((xr[i].x - mx) - ls) / T - mx2) + __expf(((xr[i].y - mx) - ls) / T - mx2) +
+               __expf(((xr[i].z - mx) - ls) / T - mx2) + __expf(((xr[i].w - mx) - ls) / T - mx2);
+      }
+      ls2 = logf(block_sum(se2, s_red));
+    }
+#pragma unroll
+    for (int i = 0; i < kBeamRegs / 4; ++i) {  // the registers now hold final scores
+      const int c0 = (tid + i * kBeamThreads) * 4;
+      xr[i].x = score(xr[i].x, c0); xr[i].y = score(xr[i].y, c0 + 1);
+      xr[i].z = score(xr[i].z, c0 + 2); xr[i].w = score(xr[i].w, c0 + 3);
+    }
+  } else {
+    for (int i = tid; i < V; i += kBeamThreads) mx = fmaxf(mx, x[i]);
+    mx = block_max(mx, s_red);
+    float se = 0.f;
+    for (int i = tid; i < V; i += kBeamThreads) se += __expf(x[i] - mx);
+    ls = logf(block_sum(se, s_red));
+    if (T != 1.0f) {
+      mx2 = (0.f - ls) / T;
+      float se2 = 0.f;
+      for (int i = tid; i < V; i += kBeamThreads) se2 += __expf(((x[i] - mx) - ls) / T - mx2);
+      ls2 = logf(block_sum(se2, s_red));
+    }
+  }
+  // f(key, score, column) for every column of this thread
+  auto each_col = [&](auto f) {
+    if constexpr (kRegs) {
+#pragma unroll
+      for (int i = 0; i < kBeamRegs / 4; ++i) {
+        const int c0 = (tid + i * kBeamThreads) * 4;
+        if (c0 < V) {  // V % 4 == 0 on this path
+          f(cand_key(xr[i].x, flat0 + c0), xr[i].x, c0); f(cand_key(xr[i].y, flat0 + c0 + 1), xr[i].y, c0 + 1);
+          f(cand_key(xr[i].z, flat0 + c0 + 2), xr[i].z, c0 + 2); f(cand_key(xr[i].w, flat0 + c0 + 3), xr[i].w, c0 + 3);
+        }
+      }
+    } else {
+      for (int i = tid; i < V; i += kBeamThreads) {
+        const float s = score(__ldg(x + i), i);
+        f(cand_key(s, flat0 + i), s, i);
+      }
+    }
+  };
+  // floor = the beam-th largest of the threads' best keys (0 = no key: then every key passes)
+  unsigned long long best = 0ull;
+  each_col([&](unsigned long long key, float, int) { best = key > best ? key : best; });
+  s_best[tid] = best;
+  if (tid == 0) { s_floor = 0ull; s_n = 0; }
+  __syncthreads();
+  int above = 0;
+  for (int j = 0; j < kBeamThreads; ++j) above += s_best[j] > best;
+  if (above == beam - 1) s_floor = best;
+  __syncthreads();
+  const unsigned long long floor_key = s_floor;
+  const RadixCut cut = radix_top(
+      [&](auto f) {
+        each_col([&](unsigned long long key, float, int) {
+          if (key >= floor_key) f(key);
+        });
+      },
+      beam, s_rs);
+  each_col([&](unsigned long long key, float s, int col) {
+    if (key >= floor_key && (key & cut.mask) >= cut.prefix) {
+      Cand cd; cd.s = s; cd.idx = flat0 + col;
+      ws_cand[(size_t)r * beam + atomicAdd(&s_n, 1)] = cd;
+    }
+  });
+  if (tid == 0) {
+    ws_stats[r * 4 + 0] = mx; ws_stats[r * 4 + 1] = ls; ws_stats[r * 4 + 2] = mx2; ws_stats[r * 4 + 3] = ls2;
+  }
+}
+
+// Phase B for wide beams — one CTA per image: the top `beam` of the rows' beam x beam candidates by the same radix select,
+// ranked among themselves, then the beam bookkeeping of beam_merge_kernel (a copy rather than a shared helper: sharing
+// changed the register allocation of the <= 8-beam merge).
+__global__ void __launch_bounds__(kBeamThreads) beam_merge_wide_kernel(const BeamArgs a, const float* __restrict__ ws_stats,
+                                                                       const Cand* __restrict__ ws_cand) {
+  const int b = blockIdx.x;
+  const int tid = threadIdx.x;
+  const int beam = a.beam;
+  sc::pdl_launch();
+  sc::pdl_wait();
+  const int n = ((a.t == 0) ? 1 : beam) * beam;
+  __shared__ unsigned long long s_key[kMaxWideBeam * kMaxWideBeam];
+  __shared__ RadixSmem s_rs;
+  __shared__ unsigned long long s_sel[kMaxWideBeam];
+  __shared__ int s_sel_src[kMaxWideBeam];
+  __shared__ Cand s_final[kMaxWideBeam];
+  __shared__ int s_src[kMaxWideBeam];
+  __shared__ int s_n, s_pos, s_last;
+  const Cand* cand = ws_cand + (size_t)b * beam * beam;
+  for (int i = tid; i < n; i += kBeamThreads) s_key[i] = cand_key(cand[i].s, cand[i].idx);
+  if (tid == 0) s_n = 0;
+  __syncthreads();
+  const RadixCut cut = radix_top(
+      [&](auto f) {
+        for (int i = tid; i < n; i += kBeamThreads) f(s_key[i]);
+      },
+      beam, s_rs);
+  for (int i = tid; i < n; i += kBeamThreads) {
+    if ((s_key[i] & cut.mask) >= cut.prefix) {
+      const int j = atomicAdd(&s_n, 1);
+      s_sel[j] = s_key[i];
+      s_sel_src[j] = i;
+    }
+  }
+  __syncthreads();
+  if (tid < beam) {
+    int rank = 0;
+    for (int j = 0; j < beam; ++j) rank += s_sel[j] > s_sel[tid];
+    s_final[rank] = cand[s_sel_src[tid]];
+    s_src[rank] = s_sel_src[tid];
+  }
+  __syncthreads();
+  // the bookkeeping of beam_merge_kernel with nb = beam winners and kBeamThreads threads
+  const int nb = beam;
+  const int V = a.V;
+  const float T = (a.t == 0) ? 1.0f : a.temperature;
+  const int L = a.L, t = a.t;
+  for (int e = tid; e < nb * L; e += kBeamThreads) {
+    const int j = e / L, s = e - j * L;
+    const int parent = s_final[j].idx / V;
+    const size_t src = ((size_t)b * nb + parent) * L + s, dst = ((size_t)b * nb + j) * L + s;
+    if (s < t) {
+      a.seq_out[dst] = a.seq_in[src];
+      a.lp_out[dst] = a.lp_in[src];
+      a.anc_out[dst] = a.anc_in[src];
+    } else if (s == t) {
+      const int word = s_final[j].idx - parent * V;
+      a.seq_out[dst] = word;
+      const float x = a.logits ? a.logits[((size_t)b * nb + parent) * V + word] : a.ws_raw[(size_t)b * nb * nb + s_src[j]];
+      const float* st = ws_stats + ((size_t)b * nb + parent) * 4;
+      float lp = (x - st[0]) - st[1];
+      if (T != 1.0f) lp = (lp / T - st[2]) - st[3];
+      if (word == a.penalized_col) lp -= 1000.f;
+      a.lp_out[dst] = lp;
+      a.anc_out[dst] = b * nb + parent;
+    } else {
+      a.seq_out[dst] = a.pad;
+      a.lp_out[dst] = 0.f;
+      a.anc_out[dst] = b * nb + j;  // slots of future steps are written by the row itself
+    }
+  }
+  __syncthreads();
+  // finished beams: stable insertion into the running top-nb (python's sorted() is stable and entries arrive
+  // chronologically); thread 0 picks the slot, L threads move the rows.
+  int cnt = a.done_count[b];
+  for (int j = 0; j < nb; ++j) {
+    const int parent = s_final[j].idx / V;
+    const int word = s_final[j].idx - parent * V;
+    float ys = s_final[j].s;
+    const bool is_end = (word == a.eos) || (t == L - 1);
+    if (is_end) {
+      if (tid == 0) {
+        // the reference scores finished beams in Python floats (double): model_utils.py:121-146
+        double p = (double)ys;
+        const double len = (double)(t + 1);
+        if (a.penalty_kind == 1) p = p / (pow(5.0 + len, (double)a.penalty_alpha) / pow(6.0, (double)a.penalty_alpha));
+        else if (a.penalty_kind == 2) p = p / len;
+        int pos = cnt < nb ? cnt : nb;
+        while (pos > 0 && a.done_p[b * nb + pos - 1] < p) --pos;
+        const int last = (cnt < nb ? cnt : nb - 1);
+        if (pos < nb) {
+          for (int m = last; m > pos; --m) a.done_p[b * nb + m] = a.done_p[b * nb + m - 1];
+          a.done_p[b * nb + pos] = p;
+        }
+        s_pos = pos; s_last = last;
+      }
+      __syncthreads();
+      const int pos = s_pos, last = s_last;
+      if (pos < nb) {
+        for (int s = tid; s < L; s += kBeamThreads) {
+          for (int m = last; m > pos; --m) {
+            a.done_seq[((size_t)b * nb + m) * L + s] = a.done_seq[((size_t)b * nb + m - 1) * L + s];
+            a.done_lp[((size_t)b * nb + m) * L + s] = a.done_lp[((size_t)b * nb + m - 1) * L + s];
+          }
+          const size_t src = ((size_t)b * nb + j) * L + s;
+          a.done_seq[((size_t)b * nb + pos) * L + s] = s <= t ? a.seq_out[src] : a.pad;
+          a.done_lp[((size_t)b * nb + pos) * L + s] = s <= t ? a.lp_out[src] : 0.f;
+        }
+        if (cnt < nb) cnt++;
+      }
+      __syncthreads();
+      ys -= 1000.f;
+    }
+    if (tid == 0) {
+      a.tokens_out[b * nb + j] = word;
+      a.sum[b * nb + j] = ys;
+    }
+  }
+  if (tid == 0) a.done_count[b] = cnt;
+}
+
 // greedy step (beam_size == 1): one warp per row
 __global__ void __launch_bounds__(256) greedy_step_kernel(const float* __restrict__ logits, int R, int V, int L, int t,
                                                           int eos, int constraint, int* __restrict__ seq,
@@ -973,7 +1410,7 @@ int sc_decode_cross_attn_step(const void* q, int ldq, const void* mem_k, const v
   SC_CHECK(dk % 8 == 0 && dk <= 256 && (dk & (dk - 1)) == 0, SC_ERR_UNSUPPORTED,
            "sc_decode_cross_attn_step: d_k=%d must be a power of two in [8,256]", dk);
   SC_CHECK(ldq % 8 == 0 && ldm % 8 == 0 && ldo % 8 == 0, SC_ERR_ALIGN, "sc_decode_cross_attn_step: ld %% 8");
-  SC_CHECK(beam <= kMaxBeam, SC_ERR_UNSUPPORTED, "sc_decode_cross_attn_step: beam=%d > %d", beam, kMaxBeam);
+  SC_CHECK(beam <= kMaxWideBeam, SC_ERR_UNSUPPORTED, "sc_decode_cross_attn_step: beam=%d > %d", beam, kMaxWideBeam);
   SC_CHECK(N <= 32 * kMaxKeyPass, SC_ERR_UNSUPPORTED, "sc_decode_cross_attn_step: N=%d > %d memory slots", N, 32 * kMaxKeyPass);
   SC_CHECK(dk <= 64, SC_ERR_UNSUPPORTED, "sc_decode_cross_attn_step: d_k=%d > 64", dk);
   if (dtype == SC_BF16 && dk == 64) {
@@ -981,7 +1418,7 @@ int sc_decode_cross_attn_step(const void* q, int ldq, const void* mem_k, const v
     if (rc != SC_ERR_UNSUPPORTED) return rc;
   }
   const int esz = dtype == SC_F32 ? 4 : 2;
-  const size_t per_warp = (size_t)N * (2 * dk * esz + 16) + (size_t)beam * dk * 4;
+  const size_t per_warp = (size_t)N * (2 * dk * esz + 16) + (size_t)(beam > kMaxBeam ? kWideChunk : beam) * dk * 4;
   int warps = (int)((96 * 1024) / per_warp);
   if (warps > 8) warps = 8;
   SC_CHECK(warps >= 1, SC_ERR_UNSUPPORTED, "sc_decode_cross_attn_step: N=%d too large for shared memory", N);
@@ -1005,9 +1442,22 @@ int sc_decode_cross_attn_step(const void* q, int ldq, const void* mem_k, const v
     case 5: XATT(T, 5); break; case 6: XATT(T, 6); break;   \
     case 7: XATT(T, 7); break; default: XATT(T, 8); break;  \
   }
-  if (dtype == SC_F32) { XATT_NB(float) }
+#define XATT_WIDE(T)                                                                                                   \
+  do {                                                                                                                 \
+    static bool attr_w = false;                                                                                        \
+    if (!attr_w) {                                                                                                     \
+      cudaFuncSetAttribute(cross_attn_step_wide_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);   \
+      attr_w = true;                                                                                                   \
+    }                                                                                                                  \
+    sc::launch_pdl(cross_attn_step_wide_kernel<T>, dim3(blocks), dim3(32 * warps), smem, stream, (const T*)q, ldq,     \
+                   (const T*)mem_k, (const T*)mem_v, ldm, att_mask, (T*)out, ldo, B, beam, N, h, dk, warps);           \
+  } while (0)
+  if (beam > kMaxBeam && dtype == SC_F32) XATT_WIDE(float);
+  else if (beam > kMaxBeam && dtype == SC_BF16) XATT_WIDE(__nv_bfloat16);
+  else if (dtype == SC_F32) { XATT_NB(float) }
   else if (dtype == SC_BF16) { XATT_NB(__nv_bfloat16) }
   else SC_CHECK(false, SC_ERR_DTYPE, "sc_decode_cross_attn_step: bad dtype %d", dtype);
+#undef XATT_WIDE
 #undef XATT_NB
 #undef XATT
   SC_LAUNCH_CHECK("sc_decode_cross_attn_step");
@@ -1022,7 +1472,9 @@ size_t sc_beam_step_workspace_bytes_impl(int B, int beam) {
 // Row pass + merge over materialised logits; a.div_hist != nullptr selects the diverse-beam row pass.
 static int beam_step_launch(const char* name, const BeamArgs& a, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
   const int B = a.B, beam = a.beam, V = a.V, L = a.L, t = a.t;
-  SC_CHECK(B > 0 && beam >= 1 && beam <= kMaxBeam, SC_ERR_UNSUPPORTED, "%s: beam=%d not in [1,%d]", name, beam, kMaxBeam);
+  const bool div = a.div_hist != nullptr;
+  const int max_beam = div ? kMaxBeam : kMaxWideBeam;  // diverse beam search: beams per group
+  SC_CHECK(B > 0 && beam >= 1 && beam <= max_beam, SC_ERR_UNSUPPORTED, "%s: beam=%d not in [1,%d]", name, beam, max_beam);
   SC_CHECK(V >= beam && L > 0 && t >= 0 && t < L, SC_ERR_SHAPE, "%s: V=%d L=%d t=%d", name, V, L, t);
   SC_CHECK(a.temperature > 0.f, SC_ERR_SHAPE, "%s: temperature must be > 0", name);
   SC_CHECK(workspace != nullptr && ((uintptr_t)workspace & 15) == 0 && workspace_bytes >= sc_beam_step_workspace_bytes_impl(B, beam),
@@ -1031,7 +1483,13 @@ static int beam_step_launch(const char* name, const BeamArgs& a, void* workspace
   float* ws_stats = (float*)workspace;
   Cand* ws_cand = (Cand*)(ws_stats + (size_t)B * beam * 4);
   const bool regs = V <= kBeamThreads * kBeamRegs && (V & 3) == 0 && ((uintptr_t)a.logits & 15) == 0;
-  const bool div = a.div_hist != nullptr;
+  if (beam > kMaxBeam) {
+    if (regs) sc::launch_pdl(beam_row_wide_kernel<true>, dim3(B * beam), dim3(kBeamThreads), 0, stream, a, ws_stats, ws_cand);
+    else sc::launch_pdl(beam_row_wide_kernel<false>, dim3(B * beam), dim3(kBeamThreads), 0, stream, a, ws_stats, ws_cand);
+    sc::launch_pdl(beam_merge_wide_kernel, dim3(B), dim3(kBeamThreads), 0, stream, a, (const float*)ws_stats, (const Cand*)ws_cand);
+    SC_LAUNCH_CHECK(name);
+    return SC_OK;
+  }
 #define BEAM_LAUNCH(NBV)                                                                                                     \
   do {                                                                                                                        \
     if (div && regs) sc::launch_pdl(beam_row_kernel<NBV, true, true>, dim3(B * NBV), dim3(kBeamThreads), 0, stream, a, ws_stats, ws_cand);   \

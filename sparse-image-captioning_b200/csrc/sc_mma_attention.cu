@@ -252,6 +252,38 @@ __global__ void __launch_bounds__(256) cross_attn_mma_kernel(const CrossAttnArgs
   store_rows(sQ, a.NB, a.out + (size_t)b * a.NB * a.ldo + hh * kDk, a.ldo, lane);
 }
 
+// 17 .. 32 beams: cross_attn_mma_kernel with a second query m-tile against the same staged K / V (a separate kernel so that
+// the <= 16-beam kernel keeps its code).
+template <int NT>
+__global__ void __launch_bounds__(256) cross_attn_mma_wide_kernel(const CrossAttnArgs a) {
+  extern __shared__ __align__(16) unsigned char smem_x[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int w = blockIdx.x * a.warps + warp;
+  // smem: [zero row][warp 0: Q (beam rows) K V (N rows each)][warp 1: ...]
+  if (threadIdx.x < kPitch / 16) *(uint4*)(smem_x + threadIdx.x * 16) = make_uint4(0u, 0u, 0u, 0u);
+  sc::pdl_launch();
+  sc::pdl_wait();
+  const int N = a.N;
+  const bool live = w < a.B * a.h;
+  const int b = live ? w / a.h : 0, hh = live ? w - b * a.h : 0;
+  unsigned char* sQ = smem_x + kPitch + (size_t)warp * (2 * N + a.NB) * kPitch;
+  unsigned char* sK = sQ + a.NB * kPitch;
+  unsigned char* sV = sK + N * kPitch;
+  if (live) {
+    stage_tile(a.q + (size_t)b * a.NB * a.ldq + hh * kDk, a.ldq, a.NB, sQ, lane);
+    stage_tile(a.mk + (size_t)b * N * a.ldm + hh * kDk, a.ldm, N, sK, lane);
+    stage_tile(a.mv + (size_t)b * N * a.ldm + hh * kDk, a.ldm, N, sV, lane);
+  }
+  cp_async_wait_all();
+  __syncthreads();  // (the zero row is shared by the CTA's warps)
+  if (!live) return;
+  const float* km = a.att_mask ? a.att_mask + (size_t)b * N : nullptr;
+  attn_mtile<NT>(sQ, sK, sV, 0, a.NB, N, nullptr, 0, km, lane, smem_u32(smem_x));
+  attn_mtile<NT>(sQ, sK, sV, 16, a.NB, N, nullptr, 0, km, lane, smem_u32(smem_x));
+  __syncwarp();
+  store_rows(sQ, a.NB, a.out + (size_t)b * a.NB * a.ldo + hh * kDk, a.ldo, lane);
+}
+
 // ---- geometry bias for all layers: bias[l, b, hh, i, j] = log(max(relu(WG_{l,hh} . emb(i,j) + b_{l,hh}), 1e-6)) ----
 struct DimMat8 { float v[8]; };
 
@@ -545,7 +577,7 @@ int sc_bias_attention_fwd(const void* q, const void* k, const void* v, int ldq, 
 // (sc_decode_cross_attn_step in sc_decode.cu then runs its generic kernel).
 int sc_cross_attn_mma_launch(const void* q, int ldq, const void* mem_k, const void* mem_v, int ldm, const float* att_mask,
                              void* out, int ldo, int B, int beam, int N, int h, cudaStream_t stream) {
-  if (beam > 16 || N > 128) return SC_ERR_UNSUPPORTED;
+  if (beam > 32 || N > 128) return SC_ERR_UNSUPPORTED;
   if ((((uintptr_t)q | (uintptr_t)mem_k | (uintptr_t)mem_v | (uintptr_t)out) & 15) != 0) return SC_ERR_UNSUPPORTED;
   CrossAttnArgs a;
   a.q = (const __nv_bfloat16*)q; a.ldq = ldq; a.mk = (const __nv_bfloat16*)mem_k; a.mv = (const __nv_bfloat16*)mem_v; a.ldm = ldm;
@@ -559,19 +591,24 @@ int sc_cross_attn_mma_launch(const void* q, int ldq, const void* mem_k, const vo
   a.warps = warps;
   const size_t smem = per_warp * warps + kPitch;
   const int blocks = (B * h + warps - 1) / warps;
-#define X_CASE(NTV)                                                                                                \
+#define X_CASE(KERN, NTV)                                                                                          \
   case NTV: {                                                                                                      \
     static bool attr = false;                                                                                      \
     if (!attr) {                                                                                                   \
-      cudaFuncSetAttribute(cross_attn_mma_kernel<NTV>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);   \
+      cudaFuncSetAttribute(KERN<NTV>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);                    \
       attr = true;                                                                                                 \
     }                                                                                                              \
-    sc::launch_pdl(cross_attn_mma_kernel<NTV>, dim3(blocks), dim3(32 * warps), smem, stream, a);                   \
+    sc::launch_pdl(KERN<NTV>, dim3(blocks), dim3(32 * warps), smem, stream, a);                                    \
   } break
-  switch (NT) {
-    X_CASE(1); X_CASE(2); X_CASE(3); X_CASE(4); X_CASE(5); X_CASE(6); X_CASE(7); X_CASE(8);
-    default: return SC_ERR_UNSUPPORTED;
+#define X_CASES(KERN)                                                                                              \
+  switch (NT) {                                                                                                    \
+    X_CASE(KERN, 1); X_CASE(KERN, 2); X_CASE(KERN, 3); X_CASE(KERN, 4);                                            \
+    X_CASE(KERN, 5); X_CASE(KERN, 6); X_CASE(KERN, 7); X_CASE(KERN, 8);                                            \
+    default: return SC_ERR_UNSUPPORTED;                                                                            \
   }
+  if (beam > 16) { X_CASES(cross_attn_mma_wide_kernel) }
+  else { X_CASES(cross_attn_mma_kernel) }
+#undef X_CASES
 #undef X_CASE
   SC_LAUNCH_CHECK("sc_decode_cross_attn_step");
   return SC_OK;
