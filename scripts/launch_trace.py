@@ -59,7 +59,7 @@ def _lookup(p):
 
 
 class Ptr(int):
-    """A pointer from lib.ptr: described through the storage table, never as its value."""
+    """The pointer lib.call passes for a tensor: described through the storage table, never as its value."""
 
 
 _tables = {}       # id -> (table, number of leading pointer columns) of the descriptor tables built by the run
@@ -180,12 +180,9 @@ PURE = {"linear_topk_parts": K.linear_topk_parts, "beam_step_workspace_bytes": l
 for _name, _f in list(vars(K).items()):
     if isinstance(_f, types.FunctionType) and _f.__module__ == K.__name__ and _name not in KEEP and not _name.startswith("__"):
         setattr(K, _name, _stub(_name, _f))
-K._chk = lambda t, name: None
 
 
 def _ptr(t):
-    if t is None:
-        return None
     _ordinal(t)
     return Ptr(t.data_ptr())
 
@@ -197,18 +194,17 @@ def _mask_descriptors(items, device, _build=K.mask_descriptors):
 
 
 K.mask_descriptors = _mask_descriptors
-
-
-lib.ptr = _ptr
+lib.address = lambda t, name, pname: 0 if t is None else t.data_ptr()   # (the traced tensors live on the CPU)
 
 
 def _call(name, *a, meta=None):
+    """Records the arguments the library would receive: a tensor as its pointer, then the stream (every entry point called
+    through lib.call ends in its stream)."""
     with _recording():
-        TRACE.append([name, _current[-1].id, desc(a)])
+        TRACE.append([name, _current[-1].id, desc([_ptr(x) if torch.is_tensor(x) else x for x in a] + [_current[-1].id])])
 
 
 lib.call = _call
-lib.stream = lambda: _current[-1].id
 lib.load = lambda: types.SimpleNamespace(sc_adam_clip_st_chunk=lambda: 4096, sc_prune_chunk=lambda: 4096, sc_set_pdl=lambda m: 0)
 
 

@@ -103,9 +103,8 @@ class CiderD:
         hi = hyp_image.to(self.dev, torch.int32).contiguous()
         out = torch.empty(H, dtype=torch.float64, device=self.dev)
         r = self._refs
-        lib.call("sc_ciderd_score", lib.ptr(h), H, L, lib.ptr(hi), self.eos, self.pad, lib.ptr(self.df_keys), lib.ptr(self.df_log), self.n_df,
-                 self.ref_len, self.sigma, lib.ptr(r["img_off"]), lib.ptr(r["ng_off"]), lib.ptr(r["keys"]), lib.ptr(r["vec"]),
-                 lib.ptr(r["norm"]), lib.ptr(r["length"]), lib.ptr(out), lib.stream())
+        lib.call("sc_ciderd_score", h, H, L, hi, self.eos, self.pad, self.df_keys, self.df_log, self.n_df, self.ref_len, self.sigma,
+                 r["img_off"], r["ng_off"], r["keys"], r["vec"], r["norm"], r["length"], out)
         return out
 
     def scst_reward(self, sample_seq: torch.Tensor, baseline_seq: Optional[torch.Tensor] = None, cider_weight: float = 1.0,

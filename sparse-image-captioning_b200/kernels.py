@@ -1,7 +1,8 @@
 """Tensor-level wrappers over the C ABI (one Python function per entry point of include/sc_b200.h).
 
-All tensors must be CUDA tensors; outputs are allocated by the caller or here with torch (plumbing only).
-Every function launches on torch's current stream, so calls are CUDA-graph capturable.
+All tensors must be CUDA tensors on the current device (lib.call checks every pointer argument); outputs are allocated by
+the caller or here with torch (plumbing only).  Every function launches on torch's current stream, so calls are CUDA-graph
+capturable.
 """
 import contextlib
 import math
@@ -12,29 +13,18 @@ from . import lib
 from .lib import F32, BF16, MASK_NONE, MASK_ROUND, MASK_BERNOULLI, MASK_RAW, MASK_UNIFORM  # noqa: F401
 
 
-def _chk(t, name):
-    if t is not None:
-        if not t.is_cuda:
-            raise RuntimeError(f"{name} must be a CUDA tensor: the B200 path has no CPU fallback")
-        if not t.is_contiguous():
-            raise RuntimeError(f"{name} must be contiguous")
-
-
 def linear(x, w, bias=None, *, mask=None, mask_mode=MASK_NONE, uniforms=None, seed=0, stream_id=0, residual=None,
            relu=False, out=None, out_dtype=None, tile_n=0):
     """y = epilogue(x @ (w (.) mask)^T): sc_linear.  x [M,K] bf16|fp32, w [N,K] bf16|fp32."""
     M, K = x.shape
     N = w.shape[0]
     assert w.shape[1] == K, (w.shape, x.shape)
-    for t, n in ((x, "x"), (w, "w"), (mask, "mask"), (uniforms, "uniforms"), (bias, "bias"), (residual, "residual")):
-        _chk(t, n)
     if out is None:
         out = torch.empty(M, N, device=x.device, dtype=out_dtype or torch.float32)
     if mask is None:
         mask_mode = MASK_NONE
-    lib.call("sc_linear", lib.ptr(x), lib.dtype_code(x.dtype), lib.ptr(w), lib.dtype_code(w.dtype), lib.ptr(mask),
-             mask_mode, lib.ptr(uniforms), seed, stream_id, lib.ptr(bias), lib.ptr(residual), lib.ptr(out),
-             lib.dtype_code(out.dtype), M, N, K, int(relu), tile_n, lib.stream(),
+    lib.call("sc_linear", x, lib.dtype_code(x.dtype), w, lib.dtype_code(w.dtype), mask, mask_mode, uniforms, seed, stream_id,
+             bias, residual, out, lib.dtype_code(out.dtype), M, N, K, int(relu), tile_n,
              meta=("gemm_bf16" if x.dtype == torch.bfloat16 else "gemm_f32", M, N, K, x.element_size(), w.element_size(),
                    out.element_size(), mask is not None, residual is not None, bool(relu), tile_n))
     return out
@@ -47,12 +37,9 @@ def linear_ln(x, w, bias=None, *, residual=None, relu=False, out=None, tile_n=0,
     M, K = x.shape
     N = w.shape[0]
     assert x.dtype == torch.bfloat16 and w.dtype == torch.bfloat16 and w.shape[1] == K
-    for t, n in ((x, "x"), (w, "w"), (bias, "bias"), (residual, "residual"), (out, "out"), (ln_stats, "ln_stats"), (ln_c, "ln_c"),
-                 (out_bf16, "out_bf16"), (stats_out, "stats_out")):
-        _chk(t, n)
-    lib.call("sc_linear_ln", lib.ptr(x), lib.ptr(w), lib.ptr(bias), lib.ptr(residual), lib.ptr(out), lib.dtype_code(out.dtype),
-             M, N, K, int(relu), tile_n, lib.ptr(ln_stats), lib.ptr(ln_c), float(eps), lib.ptr(out_bf16), lib.ptr(stats_out),
-             lib.stream(), meta=("gemm_bf16", M, N, K, 2, 2, out.element_size(), False, residual is not None, bool(relu)))
+    lib.call("sc_linear_ln", x, w, bias, residual, out, lib.dtype_code(out.dtype), M, N, K, int(relu), tile_n, ln_stats, ln_c,
+             float(eps), out_bf16, stats_out,
+             meta=("gemm_bf16", M, N, K, 2, 2, out.element_size(), False, residual is not None, bool(relu)))
     return out
 
 
@@ -109,11 +96,10 @@ def csr_spmm(x, csr, bias=None, *, residual=None, relu=False, out=None, out_dtyp
     M, K = x.shape
     N = csr.shape[0]
     assert csr.shape[1] == K and csr.val.dtype == x.dtype
-    _chk(x, "x")
     if out is None:
         out = torch.empty(M, N, device=x.device, dtype=out_dtype or torch.float32)
-    lib.call("sc_csr_spmm", lib.ptr(x), lib.dtype_code(x.dtype), lib.ptr(csr.row_ptr), lib.ptr(csr.col), lib.ptr(csr.val),
-             lib.ptr(bias), lib.ptr(residual), lib.ptr(out), lib.dtype_code(out.dtype), M, N, K, int(relu), lib.stream(),
+    lib.call("sc_csr_spmm", x, lib.dtype_code(x.dtype), csr.row_ptr, csr.col, csr.val, bias, residual, out,
+             lib.dtype_code(out.dtype), M, N, K, int(relu),
              meta=("csr_spmm", M, N, K, x.element_size(), csr.nnz, out.element_size()))
     return out
 
@@ -170,11 +156,10 @@ def sell_spmm(x, sw, bias=None, *, residual=None, relu=False, out=None, out_dtyp
     M, K = x.shape
     N = sw.shape[0]
     assert sw.shape[1] == K and sw.dtype == x.dtype
-    _chk(x, "x")
     if out is None:
         out = torch.empty(M, N, device=x.device, dtype=out_dtype or torch.float32)
-    lib.call("sc_sell_spmm", lib.ptr(x), lib.dtype_code(x.dtype), lib.ptr(sw.slab_ptr), lib.ptr(sw.entries), lib.ptr(bias),
-             lib.ptr(residual), lib.ptr(out), lib.dtype_code(out.dtype), M, N, K, int(relu), lib.stream(),
+    lib.call("sc_sell_spmm", x, lib.dtype_code(x.dtype), sw.slab_ptr, sw.entries, bias, residual, out, lib.dtype_code(out.dtype),
+             M, N, K, int(relu),
              meta=("sell_spmm", M, N, K, x.element_size(), sw.nnz, out.element_size()))
     return out
 
@@ -254,32 +239,28 @@ def gspmm(x, gw, bias=None, *, residual=None, relu=False, out=None, out_dtype=No
     """y = act(x W^T + b) + residual with W in gather-SpMM form (sc_gspmm: mma.sync over gathered activation columns)."""
     M, K = x.shape
     N = gw.shape[0]
-    assert gw.shape[1] == K and x.dtype == torch.bfloat16 and x.stride(1) == 1
+    assert gw.shape[1] == K and x.dtype == torch.bfloat16
     if out is None:
         out = torch.empty(M, N, device=x.device, dtype=out_dtype or torch.float32)
-    _chk(out, "out")
-    lib.call("sc_gspmm", lib.ptr(x), x.stride(0), lib.ptr(gw.grp_ptr), lib.ptr(gw.entries), lib.ptr(bias), lib.ptr(residual),
-             lib.ptr(out), lib.dtype_code(out.dtype), M, N, K, int(relu), lib.stream(),
+    lib.call("sc_gspmm", lib.Strided(x), x.stride(0), gw.grp_ptr, gw.entries, bias, residual, out, lib.dtype_code(out.dtype),
+             M, N, K, int(relu),
              meta=("gspmm", M, N, K, 2, gw.nnz, out.element_size()))
     return out
 
 
 def ingest_f32_bf16(host_pinned, out, ctas=0):
     """out (device bf16) = cast(host_pinned fp32): the kernel reads the pinned host tensor over PCIe itself (sc_ingest_f32_bf16)."""
-    assert host_pinned.device.type == "cpu" and host_pinned.is_pinned() and host_pinned.dtype == torch.float32 and host_pinned.is_contiguous()
-    assert out.is_cuda and out.dtype == torch.bfloat16 and out.numel() == host_pinned.numel() and out.is_contiguous()
-    lib.call("sc_ingest_f32_bf16", host_pinned.data_ptr(), lib.ptr(out), host_pinned.numel(), int(ctas), lib.stream())
+    assert host_pinned.dtype == torch.float32 and out.dtype == torch.bfloat16 and out.numel() == host_pinned.numel()
+    lib.call("sc_ingest_f32_bf16", host_pinned, out, host_pinned.numel(), int(ctas))
     return out
 
 
 def layernorm(x, a, b, *, eps=1e-6, out=None, out_dtype=None):
     rows, D = x.shape
-    _chk(x, "x")
     assert x.dtype == torch.float32
     if out is None:
         out = torch.empty(rows, D, device=x.device, dtype=out_dtype or torch.float32)
-    lib.call("sc_layernorm", lib.ptr(x), lib.ptr(a), lib.ptr(b), lib.ptr(out), lib.dtype_code(out.dtype), rows, D, eps,
-             lib.stream())
+    lib.call("sc_layernorm", x, a, b, out, lib.dtype_code(out.dtype), rows, D, eps)
     return out
 
 
@@ -292,8 +273,8 @@ def embed_pe(tokens, table, pe, *, T=1, pos0=0, mask=None, mask_mode=MASK_NONE, 
         out = torch.empty(rows, D, device=table.device, dtype=out_dtype or torch.float32)
     if mask is None:
         mask_mode = MASK_NONE
-    lib.call("sc_embed_pe", lib.ptr(tokens), lib.ptr(table), lib.ptr(mask), mask_mode, lib.ptr(uniforms), seed, stream_id,
-             lib.ptr(pe), lib.ptr(out), lib.dtype_code(out.dtype), rows, D, V, T, pos0, math.sqrt(D), lib.stream())
+    lib.call("sc_embed_pe", tokens, table, mask, mask_mode, uniforms, seed, stream_id, pe, out, lib.dtype_code(out.dtype), rows, D,
+             V, T, pos0, math.sqrt(D))
     return out
 
 
@@ -302,19 +283,16 @@ def embed_pe_stats(tokens, table, pe, x32, xb, stats, *, T=1, pos0=0):
     rows = tokens.numel()
     V, D = table.shape
     assert tokens.dtype == torch.int32 and xb.dtype == torch.bfloat16 and x32.dtype == torch.float32
-    lib.call("sc_embed_pe_stats", lib.ptr(tokens), lib.ptr(table), lib.ptr(pe), lib.ptr(x32), lib.ptr(xb), lib.ptr(stats), rows, D, V,
-             T, pos0, math.sqrt(D), lib.stream())
+    lib.call("sc_embed_pe_stats", tokens, table, pe, x32, xb, stats, rows, D, V, T, pos0, math.sqrt(D))
     return x32
 
 
 def apply_mask(w, mask, mask_mode, *, uniforms=None, seed=0, stream_id=0, out_dtype=torch.float32, out=None):
-    _chk(w, "w")
     if out is None:
         out = torch.empty(w.shape, device=w.device, dtype=out_dtype)
     if mask is None:
         mask_mode = MASK_NONE
-    lib.call("sc_apply_mask", lib.ptr(w), lib.ptr(mask), mask_mode, lib.ptr(uniforms), seed, stream_id, lib.ptr(out),
-             lib.dtype_code(out.dtype), w.numel(), lib.stream())
+    lib.call("sc_apply_mask", w, mask, mask_mode, uniforms, seed, stream_id, out, lib.dtype_code(out.dtype), w.numel())
     return out
 
 
@@ -323,30 +301,27 @@ def mask_count(logits_list, out=None):
     dev = logits_list[0].device
     cnt = torch.zeros(1, dtype=torch.int64, device=dev) if out is None else out.zero_()
     for s in logits_list:
-        _chk(s, "logits")
-        lib.call("sc_mask_count", lib.ptr(s), s.numel(), lib.ptr(cnt), lib.stream())
+        lib.call("sc_mask_count", s, s.numel(), cnt)
     return cnt
 
 
 def cast_bf16(x, out=None):
-    _chk(x, "x")
     if out is None:
         out = torch.empty(x.shape, device=x.device, dtype=torch.bfloat16)
-    lib.call("sc_cast_f32_bf16", lib.ptr(x), lib.ptr(out), x.numel(), lib.stream())
+    lib.call("sc_cast_f32_bf16", x, out, x.numel())
     return out
 
 
 def mask_rows(x, row_mask):
     rows, D = x.shape
-    lib.call("sc_mask_rows", lib.ptr(x), lib.ptr(row_mask), rows, D, lib.stream())
+    lib.call("sc_mask_rows", x, row_mask, rows, D)
     return x
 
 
 def box_attention(q, k, v, boxes, wg_w, wg_b, att_mask, out, *, B, N, h, dk, ldq, ldk, ldv, ldo, trig=True,
                   wave_len=1000.0):
-    lib.call("sc_box_attention_fwd", lib.ptr(q), lib.ptr(k), lib.ptr(v), ldq, ldk, ldv, lib.dtype_code(out.dtype),
-             lib.ptr(boxes), lib.ptr(wg_w), lib.ptr(wg_b), lib.ptr(att_mask), lib.ptr(out), ldo, B, N, h, dk, int(trig),
-             wave_len, lib.stream())
+    lib.call("sc_box_attention_fwd", lib.Strided(q), lib.Strided(k), lib.Strided(v), ldq, ldk, ldv, lib.dtype_code(out.dtype),
+             boxes, wg_w, wg_b, att_mask, lib.Strided(out), ldo, B, N, h, dk, int(trig), wave_len)
     return out
 
 
@@ -355,33 +330,29 @@ def box_bias_all(boxes, wg_w, wg_b, out, *, B, N, layers, h, trig=True, wave_len
     ``tensor_cores``: the TF32 mma variant of the bf16 inference path (sc_box_bias_all_tc) when the shape is served."""
     if (tensor_cores and trig and (layers * h) % 8 == 0 and layers * h <= 64 and 4 <= N <= 2048
             and layers * h * B * N * N * 4 < 2 ** 32):
-        for t, n in ((boxes, "boxes"), (wg_w, "wg_w"), (wg_b, "wg_b"), (out, "out")):
-            _chk(t, n)
-        lib.call("sc_box_bias_all_tc", lib.ptr(boxes), lib.ptr(wg_w), lib.ptr(wg_b), lib.ptr(out), B, N, layers, h, wave_len, lib.stream())
+        lib.call("sc_box_bias_all_tc", boxes, wg_w, wg_b, out, B, N, layers, h, wave_len)
         return out
-    lib.call("sc_box_bias_all", lib.ptr(boxes), lib.ptr(wg_w), lib.ptr(wg_b), lib.ptr(out), B, N, layers, h, int(trig),
-             wave_len, lib.stream())
+    lib.call("sc_box_bias_all", boxes, wg_w, wg_b, out, B, N, layers, h, int(trig), wave_len)
     return out
 
 
 def bias_attention(q, k, v, bias, att_mask, out, *, B, N, h, dk, ldq, ldk, ldv, ldo):
     """box_attention of one layer given its geometry bias [B,h,N,N] (bf16 tensor path, sc_bias_attention_fwd)."""
-    lib.call("sc_bias_attention_fwd", lib.ptr(q), lib.ptr(k), lib.ptr(v), ldq, ldk, ldv, lib.dtype_code(out.dtype),
-             lib.ptr(bias), lib.ptr(att_mask), lib.ptr(out), ldo, B, N, h, dk, lib.stream())
+    lib.call("sc_bias_attention_fwd", lib.Strided(q), lib.Strided(k), lib.Strided(v), ldq, ldk, ldv, lib.dtype_code(out.dtype),
+             bias, att_mask, lib.Strided(out), ldo, B, N, h, dk)
     return out
 
 
 def self_attn_step(q, k, v, cache_k, cache_v, anc, out, *, R, D, h, n_prev, write_slot, ldq, ldk, ldv, ldo, anc_ld,
                    slot_div=1):
-    lib.call("sc_decode_self_attn_step", lib.ptr(q), lib.ptr(k), lib.ptr(v), ldq, ldk, ldv, lib.dtype_code(out.dtype),
-             lib.ptr(cache_k), lib.ptr(cache_v), lib.ptr(anc), anc_ld, slot_div, lib.ptr(out), ldo, R, D, h, n_prev,
-             write_slot, lib.stream())
+    lib.call("sc_decode_self_attn_step", lib.Strided(q), lib.Strided(k), lib.Strided(v), ldq, ldk, ldv, lib.dtype_code(out.dtype),
+             cache_k, cache_v, anc, anc_ld, slot_div, lib.Strided(out), ldo, R, D, h, n_prev, write_slot)
     return out
 
 
 def cross_attn_step(q, mem_k, mem_v, att_mask, out, *, B, beam, N, D, h, ldq, ldm, ldo):
-    lib.call("sc_decode_cross_attn_step", lib.ptr(q), ldq, lib.ptr(mem_k), lib.ptr(mem_v), ldm, lib.dtype_code(out.dtype),
-             lib.ptr(att_mask), lib.ptr(out), ldo, B, beam, N, D, h, lib.stream())
+    lib.call("sc_decode_cross_attn_step", lib.Strided(q), ldq, lib.Strided(mem_k), lib.Strided(mem_v), ldm, lib.dtype_code(out.dtype),
+             att_mask, lib.Strided(out), ldo, B, beam, N, D, h)
     return out
 
 
@@ -393,11 +364,10 @@ def beam_step(logits, st, t, *, B, beam, V, L, eos, pad, temperature=1.0, constr
     ``group`` at its local step ``t`` (sc_beam_step_diverse; group_seq int32 [G, 2, B*beam, L] holds every group's seq)."""
     i, o = t & 1, (t + 1) & 1
     assert suppress_tok is None or (suppress_tok.dtype == torch.int32 and suppress_tok.numel() == B * beam)
-    head = [lib.ptr(logits), B, beam, V, L, t, eos, pad, float(temperature), int(constraint), int(penalty_kind), float(penalty_alpha),
-            lib.ptr(suppress_tok), int(penalized_col)]
-    tail = [lib.ptr(st.seq[i]), lib.ptr(st.seq[o]), lib.ptr(st.lp[i]), lib.ptr(st.lp[o]), lib.ptr(st.sum), lib.ptr(st.anc[i]),
-            lib.ptr(st.anc[o]), lib.ptr(st.tokens), lib.ptr(st.done_seq), lib.ptr(st.done_lp), lib.ptr(st.done_p),
-            lib.ptr(st.done_count), lib.ptr(st.ws), st.ws.numel(), lib.stream()]
+    head = [logits, B, beam, V, L, t, eos, pad, float(temperature), int(constraint), int(penalty_kind), float(penalty_alpha),
+            suppress_tok, int(penalized_col)]
+    tail = [st.seq[i], st.seq[o], st.lp[i], st.lp[o], st.sum, st.anc[i], st.anc[o], st.tokens, st.done_seq, st.done_lp, st.done_p,
+            st.done_count, st.ws, st.ws.numel()]
     if diverse is None:
         lib.call("sc_beam_step", *head, *tail)
     else:
@@ -406,8 +376,8 @@ def beam_step(logits, st, t, *, B, beam, V, L, eos, pad, temperature=1.0, constr
 
 def _diverse_args(diverse, B, beam, L):
     hist, group, lam = diverse
-    assert hist.dtype == torch.int32 and hist.is_contiguous() and tuple(hist.shape[1:]) == (2, B * beam, L) and group < hist.shape[0]
-    return [lib.ptr(hist), int(group), float(lam)]
+    assert hist.dtype == torch.int32 and tuple(hist.shape[1:]) == (2, B * beam, L) and group < hist.shape[0]
+    return [hist, int(group), float(lam)]
 
 
 def linear_hmask(x, w, h, out, *, scale=1.0, colsum=None):
@@ -415,9 +385,7 @@ def linear_hmask(x, w, h, out, *, scale=1.0, colsum=None):
     M, K = x.shape
     N = w.shape[0]
     assert x.dtype == w.dtype == h.dtype == out.dtype == torch.bfloat16 and tuple(h.shape) == tuple(out.shape) == (M, N)
-    for t, n in ((x, "x"), (w, "w"), (h, "h"), (out, "out"), (colsum, "colsum")):
-        _chk(t, n)
-    lib.call("sc_linear_hmask", lib.ptr(x), lib.ptr(w), lib.ptr(h), float(scale), lib.ptr(colsum), lib.ptr(out), M, N, K, lib.stream(),
+    lib.call("sc_linear_hmask", x, w, h, float(scale), colsum, out, M, N, K,
              meta=("gemm_bf16", M, N, K, 2, 2, 2, False, False, False))
     return out
 
@@ -433,10 +401,8 @@ def linear_topk(x, w, bias, partials, candidates=5):
     M, K = x.shape
     N = w.shape[0]
     assert x.dtype == torch.bfloat16 and w.dtype == torch.bfloat16 and w.shape[1] == K
-    assert tuple(partials.shape) == (M, linear_topk_parts(N), 12) and partials.dtype == torch.float32 and partials.is_contiguous()
-    for t, n in ((x, "x"), (w, "w"), (bias, "bias"), (partials, "partials")):
-        _chk(t, n)
-    lib.call("sc_linear_topk", lib.ptr(x), lib.ptr(w), lib.ptr(bias), M, N, K, lib.ptr(partials), int(candidates), lib.stream(),
+    assert tuple(partials.shape) == (M, linear_topk_parts(N), 12) and partials.dtype == torch.float32
+    lib.call("sc_linear_topk", x, w, bias, M, N, K, partials, int(candidates),
              meta=("gemm_bf16", M, N, K, 2, 2, 0, False, False, False))
     return partials
 
@@ -445,10 +411,9 @@ def beam_step_partials(partials, st, t, *, B, beam, V, L, eos, pad, penalty_kind
     """Beam step from sc_linear_topk records (temperature 1, no decoding constraint, beam <= 5).  ``diverse``: as in
     ``beam_step`` (the records must hold (group + 1) * beam candidates per row)."""
     i, o = t & 1, (t + 1) & 1
-    head = [lib.ptr(partials), partials.shape[1], B, beam, V, L, t, eos, pad, int(penalty_kind), float(penalty_alpha)]
-    tail = [lib.ptr(st.seq[i]), lib.ptr(st.seq[o]), lib.ptr(st.lp[i]), lib.ptr(st.lp[o]), lib.ptr(st.sum), lib.ptr(st.anc[i]),
-            lib.ptr(st.anc[o]), lib.ptr(st.tokens), lib.ptr(st.done_seq), lib.ptr(st.done_lp), lib.ptr(st.done_p),
-            lib.ptr(st.done_count), lib.ptr(st.ws), st.ws.numel(), lib.stream()]
+    head = [partials, partials.shape[1], B, beam, V, L, t, eos, pad, int(penalty_kind), float(penalty_alpha)]
+    tail = [st.seq[i], st.seq[o], st.lp[i], st.lp[o], st.sum, st.anc[i], st.anc[o], st.tokens, st.done_seq, st.done_lp, st.done_p,
+            st.done_count, st.ws, st.ws.numel()]
     if diverse is None:
         lib.call("sc_beam_step_partials", *head, *tail)
     else:
@@ -460,14 +425,13 @@ def beam_step_workspace_bytes(B, beam):
 
 
 def greedy_step(logits, st, t, *, R, V, L, eos, constraint=0):
-    lib.call("sc_greedy_step", lib.ptr(logits), R, V, L, t, eos, int(constraint), lib.ptr(st.seq), lib.ptr(st.lp),
-             lib.ptr(st.tokens), lib.ptr(st.unfinished), lib.ptr(st.live), lib.stream())
+    lib.call("sc_greedy_step", logits, R, V, L, t, eos, int(constraint), st.seq, st.lp, st.tokens, st.unfinished, st.live)
 
 
 def sample_step(logits, st, t, *, R, V, L, eos, constraint=0, temperature=1.0, uniforms=None, seed=0):
     """Multinomial step on a GreedyState (one row per sample): sc_sample_step."""
-    lib.call("sc_sample_step", lib.ptr(logits), R, V, L, t, eos, int(constraint), float(temperature), lib.ptr(uniforms), seed,
-             lib.ptr(st.seq), lib.ptr(st.lp), lib.ptr(st.tokens), lib.ptr(st.unfinished), lib.ptr(st.live), lib.stream())
+    lib.call("sc_sample_step", logits, R, V, L, t, eos, int(constraint), float(temperature), uniforms, seed,
+             st.seq, st.lp, st.tokens, st.unfinished, st.live)
 
 
 def cache_reorder(src, idx, out=None):
@@ -477,7 +441,7 @@ def cache_reorder(src, idx, out=None):
     if out is None:
         out = torch.empty((rows,) + tuple(src.shape[1:]), device=src.device, dtype=src.dtype)
     assert idx.dtype == torch.int32
-    lib.call("sc_cache_reorder", lib.ptr(src), lib.ptr(out), lib.ptr(idx), rows, row_bytes, lib.stream())
+    lib.call("sc_cache_reorder", src, out, idx, rows, row_bytes)
     return out
 
 
@@ -497,9 +461,8 @@ def linear_dropout(x, w, bias=None, *, mask=None, mask_mode=MASK_NONE, uniforms=
         out = torch.empty(M, N, device=x.device, dtype=out_dtype or torch.float32)
     if mask is None:
         mask_mode = MASK_NONE
-    lib.call("sc_linear_dropout", lib.ptr(x), lib.dtype_code(x.dtype), lib.ptr(w), lib.dtype_code(w.dtype), lib.ptr(mask),
-             mask_mode, lib.ptr(uniforms), seed, stream_id, lib.ptr(bias), lib.ptr(residual), lib.ptr(out),
-             lib.dtype_code(out.dtype), M, N, K, int(relu), tile_n, float(p), drop_seed, drop_stream, lib.stream(),
+    lib.call("sc_linear_dropout", x, lib.dtype_code(x.dtype), w, lib.dtype_code(w.dtype), mask, mask_mode, uniforms, seed,
+             stream_id, bias, residual, out, lib.dtype_code(out.dtype), M, N, K, int(relu), tile_n, float(p), drop_seed, drop_stream,
              meta=("gemm_bf16" if x.dtype == torch.bfloat16 else "gemm_f32", M, N, K, x.element_size(), w.element_size(),
                    out.element_size(), mask is not None, residual is not None, bool(relu), p > 0, tile_n))
     return out
@@ -513,9 +476,9 @@ def linear_wgrad(dyT, xT, w, mask, mask_mode, dw, ds, *, M, uniforms=None, seed=
     assert dyT.shape[0] == N and xT.shape[0] == K and dyT.shape[1] == xT.shape[1] == M
     if mask is None:
         mask_mode = MASK_NONE
-    lib.call("sc_linear_wgrad", lib.ptr(dyT), lib.ptr(xT), lib.dtype_code(dyT.dtype), lib.ptr(w), lib.ptr(mask), mask_mode,
-             lib.ptr(uniforms), seed, stream_id, int(bypass), float(sp_coeff), lib.ptr(dw), lib.ptr(ds), int(accumulate), N, K,
-             M, tile_n, lib.ptr(workspace), 0 if workspace is None else workspace.numel() * workspace.element_size(), lib.stream(),
+    lib.call("sc_linear_wgrad", dyT, xT, lib.dtype_code(dyT.dtype), w, mask, mask_mode, uniforms, seed, stream_id, int(bypass),
+             float(sp_coeff), dw, ds, int(accumulate), N, K, M, tile_n, workspace,
+             0 if workspace is None else workspace.numel() * workspace.element_size(),
              meta=("gemm_bf16" if dyT.dtype == torch.bfloat16 else "gemm_f32", N, K, M, dyT.element_size(), xT.element_size(), 4, False))
 
 
@@ -525,12 +488,11 @@ def linear_wgrad_rowmajor(dy, x, w, mask, mask_mode, dw, ds, *, workspace, unifo
     N, K = w.shape
     M = dy.shape[0]
     assert dy.shape[1] == N and tuple(x.shape) == (M, K) and dy.dtype == x.dtype == torch.bfloat16
-    _chk(dy, "dy"), _chk(x, "x")
     if mask is None:
         mask_mode = MASK_NONE
-    lib.call("sc_linear_wgrad_rowmajor", lib.ptr(dy), lib.ptr(x), lib.ptr(w), lib.ptr(mask), mask_mode, lib.ptr(uniforms), seed,
-             stream_id, int(bypass), float(sp_coeff), lib.ptr(dw), lib.ptr(ds), int(accumulate), N, K, M, lib.ptr(workspace),
-             workspace.numel() * workspace.element_size(), lib.stream(), meta=("gemm_bf16", N, K, M, 2, 2, 4, False))
+    lib.call("sc_linear_wgrad_rowmajor", dy, x, w, mask, mask_mode, uniforms, seed, stream_id, int(bypass), float(sp_coeff), dw,
+             ds, int(accumulate), N, K, M, workspace, workspace.numel() * workspace.element_size(),
+             meta=("gemm_bf16", N, K, M, 2, 2, 4, False))
 
 
 def prep_grad(g, *, h=None, out=None, outT=None, scale=1.0, p=0.0, seed=0, stream_id=0, colsum=None):
@@ -540,15 +502,13 @@ def prep_grad(g, *, h=None, out=None, outT=None, scale=1.0, p=0.0, seed=0, strea
     assert g.dtype == torch.float32
     ref = out if out is not None else outT
     ldT = outT.shape[1] if outT is not None else rows
-    lib.call("sc_prep_grad", lib.ptr(g), lib.ptr(h), lib.dtype_code(h.dtype) if h is not None else F32, lib.ptr(out),
-             lib.ptr(outT), ldT, lib.dtype_code(ref.dtype), rows, cols, float(scale), float(p), seed, stream_id, lib.ptr(colsum),
-             lib.stream())
+    lib.call("sc_prep_grad", g, h, lib.dtype_code(h.dtype) if h is not None else F32, out, outT, ldT, lib.dtype_code(ref.dtype), rows,
+             cols, float(scale), float(p), seed, stream_id, colsum)
 
 
 def transpose(x, outT):
     rows, cols = x.shape
-    lib.call("sc_transpose", lib.ptr(x), lib.dtype_code(x.dtype), lib.ptr(outT), outT.shape[1], lib.dtype_code(outT.dtype), rows,
-             cols, lib.stream())
+    lib.call("sc_transpose", x, lib.dtype_code(x.dtype), outT, outT.shape[1], lib.dtype_code(outT.dtype), rows, cols)
     return outT
 
 
@@ -558,8 +518,7 @@ def apply_mask_transposed(w, mask, mask_mode, outT, *, uniforms=None, seed=0, st
     assert tuple(outT.shape) == (K, N) and (out is None or (tuple(out.shape) == (N, K) and out.dtype == outT.dtype))
     if mask is None:
         mask_mode = MASK_NONE
-    lib.call("sc_apply_mask_transposed", lib.ptr(w), lib.ptr(mask), mask_mode, lib.ptr(uniforms), seed, stream_id, lib.ptr(outT),
-             lib.dtype_code(outT.dtype), N, K, lib.ptr(out), lib.stream())
+    lib.call("sc_apply_mask_transposed", w, mask, mask_mode, uniforms, seed, stream_id, outT, lib.dtype_code(outT.dtype), N, K, out)
     return outT
 
 
@@ -567,32 +526,31 @@ def mask_descriptors(items, device):
     """Descriptor table of sc_apply_mask_batched.  items: (w [N,K] fp32, s | None, u | None, out | None, outT | None, stream_id).
     Returns (int64 device tensor [n, 10], total 64x64 tiles)."""
     rows, start = [], 0
-    for w, s, u, out, outT, sid in items:
+    for i, (w, s, u, out, outT, sid) in enumerate(items):
         N, K = w.shape
-        assert K % 4 == 0 and w.is_contiguous() and (out is None or out.is_contiguous()) and (outT is None or outT.is_contiguous())
+        assert K % 4 == 0
         tk = (K + 63) // 64
-        rows.append([w.data_ptr(), 0 if s is None else s.data_ptr(), 0 if u is None else u.data_ptr(),
-                     0 if out is None else out.data_ptr(), 0 if outT is None else outT.data_ptr(), N, K, int(sid), start, tk])
+        rows.append([lib.address(t, "sc_apply_mask_batched", f"descs[{i}].{f}") for t, f in
+                     ((w, "w"), (s, "s"), (u, "uniforms"), (out, "out"), (outT, "outT"))] + [N, K, int(sid), start, tk])
         start += tk * ((N + 63) // 64)
     return torch.tensor(rows, dtype=torch.int64).to(device), start
 
 
 def apply_mask_batched(desc, total_tiles, mask_mode, *, seed=0, stream_base=0, out_dtype=torch.bfloat16):
-    lib.call("sc_apply_mask_batched", lib.ptr(desc), desc.shape[0], total_tiles, mask_mode, seed, stream_base,
-             lib.dtype_code(out_dtype), lib.stream())
+    lib.call("sc_apply_mask_batched", desc, desc.shape[0], total_tiles, mask_mode, seed, stream_base, lib.dtype_code(out_dtype))
 
 
 def mask_grad(dwm, w, mask, mask_mode, dw, ds, *, uniforms=None, seed=0, stream_id=0, bypass=False, sp_coeff=0.0,
               accumulate=False):
     if mask is None:
         mask_mode = MASK_NONE
-    lib.call("sc_mask_grad", lib.ptr(dwm), lib.ptr(w), lib.ptr(mask), mask_mode, lib.ptr(uniforms), seed, stream_id, int(bypass),
-             float(sp_coeff), lib.ptr(dw), lib.ptr(ds), int(accumulate), w.numel(), lib.stream())
+    lib.call("sc_mask_grad", dwm, w, mask, mask_mode, uniforms, seed, stream_id, int(bypass), float(sp_coeff), dw, ds,
+             int(accumulate), w.numel())
 
 
 def colsum(x, out, accumulate=False):
     rows, cols = x.shape
-    lib.call("sc_colsum", lib.ptr(x), lib.dtype_code(x.dtype), lib.ptr(out), rows, cols, int(accumulate), lib.stream())
+    lib.call("sc_colsum", x, lib.dtype_code(x.dtype), out, rows, cols, int(accumulate))
     return out
 
 
@@ -601,21 +559,18 @@ def layernorm_bwd(x, a, dy, dx, da, db, *, dres=None, eps=1e-6, next_gb=None, ne
     the next linear in the backward chain and add its column sums to ``next_colsum`` (sc_layernorm_bwd_fused)."""
     rows, D = x.shape
     if next_gb is None:
-        lib.call("sc_layernorm_bwd", lib.ptr(x), lib.ptr(a), lib.ptr(dy), lib.dtype_code(dy.dtype), lib.ptr(dres), lib.ptr(dx),
-                 lib.ptr(da), lib.ptr(db), rows, D, eps, lib.stream())
+        lib.call("sc_layernorm_bwd", x, a, dy, lib.dtype_code(dy.dtype), dres, dx, da, db, rows, D, eps)
     else:
-        assert next_gb.dtype == torch.bfloat16 and tuple(next_gb.shape) == (rows, D) and next_gb.is_contiguous()
-        lib.call("sc_layernorm_bwd_fused", lib.ptr(x), lib.ptr(a), lib.ptr(dy), lib.dtype_code(dy.dtype), lib.ptr(dres), lib.ptr(dx),
-                 lib.ptr(da), lib.ptr(db), rows, D, eps, lib.ptr(next_gb), lib.ptr(next_colsum), float(next_p), seed, stream_id,
-                 lib.stream())
+        assert next_gb.dtype == torch.bfloat16 and tuple(next_gb.shape) == (rows, D)
+        lib.call("sc_layernorm_bwd_fused", x, a, dy, lib.dtype_code(dy.dtype), dres, dx, da, db, rows, D, eps, next_gb, next_colsum,
+                 float(next_p), seed, stream_id)
     return dx
 
 
 def logsoftmax_nll(logits, target=None, weight=None, inv_norm=None, loss_sum=None, dlogits=None, logprobs=None):
     rows, V = logits.shape
-    lib.call("sc_logsoftmax_nll", lib.ptr(logits), lib.ptr(target), lib.ptr(weight), lib.ptr(inv_norm), lib.ptr(loss_sum),
-             lib.ptr(dlogits), lib.dtype_code(dlogits.dtype) if dlogits is not None else F32, lib.ptr(logprobs), rows, V,
-             lib.stream())
+    lib.call("sc_logsoftmax_nll", logits, target, weight, inv_norm, loss_sum, dlogits,
+             lib.dtype_code(dlogits.dtype) if dlogits is not None else F32, logprobs, rows, V)
 
 
 def scst_targets(seq, score, base_score, *, S, cider_weight, bos, pad, tokens, targets, tok_w, key_valid, inv_norm, mask_sum=None,
@@ -623,25 +578,23 @@ def scst_targets(seq, score, base_score, *, S, cider_weight, bos, pad, tokens, t
     """SCST rollout seq int32 [R, L] + CIDEr-D scores float64 [R] (+ greedy baseline scores float64 [R // S], or None: mean of
     the image's other samples) -> the training step's tokens / targets / tok_w / key_valid [R * L] and inv_norm (sc_scst_targets)."""
     R, L = seq.shape
-    assert seq.dtype == torch.int32 and seq.is_contiguous() and score.dtype == torch.float64 and score.numel() == R
+    assert seq.dtype == torch.int32 and score.dtype == torch.float64 and score.numel() == R
     assert base_score is None or (base_score.dtype == torch.float64 and base_score.numel() == R // S)
     for t, dt in ((tokens, torch.int32), (targets, torch.int32), (tok_w, torch.float32), (key_valid, torch.float32)):
-        assert t.dtype == dt and t.numel() == R * L and t.is_contiguous()
-    lib.call("sc_scst_targets", lib.ptr(seq), R, L, int(S), lib.ptr(score), lib.ptr(base_score), float(cider_weight), int(bos), int(pad),
-             lib.ptr(tokens), lib.ptr(targets), lib.ptr(tok_w), lib.ptr(key_valid), lib.ptr(mask_sum), lib.ptr(inv_norm),
-             lib.ptr(norm_in), lib.ptr(mean_reward), lib.stream())
+        assert t.dtype == dt and t.numel() == R * L
+    lib.call("sc_scst_targets", seq, R, L, int(S), score, base_score, float(cider_weight), int(bos), int(pad), tokens, targets, tok_w,
+             key_valid, mask_sum, inv_norm, norm_in, mean_reward)
 
 
 def embedding_bwd(tokens, dy, dtable, scale):
     rows, D = dy.shape
-    lib.call("sc_embedding_bwd", lib.ptr(tokens), lib.ptr(dy), lib.ptr(dtable), rows, D, dtable.shape[0], float(scale), lib.stream())
+    lib.call("sc_embedding_bwd", tokens, dy, dtable, rows, D, dtable.shape[0], float(scale))
 
 
 def adam_clip(param, grad, m, v, *, lr, betas, eps, weight_decay, clip, grad_scale, step, sigmoid_grad_coeff=None, dyn=None):
     """``dyn``: optional device fp32 [3] = {lr, 1 - b1^step, sqrt(1 - b2^step)} read at run time (CUDA-graph replay)."""
-    lib.call("sc_adam_clip", lib.ptr(param), lib.ptr(grad), lib.ptr(m), lib.ptr(v), param.numel(), float(lr), float(betas[0]),
-             float(betas[1]), float(eps), float(weight_decay), float(clip), float(grad_scale), int(step),
-             lib.ptr(sigmoid_grad_coeff), lib.ptr(dyn), lib.stream())
+    lib.call("sc_adam_clip", param, grad, m, v, param.numel(), float(lr), float(betas[0]), float(betas[1]), float(eps),
+             float(weight_decay), float(clip), float(grad_scale), int(step), sigmoid_grad_coeff, dyn)
 
 
 def st_descriptors(segments, device):
@@ -659,10 +612,9 @@ def adam_clip_st(desc, blocks, w, g, m_w, v_w, s, m_s, v_s, *, uniforms, mask_mo
                  weight_decay, mask_lr, mask_eps, betas, clip, grad_scale, step, sigmoid_grad_coeff=None, dyn=None):
     """One-launch optimizer step over a descriptor table (sc_adam_clip_st): straight-through dW / dS from the exchanged dWm
     with the mask sample regenerated, then clip + Adam for the weight and the mask-logit groups."""
-    lib.call("sc_adam_clip_st", lib.ptr(desc), desc.shape[0], blocks, lib.ptr(w), lib.ptr(g), lib.ptr(m_w), lib.ptr(v_w), lib.ptr(s),
-             lib.ptr(m_s), lib.ptr(v_s), lib.ptr(uniforms), int(mask_mode), int(bypass), int(update_logits), seed, stream_base,
-             float(lr), float(eps), float(weight_decay), float(mask_lr), float(mask_eps), float(betas[0]), float(betas[1]), float(clip),
-             float(grad_scale), int(step), lib.ptr(sigmoid_grad_coeff), lib.ptr(dyn), lib.stream())
+    lib.call("sc_adam_clip_st", desc, desc.shape[0], blocks, w, g, m_w, v_w, s, m_s, v_s, uniforms, int(mask_mode), int(bypass),
+             int(update_logits), seed, stream_base, float(lr), float(eps), float(weight_decay), float(mask_lr), float(mask_eps),
+             float(betas[0]), float(betas[1]), float(clip), float(grad_scale), int(step), sigmoid_grad_coeff, dyn)
 
 
 PRUNE_ABS, PRUNE_DIST, PRUNE_SNIP = 0, 1, 2
@@ -692,13 +644,12 @@ def _to_device(t, device):
 def prune_stats(desc, blocks, src, *, binarize=False, centered=False):
     """Per-segment {sum x, sum x^2} (float64 [n_desc, 2]) of ``src`` (or of rint(sigmoid(src)) with ``binarize``); ``centered``:
     {sum x, sum (x - mean)^2} from a second pass (the two-pass variance of mag_dist)."""
-    assert src.dtype == torch.float32 and src.is_contiguous()
+    assert src.dtype == torch.float32
     partials = torch.empty(blocks, 2, dtype=torch.float64, device=src.device)
 
     def run(center):
         sums = torch.empty(desc.shape[0], 2, dtype=torch.float64, device=src.device)
-        lib.call("sc_prune_stats", lib.ptr(desc), desc.shape[0], blocks, lib.ptr(src), int(binarize), lib.ptr(center), lib.ptr(partials),
-                 lib.ptr(sums), lib.stream())
+        lib.call("sc_prune_stats", desc, desc.shape[0], blocks, src, int(binarize), center, partials, sums)
         return sums
 
     sums = run(None)
@@ -711,80 +662,73 @@ def prune_select(desc, blocks, group_k, criterion, src, mask_out, *, sums=None):
     prune_stats of ``src`` for PRUNE_SNIP, prune_stats(centered=True) for PRUNE_DIST."""
     if not torch.is_tensor(group_k):
         group_k = _to_device(torch.tensor(group_k, dtype=torch.int64), src.device)
-    assert src.dtype == mask_out.dtype == torch.float32 and group_k.dtype == torch.int64 and group_k.is_cuda
+    assert src.dtype == mask_out.dtype == torch.float32 and group_k.dtype == torch.int64
     n_groups = group_k.numel()
     ws = torch.empty(n_groups * 1056 + desc.shape[0] * 8, dtype=torch.uint8, device=src.device)
-    lib.call("sc_prune_select", lib.ptr(desc), desc.shape[0], blocks, n_groups, lib.ptr(group_k), int(criterion), lib.ptr(src),
-             lib.ptr(sums), lib.ptr(mask_out), lib.ptr(ws), ws.numel(), lib.stream())
+    lib.call("sc_prune_select", desc, desc.shape[0], blocks, n_groups, group_k, int(criterion), src, sums, mask_out, ws, ws.numel())
     return mask_out
 
 
 def sparsity_coeff(count, total, target, scale, out3, scale_dev=None):
     """out3 = [|target - sparsity|, d(scaled loss)/d(nnz), sparsity] from the device-side binarized-mask count."""
-    lib.call("sc_sparsity_coeff", lib.ptr(count), float(total), float(target), float(scale), lib.ptr(scale_dev), lib.ptr(out3),
-             lib.stream())
+    lib.call("sc_sparsity_coeff", count, float(total), float(target), float(scale), scale_dev, out3)
     return out3
 
 
 def attention_fwd(q, k, v, out, probs, *, G, Tq, Tk, h, dk, ldq, ldk, ldv, ldo, key_valid=None, bias=None, causal_T=0, p=0.0,
                   seed=0, stream_id=0):
-    lib.call("sc_attention_fwd", lib.ptr(q), lib.ptr(k), lib.ptr(v), ldq, ldk, ldv, lib.dtype_code(out.dtype), lib.ptr(key_valid),
-             lib.ptr(bias), lib.ptr(probs), lib.ptr(out), ldo, G, Tq, Tk, h, dk, causal_T, float(p), seed, stream_id, lib.stream())
+    lib.call("sc_attention_fwd", lib.Strided(q), lib.Strided(k), lib.Strided(v), ldq, ldk, ldv, lib.dtype_code(out.dtype), key_valid,
+             bias, probs, lib.Strided(out), ldo, G, Tq, Tk, h, dk, causal_T, float(p), seed, stream_id)
     return out
 
 
 def attention_bwd(q, k, v, probs, d_out, dq, dk_, dv, *, dtype, G, Tq, Tk, h, dk, ldq, ldk, ldv, ldd, ldgq, ldgk, ldgv, dbias=None,
                   p=0.0, seed=0, stream_id=0):
-    lib.call("sc_attention_bwd", lib.ptr(q), lib.ptr(k), lib.ptr(v), ldq, ldk, ldv, lib.dtype_code(dtype), lib.ptr(probs),
-             lib.ptr(d_out), ldd, lib.ptr(dq), lib.ptr(dk_), lib.ptr(dv), ldgq, ldgk, ldgv, lib.ptr(dbias), G, Tq, Tk, h, dk,
-             float(p), seed, stream_id, lib.stream())
+    lib.call("sc_attention_bwd", lib.Strided(q), lib.Strided(k), lib.Strided(v), ldq, ldk, ldv, lib.dtype_code(dtype), probs,
+             lib.Strided(d_out), ldd, lib.Strided(dq), lib.Strided(dk_), lib.Strided(dv), ldgq, ldgk, ldgv, dbias, G, Tq, Tk, h, dk,
+             float(p), seed, stream_id)
 
 
 def attention_bwd_bf16out(q, k, v, probs, d_out, dq, dk_, dv, *, G, Tq, Tk, h, dk, ldq, ldk, ldv, ldd, ldgq, ldgk, ldgv, bq=None, bk=None,
                           bv=None, dbias=None, p=0.0, seed=0, stream_id=0):
     """attention_bwd whose dq / dk / dv are bf16 GEMM operands and whose bias gradients (column sums) go to bq / bk / bv."""
     assert dq.dtype == dk_.dtype == dv.dtype == torch.bfloat16
-    lib.call("sc_attention_bwd_bf16out", lib.ptr(q), lib.ptr(k), lib.ptr(v), ldq, ldk, ldv, lib.ptr(probs), lib.ptr(d_out), ldd,
-             lib.ptr(dq), lib.ptr(dk_), lib.ptr(dv), ldgq, ldgk, ldgv, lib.ptr(bq), lib.ptr(bk), lib.ptr(bv), lib.ptr(dbias), G, Tq, Tk,
-             h, dk, float(p), seed, stream_id, lib.stream())
+    lib.call("sc_attention_bwd_bf16out", lib.Strided(q), lib.Strided(k), lib.Strided(v), ldq, ldk, ldv, probs, lib.Strided(d_out),
+             ldd, lib.Strided(dq), lib.Strided(dk_), lib.Strided(dv), ldgq, ldgk, ldgv, bq, bk, bv, dbias, G, Tq, Tk, h, dk, float(p),
+             seed, stream_id)
 
 
 def box_bias_fwd(boxes, wg_w, wg_b, bias, *, B, N, h, trig=True, wave_len=1000.0):
-    lib.call("sc_box_bias_fwd", lib.ptr(boxes), lib.ptr(wg_w), lib.ptr(wg_b), lib.ptr(bias), B, N, h, int(trig), wave_len,
-             lib.stream())
+    lib.call("sc_box_bias_fwd", boxes, wg_w, wg_b, bias, B, N, h, int(trig), wave_len)
     return bias
 
 
 def box_bias_bwd(boxes, bias, dbias, dwg_w, dwg_b, *, B, N, h, trig=True, wave_len=1000.0):
-    lib.call("sc_box_bias_bwd", lib.ptr(boxes), lib.ptr(bias), lib.ptr(dbias), lib.ptr(dwg_w), lib.ptr(dwg_b), B, N, h, int(trig),
-             wave_len, lib.stream())
+    lib.call("sc_box_bias_bwd", boxes, bias, dbias, dwg_w, dwg_b, B, N, h, int(trig), wave_len)
 
 
 def box_embedding(boxes, *, trig=True, wave_len=1000.0, out=None):
     """BoxRelationalEmbedding (relation_transformer.py:196-256): boxes fp32 [B,N,4] -> fp32 [B,N,N,64] (or [B,N,N,4])."""
     B, N = boxes.shape[:2]
-    _chk(boxes, "boxes")
     assert boxes.dtype == torch.float32
     if out is None:
         out = torch.empty(B, N, N, 64 if trig else 4, device=boxes.device)
-    lib.call("sc_box_embedding", lib.ptr(boxes), lib.ptr(out), B, N, int(trig), float(wave_len), lib.stream())
+    lib.call("sc_box_embedding", boxes, out, B, N, int(trig), float(wave_len))
     return out
 
 
 def log_clamp(x, *, lo=1e-6, dy=None, out=None):
     """out = log(max(x, lo)); with ``dy``: out = dy / x where x > lo else 0 (its gradient).  fp32."""
-    _chk(x, "x"), _chk(dy, "dy")
     if out is None:
         out = torch.empty_like(x)
-    lib.call("sc_log_clamp", lib.ptr(x), lib.ptr(dy), lib.ptr(out), x.numel(), float(lo), lib.stream())
+    lib.call("sc_log_clamp", x, dy, out, x.numel(), float(lo))
     return out
 
 
 def logsoftmax_bwd(logprobs, dy, out=None):
     """dx = dy - exp(logprobs) * rowsum(dy): backward of log_softmax (sc_logsoftmax_bwd)."""
     rows, V = logprobs.shape
-    _chk(logprobs, "logprobs"), _chk(dy, "dy")
     if out is None:
         out = torch.empty_like(logprobs)
-    lib.call("sc_logsoftmax_bwd", lib.ptr(logprobs), lib.ptr(dy), lib.ptr(out), rows, V, lib.stream())
+    lib.call("sc_logsoftmax_bwd", logprobs, dy, out, rows, V)
     return out

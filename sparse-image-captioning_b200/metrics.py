@@ -107,16 +107,13 @@ class CaptionMetrics:
         idx = torch.as_tensor(image_idx).to(self.dev, torch.int32).contiguous()
         if idx.shape != (H,):
             raise ValueError(f"image_idx has shape {tuple(idx.shape)}, expected ({H},)")
-        n, s, c = self.n_images, lib.stream(), self._cider
-        lib.call("sc_bleu_stats", lib.ptr(h), H, L, lib.ptr(idx), n, self.eos, self.pad, lib.ptr(self._key_off), lib.ptr(self._keys),
-                 lib.ptr(self._max_count), lib.ptr(self._img_ref_off), lib.ptr(self._tok_off), lib.ptr(self._stats),
-                 lib.ptr(self._count), lib.ptr(self._count[n:]), s)
-        lib.call("sc_rouge_l", lib.ptr(h), H, L, lib.ptr(idx), n, self.eos, self.pad, lib.ptr(self._img_ref_off), lib.ptr(self._tok_off),
-                 lib.ptr(self._toks), lib.ptr(self._rouge), s)
+        n, c = self.n_images, self._cider
+        lib.call("sc_bleu_stats", h, H, L, idx, n, self.eos, self.pad, self._key_off, self._keys, self._max_count, self._img_ref_off,
+                 self._tok_off, self._stats, self._count, self._count[n:])
+        lib.call("sc_rouge_l", h, H, L, idx, n, self.eos, self.pad, self._img_ref_off, self._tok_off, self._toks, self._rouge)
         r = c._refs
-        lib.call("sc_cider_score", lib.ptr(h), H, L, lib.ptr(idx), n, self.eos, self.pad, lib.ptr(c.df_keys), lib.ptr(c.df_log), c.n_df,
-                 c.ref_len, lib.ptr(r["img_off"]), lib.ptr(r["ng_off"]), lib.ptr(r["keys"]), lib.ptr(r["vec"]), lib.ptr(r["norm"]),
-                 lib.ptr(self._cider_out), s)
+        lib.call("sc_cider_score", h, H, L, idx, n, self.eos, self.pad, c.df_keys, c.df_log, c.n_df, c.ref_len, r["img_off"],
+                 r["ng_off"], r["keys"], r["vec"], r["norm"], self._cider_out)
 
     def compute(self) -> Tuple[Dict[str, float], torch.Tensor]:
         """One reduction launch and one device-to-host copy.  Raises ValueError unless every image of the split received exactly
@@ -124,8 +121,7 @@ class CaptionMetrics:
         if not self.n_images:
             raise RuntimeError("call set_refs() with the split's reference captions first")
         n = self.n_images
-        lib.call("sc_caption_metrics_reduce", lib.ptr(self._stats), lib.ptr(self._rouge), lib.ptr(self._cider_out), lib.ptr(self._count),
-                 lib.ptr(self._count[n:]), n, lib.ptr(self._out), lib.stream())
+        lib.call("sc_caption_metrics_reduce", self._stats, self._rouge, self._cider_out, self._count, self._count[n:], n, self._out)
         out = self._out.cpu()
         missing, repeated, bad = (int(v) for v in out[6:9].tolist())
         if missing or repeated or bad:

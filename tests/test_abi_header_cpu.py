@@ -1,5 +1,5 @@
 """include/sc_b200.h is the C interface that C and C++ callers include: it must compile on its own as C and as C++ (the
-ctypes table in test_abi_cpu.py reads it with comments stripped and would not notice a broken comment or declaration)."""
+ctypes binding in lib.py reads it with comments stripped and would not notice a broken comment or declaration)."""
 import os
 import shutil
 import subprocess

@@ -127,12 +127,12 @@ def test_diverse_partials_match_diverse_beam_step(K, G, bdash):
         torch.testing.assert_close(sa[g].done_lp, sb[g].done_lp, rtol=1e-5, atol=2e-5)
 
 
-def test_diverse_entry_points_reject_bad_arguments(K):
+def test_diverse_entry_points_report_library_errors(K):
     hist, sts = _states(2, 2, 3, 4)
     logits = torch.zeros(6, 100, device=DEV)
     with pytest.raises(RuntimeError, match="sc_beam_step_diverse"):
-        K.lib.call("sc_beam_step_diverse", K.lib.ptr(logits), 2, 3, 100, 4, 0, 3, 0, 1.0, 0, 0, 0.0, None, -1, None, 1, 0.5,
-                   *([K.lib.ptr(logits)] * 12), K.lib.ptr(sts[0].ws), sts[0].ws.numel(), K.lib.stream())
+        K.lib.call("sc_beam_step_diverse", logits, 2, 3, 100, 4, 0, 3, 0, 1.0, 0, 0, 0.0, None, -1, None, 1, 0.5, *([logits] * 12),
+                   sts[0].ws, sts[0].ws.numel())
     part = torch.zeros(6, K.linear_topk_parts(100), 12, device=DEV)
     with pytest.raises(RuntimeError, match="sc_beam_step_partials_diverse"):
         K.beam_step_partials(part, sts[1], 0, B=2, beam=3, V=100, L=4, eos=3, pad=0, diverse=(hist, 1, 0.5))

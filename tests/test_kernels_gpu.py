@@ -630,7 +630,7 @@ def test_ingest_pinned_host_features(K):
     assert torch.equal(out, x.cuda().bfloat16().view(-1))
 
 
-def test_new_entry_points_reject_bad_arguments(K):
+def test_new_entry_points_report_library_errors(K):
     """Error behaviour of the entry points added this round: negative status -> RuntimeError with the library's message,
     nothing launched."""
     from sparse_caption_b200.engine import BeamState
@@ -649,8 +649,34 @@ def test_new_entry_points_reject_bad_arguments(K):
     with pytest.raises(RuntimeError, match="beam=7"):
         K.beam_step_partials(torch.empty(14, 4, 12, device="cuda"), st, 0, B=2, beam=7, V=300, L=4, eos=3, pad=0)
     with pytest.raises(RuntimeError, match="sc_ingest_f32_bf16"):
-        K.lib.call("sc_ingest_f32_bf16", torch.randn(16, device="cuda").data_ptr(), torch.empty(16, device="cuda", dtype=torch.bfloat16).data_ptr(),
-                   16, 0, K.lib.stream())                       # a device pointer is not pinned host memory
+        K.lib.call("sc_ingest_f32_bf16", torch.randn(16, device="cuda").data_ptr(), torch.empty(16, device="cuda", dtype=torch.bfloat16),
+                   16, 0)                                       # a raw device address is not pinned host memory
+
+
+def test_pointer_arguments_are_checked_before_the_launch(K):
+    """lib.call refuses, in Python and before anything is enqueued, a CUDA or pageable tensor for the pinned host pointer of
+    sc_ingest_f32_bf16, a CPU tensor for a device pointer and a non-contiguous tensor; the launch count does not move."""
+    out = torch.empty(16, device="cuda", dtype=torch.bfloat16)
+    before = K.lib.launch_count
+    with pytest.raises(RuntimeError, match="^sc_ingest_f32_bf16: pinned_host must be a pinned CPU tensor, got a CUDA tensor"):
+        K.ingest_f32_bf16(torch.randn(16, device="cuda"), out)
+    with pytest.raises(RuntimeError, match="^sc_ingest_f32_bf16: pinned_host must be a pinned CPU tensor, got a pageable CPU tensor"):
+        K.ingest_f32_bf16(torch.randn(16), out)
+    with pytest.raises(RuntimeError, match="^sc_ingest_f32_bf16: y must be a CUDA tensor, got a cpu tensor"):
+        K.ingest_f32_bf16(torch.randn(16).pin_memory(), out.cpu())
+    with pytest.raises(RuntimeError, match="^sc_cast_f32_bf16: x must be contiguous"):
+        K.cast_bf16(torch.randn(8, 2, device="cuda").t())
+    assert K.lib.launch_count == before
+
+
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
+def test_tensor_on_another_device_is_refused(K):
+    x = torch.randn(16, device="cuda:1")
+    with torch.cuda.device(0):
+        with pytest.raises(RuntimeError, match=r"^sc_cast_f32_bf16: x is on cuda:1, not on the current device cuda:0"):
+            K.cast_bf16(x, out=torch.empty(16, device="cuda:0", dtype=torch.bfloat16))
+        with pytest.raises(RuntimeError, match=r"^sc_apply_mask_batched: descs\[0\]\.w is on cuda:1"):
+            K.mask_descriptors([(x.view(4, 4), None, None, None, None, 0)], "cuda:0")
 
 
 @pytest.mark.parametrize("mode", ["0", "1", "3"])
